@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — test rows/s of MMPFN ``predict_proba`` on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload at N=1 (BASELINE.json configs[1]): PAD-UFES-20 shape — 2000 train / 300 test rows,
 21 tabular features + one 768-d image embedding per row, 8 estimators, bf16, random-init
@@ -173,7 +173,7 @@ def _token_counts(clf):
     return sorted({(np.asarray(x).shape[1] + 1) // 2 + 8 + 1 for x in clf.executor_.X_trains}, reverse=True)
 
 
-def reference_cpu_sample(max_steps, warmup, budget_s):
+def reference_cpu_sample(steps, warmup):
     """Times the reference's own ``predict_proba`` (``classifier.py:517-576``, unmodified, diagnostic loop
     ``transformer.py:809-813`` included) on the host cores.  The estimators are a serial loop in the reference
     (``inference.py:294-349``) and its default ensemble alternates two preprocessing recipes, so a call with
@@ -184,17 +184,13 @@ def reference_cpu_sample(max_steps, warmup, budget_s):
     clf, d = _reference_classifier("cpu", 2)
     Ts = _token_counts(clf)
     times = []
-    t_start = time.perf_counter()
-    for i in range(warmup + max_steps):
+    for i in range(warmup + steps):
         t0 = time.perf_counter()
         p = clf.predict_proba(d["X_test"], d["img_test"])
         dt = time.perf_counter() - t0
         assert p.shape[0] == len(d["y_test"]) and np.allclose(p.sum(1), 1.0, atol=1e-5)
         if i >= warmup:
             times.append(dt)
-        # bounded: stop once another step would overrun the budget (at least one timed step)
-        if times and time.perf_counter() - t_start + dt > budget_s:
-            break
     return times, Ts, len(d["y_test"])
 
 
@@ -202,7 +198,7 @@ def run_reference(args):
     """--impl reference: the reference's own CPU implementation of the path, all host cores.  One step = one
     ``predict_proba`` call of the unmodified reference with 2 of the 8 estimators (see
     ``reference_cpu_sample``); ``ms_per_step`` is the time actually spent per step, ``value`` = test rows /
-    (4 x that).  ``steps`` is what was run inside the time bound, ``steps_requested`` what was asked for."""
+    (4 x that); exactly ``--steps`` steps are timed."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
@@ -211,7 +207,7 @@ def run_reference(args):
     n_tr, n_te = DATASETS[WORKLOAD][:2]
     cores = os.cpu_count() or 1
     if ref_compat.reference_available():
-        times, Ts, n_te = reference_cpu_sample(max(args.steps, 1), min(args.warmup, 1), budget_s=170.0)
+        times, Ts, n_te = reference_cpu_sample(args.steps, min(args.warmup, 1))
         step_s = float(np.mean(times))
         value = n_te / (step_s * (N_EST / 2))
         kind = "reference"
@@ -219,7 +215,6 @@ def run_reference(args):
                   f"{cores} threads, 2 of {N_EST} estimators per step (one of each preprocessing recipe, T={Ts}; "
                   f"the reference loops estimators serially), full {n_tr} train / {n_te} test rows, diagnostic loop "
                   f"included; value = {n_te} rows / ({N_EST // 2} x measured step)")
-        steps_run = len(times)
     else:                                            # no reference snapshot on this box: the oracle port
         total, n_tr, n_te = full_flops()
         t1, f1, _ = cpu_sample(1)
@@ -232,10 +227,9 @@ def run_reference(args):
         value = n_te / (step_s * total / fl)
         kind = "port"
         sample = f"oracle port: 1 of {N_EST} estimators (T=27), {layers} of {L} layers per step, scaled by algorithmic FLOPs"
-        steps_run = len(times)
     line = {
         "impl": "reference", "metric": "test rows/sec predict_proba", "value": value, "unit": "rows/s",
-        "n_gpus": args.gpus, "steps": steps_run, "steps_requested": args.steps, "warmup": min(args.warmup, 1),
+        "n_gpus": args.gpus, "steps": len(times), "warmup": min(args.warmup, 1),
         "ms_per_step": step_s * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
         "data": "synthetic",
         "config": {"workload": f"{WORKLOAD}: {n_tr} train / {n_te} test rows, 21 feats + 768-d image emb, "
@@ -422,6 +416,10 @@ def run_ours(args):
     value = world * n_te / (ms * 1e-3)
     proba_dev = proba_from_logits(lg, perms, n_classes=clf.n_classes_)
     assert np.allclose(proba_dev.sum(1), 1.0, atol=1e-5)
+    if args.dump_outputs and rank == 0:
+        # with N > 1 the step ends with every rank's probabilities all-gathered: that array is the step's result
+        dump_outputs(args.dump_outputs, logits=lg.float().cpu().numpy(),
+                     proba=gathered["p"].float().cpu().numpy() if world > 1 else proba_dev)
     strong = None
     if world > 1:
         pg = gathered["p"]
@@ -539,7 +537,7 @@ def run_ours(args):
     cpu = None
     if args.cpu_baseline:
         if have_ref:
-            times, Tref, _ = reference_cpu_sample(1, 0, budget_s=60.0)
+            times, Tref, _ = reference_cpu_sample(1, 0)
             cpu = {"value": n_te / (times[0] * (N_EST / 2)), "unit": "rows/s", "cores": os.cpu_count() or 1,
                    "kind": "reference",
                    "sample": f"unmodified reference predict_proba (oracle/_ref), device=cpu fp32, 2 of {N_EST} estimators "
@@ -580,6 +578,13 @@ def run_ours(args):
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(dirname, **arrays):
+    """Writes each array as ``dirname/<name>.npy`` in float32, so that the outputs of two builds can be compared."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
 
 
 def _time_kernel(torch, fn, iters=20, warm=3):
@@ -723,7 +728,14 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="launch kernels eagerly instead of replaying a CUDA graph")
     ap.add_argument("--profile", action="store_true",
                     help="for ncu: 1 warm-up + K device-resident steps only (no e2e / roofline / CPU legs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's per-estimator logits (rank 0) and the test rows' "
+                         "probabilities (all ranks) as DIR/logits.npy and DIR/proba.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours only")
     if args.impl == "ours" and not args.profile:
         args.warmup = max(args.warmup, 3)
     if args.impl == "reference":

@@ -187,7 +187,7 @@ def run_clf8():
         out[f"logits_{e}"] = lg
         out[f"class_perm_{e}"] = (np.arange(clf.n_classes_) if cfg.class_permutation is None
                                   else np.asarray(cfg.class_permutation))
-    np.savez_compressed(os.path.join(OUT, "large_clf8_pad_ufes.npz"), **out)
+    np.savez_compressed(os.path.join(OUT, "large_clf8_pad_ufes.npz"), **cases.pack_tables(out))
     print(f"clf8: proba {proba.shape}, F' {[r[0].shape[1] for r in rec]}, {time.time() - t0:.0f} s", flush=True)
 
 

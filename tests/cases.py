@@ -12,7 +12,31 @@ GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def load_golden(name):
-    return dict(np.load(os.path.join(GOLDEN, name + ".npz")))
+    g = dict(np.load(os.path.join(GOLDEN, name + ".npz")))
+    if "X_cols" in g:                                   # tables stored by pack_tables
+        cols = g.pop("X_cols")
+        for k in [k for k in g if k.startswith("X_col_index_")]:
+            g["X_full_" + k[len("X_col_index_"):]] = cols[:, g.pop(k)]
+    return g
+
+
+def pack_tables(out):
+    """Replaces the ``X_full_<e>`` tables of a golden dict by the pool of their distinct columns (``X_cols``) and one
+    column index per table (``X_col_index_<e>``): the estimators' tables share most of their columns, and stored
+    whole the 8-estimator PAD-UFES tables take more than 1 MB.  ``load_golden`` restores them bit for bit."""
+    pool, where = [], {}
+    for k in [k for k in out if k.startswith("X_full_")]:
+        X = out.pop(k)
+        idx = []
+        for j in range(X.shape[1]):
+            key = X[:, j].tobytes()
+            if key not in where:
+                where[key] = len(pool)
+                pool.append(X[:, j])
+            idx.append(where[key])
+        out["X_col_index_" + k[len("X_full_"):]] = np.asarray(idx, np.int16)
+    out["X_cols"] = np.stack(pool, 1)
+    return out
 
 
 def model_case(name):
