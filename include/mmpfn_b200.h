@@ -223,6 +223,46 @@ int mmpfn_layers_run(const mmpfn_geometry* g, const mmpfn_weights* w, float* sta
                      const mmpfn_kv_segment* segs, int n_seg, int S, int n_train, int train, int layer_begin,
                      int layer_end, int phase, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- per-entry row counts ("ragged" passes) ------------------------------------------------------------------
+ * Independent tasks of different sizes share one pass.  A batch ENTRY is one (task, estimator) pair; a pass has a
+ * row capacity S (train pass: S train rows; test pass: S test rows against n_train context rows) and entry b uses
+ * its first n_rows[b] rows (test pass: attends to its first n_ctx[b] context rows).  The counts are device int32
+ * arrays with one element per entry (over all segments, in list order); NULL = every entry uses all rows, which runs
+ * exactly the kernels of mmpfn_layers_*_multi / mmpfn_layers_train / _test.
+ *
+ * Pad-row contract: the rows between an entry's count and the capacity must be ZERO when a kernel reads them.
+ * mmpfn_stem_tokens_ragged writes them as zeros, and the layers keep them exactly zero (no biases; LayerNorm of a
+ * zero row, GELU(0), attention over zero tokens are zero; the item attention writes zeros for pad queries), so the
+ * K/V rows a pad row produces are the zeros the TMA out-of-bounds fill gives an entry run alone: every entry's result
+ * is bit-identical to a pass over that entry alone. */
+
+/* mmpfn_stem_tab_fit (encoders.py:515, :461, :133-162, :53-99, :615-619) per entry: entry b's rows are the first
+ * n_rows[b] rows of its S-row block of x, train rows (n_train[b] of them) first; its statistics are those of a call
+ * over that entry alone (the reductions run in the same order). */
+int mmpfn_stem_tab_fit_ragged(const mmpfn_geometry* g, const float* x, int B, int S, int F, const int32_t* n_rows,
+                              const int32_t* n_train, float n_sigma, float* stats, void* stream);
+/* mmpfn_stem_tokens (transformer.py:682-788) per entry: rows s >= n_rows[b] of entry b are written as all zeros (no
+ * positional embedding, never a NaN flag; n_rows NULL = all S rows).  img_offset [B] (int64, elements; required with img_tok): entry b's
+ * [S][H_img][E] image tokens start at img_tok + img_offset[b] (estimators of one task share one set). */
+int mmpfn_stem_tokens_ragged(const mmpfn_geometry* g, const mmpfn_weights* w, const float* x, const float* stats,
+                             const float* img_tok, const float* y, const float* y_mean, const uint64_t* y_present_mask,
+                             const float* pos_emb, int B, int S, int F, int H_img, long long x_bstride,
+                             long long y_bstride, const int64_t* img_offset, const int32_t* n_rows, float* state_f32,
+                             uint16_t* state_bf16, int32_t* nan_flag, void* stream);
+/* The 12 layers over segments (layout of mmpfn_layers_train_multi: same S, own B_i and T_i, states back to back;
+ * kv[i] = segment i's context, mmpfn_kv_bytes(B_i, n_train, T_i, precision)) with per-entry counts, both precisions:
+ * layer.py:272-457 with the item attention (layer.py:341-379, multi_head_attention.py:436-445) of entry b over its
+ * own rows only.  bf16: the segments share the row-wise launches; fp32: one segment after another.
+ * state_bf16 is unused (may be NULL) in MMPFN_F32. */
+size_t mmpfn_layers_ragged_ws_bytes(const mmpfn_geometry* g, const mmpfn_segment* segs, int n_seg, int S, int precision);
+int mmpfn_layers_train_ragged(const mmpfn_geometry* g, const mmpfn_weights* w, float* state_f32, uint16_t* state_bf16,
+                              const mmpfn_segment* segs, int n_seg, int S, const int32_t* n_rows, int precision,
+                              void* const* kv, void* workspace, size_t workspace_bytes, void* stream);
+int mmpfn_layers_test_ragged(const mmpfn_geometry* g, const mmpfn_weights* w, float* state_f32, uint16_t* state_bf16,
+                             const mmpfn_segment* segs, int n_seg, int S, int n_train, const int32_t* n_rows,
+                             const int32_t* n_ctx, int precision, void* const* kv, void* workspace,
+                             size_t workspace_bytes, void* stream);
+
 /* ---- decoder + probability tail ------------------------------------------------------------ */
 /* transformer.py:392-396, :850-853: logits[b][s][:] = W2 gelu(W1 state[b][s][T-1] + b1) + b2.
  * state [B][S][T][E] -> logits [B][S][n_out]; hidden scratch [B*S][nhid] fp32. */
@@ -277,6 +317,18 @@ int mmpfn_mlp_bf16(float* state_f32, uint16_t* state_bf16, const uint16_t* w1, c
  * hold finite values — mmpfn_item_qkv_bf16 writes zeros there. */
 int mmpfn_item_attention_bf16(const uint16_t* q, const uint16_t* k, const uint16_t* vt, int B, int T, int n_q,
                               int Sq_pad, int n_kv, int Skv_pad, int shared_kv, uint16_t* out, void* stream);
+
+/* The same with per-entry counts (entry b = plane column / T): entry b attends over its first kv_len[b] keys
+ * (1..n_kv) and its output rows q_len[b] .. n_q-1 are zeros.  Key rows between kv_len[b] and n_kv must be zero. */
+int mmpfn_item_attention_bf16_ragged(const uint16_t* q, const uint16_t* k, const uint16_t* vt, int B, int T, int n_q,
+                                     int Sq_pad, int n_kv, int Skv_pad, int shared_kv, const int32_t* q_len,
+                                     const int32_t* kv_len, uint16_t* out, void* stream);
+/* Item-axis attention of the fp32 parity mode (layer.py:341-379), for unit tests:
+ *   q, out [B][n_q][T][nhead*32];  shared_kv = 0: k, v [B][n_kv][T][nhead*32];  shared_kv = 1 (every query head reads
+ *   head 0, multi_head_attention.py:436-445): k, v [B][T][n_kv][32].
+ * q_len / kv_len: per-entry counts as above, or NULL. */
+int mmpfn_item_attention_f32(const float* q, const float* k, const float* v, int B, int T, int n_q, int n_kv,
+                             int shared_kv, const int32_t* q_len, const int32_t* kv_len, float* out, void* stream);
 
 /* Feature-axis attention alone (layer.py:332-339: per table row, 6 heads over the row's T tokens, d = 32), bf16
  * tensor-core kernel, for unit tests and HBM-roofline timing.

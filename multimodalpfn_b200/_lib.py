@@ -13,6 +13,7 @@ from . import build as _build
 c_void_p, c_int, c_float, c_size_t, c_int64, c_ll = C.c_void_p, C.c_int, C.c_float, C.c_size_t, C.c_int64, C.c_longlong
 
 F32, BF16 = 0, 1
+MAX_SEGMENTS = 8          # MMPFN_MAX_SEGMENTS
 MIXER = {"none": 0, "MGM": 1, "MGM+CAP": 2, "MoE": 3}
 ERRORS = {-1: "EINVAL", -2: "ENODEVICE", -3: "ECUDA", -4: "EUNSUPPORTED"}
 
@@ -88,6 +89,20 @@ SIGNATURES = {
     "mmpfn_feature_qkv_attention_bf16": (c_int, [c_void_p, c_void_p, c_ll, c_int, c_void_p, c_void_p]),
     "mmpfn_item_attention_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int,
                                           c_int, c_void_p, c_void_p]),
+    "mmpfn_stem_tab_fit_ragged": (c_int, [PG, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_float, c_void_p,
+                                          c_void_p]),
+    "mmpfn_stem_tokens_ragged": (c_int, [PG, PW, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                         c_int, c_int, c_int, c_int, c_ll, c_ll, c_void_p, c_void_p, c_void_p, c_void_p,
+                                         c_void_p, c_void_p]),
+    "mmpfn_layers_ragged_ws_bytes": (c_size_t, [PG, PS, c_int, c_int, c_int]),
+    "mmpfn_layers_train_ragged": (c_int, [PG, PW, c_void_p, c_void_p, PS, c_int, c_int, c_void_p, c_int, PVP, c_void_p,
+                                          c_size_t, c_void_p]),
+    "mmpfn_layers_test_ragged": (c_int, [PG, PW, c_void_p, c_void_p, PS, c_int, c_int, c_int, c_void_p, c_void_p, c_int,
+                                         PVP, c_void_p, c_size_t, c_void_p]),
+    "mmpfn_item_attention_bf16_ragged": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int,
+                                                 c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "mmpfn_item_attention_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p,
+                                         c_void_p, c_void_p, c_void_p]),
 }
 
 _lib = None

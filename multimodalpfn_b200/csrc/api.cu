@@ -191,6 +191,17 @@ int mmpfn_stem_tab_fit(const mmpfn_geometry* g, const float* x, int B, int S, in
   return launch_tab_fit(x, B, S, F, g->features_per_group, n_train, n_sigma, stats, (cudaStream_t)stream);
 }
 
+int mmpfn_stem_tab_fit_ragged(const mmpfn_geometry* g, const float* x, int B, int S, int F, const int32_t* n_rows,
+                              const int32_t* n_train, float n_sigma, float* stats, void* stream) {
+  MMPFN_TRY(check_geometry(g));
+  MMPFN_TRY(require_device());
+  if (!x || !stats || !n_rows || !n_train || B < 1 || S < 1 || F < 1) {
+    set_error("stem_tab_fit_ragged: bad arguments (B %d S %d F %d)", B, S, F);
+    return MMPFN_EINVAL;
+  }
+  return launch_tab_fit(x, B, S, F, g->features_per_group, 0, n_sigma, stats, (cudaStream_t)stream, n_rows, n_train);
+}
+
 // image stem scratch (floats)
 struct ImgWs {
   float *xhat, *u, *src, *srcn, *kv, *o, *o2, *f1, *f2, *gl;
@@ -317,6 +328,23 @@ int mmpfn_stem_tokens(const mmpfn_geometry* g, const mmpfn_weights* w, const flo
                             x_bstride, y_bstride, img_bstride, state_f32, state_bf16, nan_flag, (cudaStream_t)stream);
 }
 
+int mmpfn_stem_tokens_ragged(const mmpfn_geometry* g, const mmpfn_weights* w, const float* x, const float* stats,
+                             const float* img_tok, const float* y, const float* y_mean, const uint64_t* y_present_mask,
+                             const float* pos_emb, int B, int S, int F, int H_img, long long x_bstride,
+                             long long y_bstride, const int64_t* img_offset, const int32_t* n_rows, float* state_f32,
+                             uint16_t* state_bf16, int32_t* nan_flag, void* stream) {
+  MMPFN_TRY(check_geometry(g));
+  MMPFN_TRY(require_device());
+  if (!w || !y || !y_mean || !y_present_mask || !pos_emb || !state_f32 || !nan_flag || B < 1 || S < 1 ||
+      (x && (!stats || F < 1)) || (!x && !img_tok) || (img_tok && (H_img < 1 || !img_offset)) || (!img_tok && H_img != 0)) {
+    set_error("stem_tokens_ragged: bad arguments");
+    return MMPFN_EINVAL;
+  }
+  return launch_stem_tokens(g, w, x, stats, img_tok, y, y_mean, y_present_mask, pos_emb, B, S, x ? F : 0, H_img,
+                            x_bstride, y_bstride, 0, state_f32, state_bf16, nan_flag, (cudaStream_t)stream,
+                            (const long long*)img_offset, n_rows);
+}
+
 size_t mmpfn_layers_ws_bytes(const mmpfn_geometry* g, int B, int S, int T, int precision) {
   if (check_geometry(g) != MMPFN_OK) return 0;
   return carve(nullptr, (long long)B * S * T, B, S, T, precision).bytes;
@@ -415,7 +443,47 @@ static int check_layers_args(const mmpfn_geometry* g, const mmpfn_weights* w, fl
 
 static int layers_run(const mmpfn_geometry* g, const mmpfn_weights* w, float* state, uint16_t* state_b,
                       const mmpfn_kv_segment* ks, int n_seg, int S, int n_train, int train, int layer_begin,
-                      int layer_end, int phase, void* workspace, size_t workspace_bytes, cudaStream_t st);
+                      int layer_end, int phase, void* workspace, size_t workspace_bytes, cudaStream_t st,
+                      const int* n_rows = nullptr, const int* n_ctx = nullptr);
+
+// The fp32 (parity mode) passes over one [B][S][T] state.  train != 0: self-attention over the S rows, head-0 K/V
+// written to kv (may be NULL); else the S rows attend to the n_train rows of the context kv.  n_rows / n_ctx (device
+// [B], or NULL = S / n_train): entry b's own row count in this pass and context rows of the test pass.
+static int layers_f32(const mmpfn_geometry* g, const mmpfn_weights* w, float* state, int B, int S, int T, int n_train,
+                      int train, void* kv, const int* n_rows, const int* n_ctx, const LayerWs& ws, cudaStream_t st) {
+  const long long M = (long long)B * S * T;
+  for (int l = 0; l < g->nlayers; ++l) {
+    const LayerW lw = layer_w(w, l);
+    MMPFN_TRY(feature_attention(lw, state, nullptr, M, (long long)B * S, T, MMPFN_F32, ws, st));
+    ItemAttnF32 a{};
+    a.out = ws.att;
+    a.o_outer = (long long)S * T * kE; a.o_inner = kE; a.o_row = (long long)T * kE;
+    a.planes = B * T; a.inner = T; a.n_q = S; a.q_len = n_rows;
+    if (train) {
+      MMPFN_TRY(launch_sgemm(gemm(state, kE, lw.iqkv, kE, nullptr, ws.qkv, 3 * kE, (int)M, 3 * kE, kE), EPI_NONE, st));
+      if (kv) {
+        float* kvl = (float*)kv + (size_t)l * B * T * S * 2 * kD;
+        MMPFN_TRY(launch_kv_extract_f32(ws.qkv, kvl, B, S, T, st, n_rows));
+      }
+      a.q = ws.qkv; a.k = ws.qkv + kE; a.v = ws.qkv + 2 * kE;
+      a.q_outer = (long long)S * T * 3 * kE; a.q_inner = 3 * kE; a.q_row = (long long)T * 3 * kE;
+      a.kv_outer = a.q_outer; a.kv_inner = a.q_inner; a.kv_row = a.q_row;
+      a.n_kv = S; a.shared_kv = 0; a.kv_len = n_rows;
+    } else {
+      // queries only (multi_head_attention.py:432-434); K/V come from the context
+      MMPFN_TRY(launch_sgemm(gemm(state, kE, lw.iqkv, kE, nullptr, ws.qkv, kE, (int)M, kE, kE), EPI_NONE, st));
+      const float* kvl = (const float*)kv + (size_t)l * B * T * n_train * 2 * kD;
+      a.q = ws.qkv; a.k = kvl; a.v = kvl + kD;
+      a.q_outer = (long long)S * T * kE; a.q_inner = kE; a.q_row = (long long)T * kE;
+      a.kv_outer = (long long)T * n_train * 2 * kD; a.kv_inner = (long long)n_train * 2 * kD; a.kv_row = 2 * kD;
+      a.n_kv = n_train; a.shared_kv = 1; a.kv_len = n_ctx;
+    }
+    MMPFN_TRY(launch_item_attn_f32(a, st));
+    MMPFN_TRY(out_proj_ln(lw, state, nullptr, M, MMPFN_F32, ws, st));
+    MMPFN_TRY(mlp(lw, state, nullptr, M, MMPFN_F32, ws, st));
+  }
+  return MMPFN_OK;
+}
 
 int mmpfn_layers_train(const mmpfn_geometry* g, const mmpfn_weights* w, float* state, uint16_t* state_b, int B, int S,
                        int T, int precision, void* kv, void* workspace, size_t workspace_bytes, void* stream) {
@@ -427,28 +495,7 @@ int mmpfn_layers_train(const mmpfn_geometry* g, const mmpfn_weights* w, float* s
     k.B = B; k.T = T; k.kv = kv;
     return layers_run(g, w, state, state_b, &k, 1, S, 0, 1, 0, g->nlayers, 0, workspace, workspace_bytes, st);
   }
-  const long long M = (long long)B * S * T;
-  for (int l = 0; l < g->nlayers; ++l) {
-    const LayerW lw = layer_w(w, l);
-    MMPFN_TRY(feature_attention(lw, state, state_b, M, (long long)B * S, T, precision, ws, st));
-    {
-      MMPFN_TRY(launch_sgemm(gemm(state, kE, lw.iqkv, kE, nullptr, ws.qkv, 3 * kE, (int)M, 3 * kE, kE), EPI_NONE, st));
-      if (kv) {
-        float* kvl = (float*)kv + (size_t)l * B * T * S * 2 * kD;
-        MMPFN_TRY(launch_kv_extract_f32(ws.qkv, kvl, B, S, T, st));
-      }
-      ItemAttnF32 a{};
-      a.q = ws.qkv; a.k = ws.qkv + kE; a.v = ws.qkv + 2 * kE; a.out = ws.att;
-      a.q_outer = (long long)S * T * 3 * kE; a.q_inner = 3 * kE; a.q_row = (long long)T * 3 * kE;
-      a.kv_outer = a.q_outer; a.kv_inner = a.q_inner; a.kv_row = a.q_row;
-      a.o_outer = (long long)S * T * kE; a.o_inner = kE; a.o_row = (long long)T * kE;
-      a.planes = B * T; a.inner = T; a.n_q = S; a.n_kv = S; a.shared_kv = 0;
-      MMPFN_TRY(launch_item_attn_f32(a, st));
-    }
-    MMPFN_TRY(out_proj_ln(lw, state, state_b, M, precision, ws, st));
-    MMPFN_TRY(mlp(lw, state, state_b, M, precision, ws, st));
-  }
-  return MMPFN_OK;
+  return layers_f32(g, w, state, B, S, T, 0, 1, kv, nullptr, nullptr, ws, st);
 }
 
 int mmpfn_layers_test(const mmpfn_geometry* g, const mmpfn_weights* w, float* state, uint16_t* state_b, int B, int S,
@@ -463,26 +510,7 @@ int mmpfn_layers_test(const mmpfn_geometry* g, const mmpfn_weights* w, float* st
     k.B = B; k.T = T; k.kv = const_cast<void*>(kv);
     return layers_run(g, w, state, state_b, &k, 1, S, n_train, 0, 0, g->nlayers, 0, workspace, workspace_bytes, st);
   }
-  const long long M = (long long)B * S * T;
-  for (int l = 0; l < g->nlayers; ++l) {
-    const LayerW lw = layer_w(w, l);
-    MMPFN_TRY(feature_attention(lw, state, state_b, M, (long long)B * S, T, precision, ws, st));
-    {
-      // queries only (multi_head_attention.py:432-434); K/V come from the context
-      MMPFN_TRY(launch_sgemm(gemm(state, kE, lw.iqkv, kE, nullptr, ws.qkv, kE, (int)M, kE, kE), EPI_NONE, st));
-      const float* kvl = (const float*)kv + (size_t)l * B * T * n_train * 2 * kD;
-      ItemAttnF32 a{};
-      a.q = ws.qkv; a.k = kvl; a.v = kvl + kD; a.out = ws.att;
-      a.q_outer = (long long)S * T * kE; a.q_inner = kE; a.q_row = (long long)T * kE;
-      a.kv_outer = (long long)T * n_train * 2 * kD; a.kv_inner = (long long)n_train * 2 * kD; a.kv_row = 2 * kD;
-      a.o_outer = (long long)S * T * kE; a.o_inner = kE; a.o_row = (long long)T * kE;
-      a.planes = B * T; a.inner = T; a.n_q = S; a.n_kv = n_train; a.shared_kv = 1;
-      MMPFN_TRY(launch_item_attn_f32(a, st));
-    }
-    MMPFN_TRY(out_proj_ln(lw, state, state_b, M, precision, ws, st));
-    MMPFN_TRY(mlp(lw, state, state_b, M, precision, ws, st));
-  }
-  return MMPFN_OK;
+  return layers_f32(g, w, state, B, S, T, n_train, 0, const_cast<void*>(kv), nullptr, nullptr, ws, st);
 }
 
 // ---- several estimator groups (segments) in one call -------------------------------------------------
@@ -542,9 +570,12 @@ static size_t kv_block_elems(int c, int T, int n_pad) { return (size_t)2 * c * T
 
 // train != 0: self-attention over the S rows, head-0 K/V written to segs[i].kv (may be NULL);
 // train == 0: the S rows are test rows attending to the n_train rows' context segs[i].kv
+// n_rows / n_ctx (device, one entry per estimator of every segment in list order, or NULL): per-entry row counts of
+// this pass and context rows of the test pass (mmpfn_layers_*_ragged)
 static int layers_run(const mmpfn_geometry* g, const mmpfn_weights* w, float* state, uint16_t* state_b,
                       const mmpfn_kv_segment* ks, int n_seg, int S, int n_train, int train, int layer_begin,
-                      int layer_end, int phase, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+                      int layer_end, int phase, void* workspace, size_t workspace_bytes, cudaStream_t st,
+                      const int* n_rows, const int* n_ctx) {
   MMPFN_TRY(check_geometry(g));
   MMPFN_TRY(require_device());
   if (!ks || n_seg < 1 || n_seg > MMPFN_MAX_SEGMENTS) { set_error("layers_run: bad segment list"); return MMPFN_EINVAL; }
@@ -610,7 +641,7 @@ static int layers_run(const mmpfn_geometry* g, const mmpfn_weights* w, float* st
     }
     // items: QKV scatter + attention per segment (tiles follow T_i), out-projection + LN over all
     {
-      long long off = 0;
+      long long off = 0, entry = 0;
       for (int i = 0; i < n_seg; ++i) {
         const int B = segs[i].B, T = segs[i].T;
         TcGemm q{};
@@ -618,6 +649,8 @@ static int layers_run(const mmpfn_geometry* g, const mmpfn_weights* w, float* st
         q.epi = TC_EPI_QKV_ITEMS; q.q_out = ws.seg[i].qi; q.S_pad = Sp;
         TcItemAttn a{};
         a.q = ws.seg[i].qi; a.out = ws.att_b + off * kE; a.B = B; a.T = T; a.n_q = S; a.Sq_pad = Sp;
+        a.q_len = n_rows ? n_rows + entry : nullptr;
+        a.kv_len = train ? a.q_len : (n_ctx ? n_ctx + entry : nullptr);
         const bool rows_mode = train && ks[i].seg_rows > 0;
         if (rows_mode) {
           // row-sharded build: this rank's K / V^T planes go into its chunk of the gather buffers; after the
@@ -661,6 +694,7 @@ static int layers_run(const mmpfn_geometry* g, const mmpfn_weights* w, float* st
         if (phase != 2) MMPFN_TRY(proj_gemm(q, st));
         if (phase != 1) MMPFN_TRY(launch_tc_item_attn(a, st));
         off += (long long)B * S * T;
+        entry += B;
       }
       if (phase != 1) MMPFN_TRY(out_proj_ln(lw, state, state_b, M, MMPFN_BF16, flat, st));
     }
@@ -698,6 +732,72 @@ int mmpfn_layers_run(const mmpfn_geometry* g, const mmpfn_weights* w, float* sta
                      int layer_end, int phase, void* workspace, size_t workspace_bytes, void* stream) {
   return layers_run(g, w, state_f32, state_bf16, segs, n_seg, S, n_train, train, layer_begin, layer_end, phase, workspace,
                     workspace_bytes, (cudaStream_t)stream);
+}
+
+// ---- per-entry row counts ----------------------------------------------------------------------------
+size_t mmpfn_layers_ragged_ws_bytes(const mmpfn_geometry* g, const mmpfn_segment* segs, int n_seg, int S, int precision) {
+  long long M = 0;
+  if (check_geometry(g) != MMPFN_OK || check_segments(segs, n_seg, S, &M) != MMPFN_OK) return 0;
+  if (precision == MMPFN_BF16) return carve_multi(nullptr, segs, n_seg, S, M).bytes;
+  if (precision != MMPFN_F32) return 0;
+  long long m_max = 0;         // fp32: one segment after another
+  for (int i = 0; i < n_seg; ++i) {
+    const long long m = (long long)segs[i].B * S * segs[i].T;
+    if (m > m_max) m_max = m;
+  }
+  return carve(nullptr, m_max, 1, S, 2, MMPFN_F32).bytes;
+}
+
+static int layers_ragged(const mmpfn_geometry* g, const mmpfn_weights* w, float* state, uint16_t* state_b,
+                         const mmpfn_segment* segs, int n_seg, int S, int n_train, int train, const int* n_rows,
+                         const int* n_ctx, int precision, void* const* kv, void* workspace, size_t workspace_bytes,
+                         cudaStream_t st) {
+  MMPFN_TRY(check_geometry(g));
+  MMPFN_TRY(require_device());
+  long long M = 0;
+  if (!kv) { set_error("layers_ragged: null context list"); return MMPFN_EINVAL; }
+  MMPFN_TRY(check_segments(segs, n_seg, S, &M));
+  if (!train && n_train < 1) { set_error("layers_ragged: the test pass needs n_train >= 1"); return MMPFN_EINVAL; }
+  if (precision == MMPFN_BF16) {
+    mmpfn_kv_segment ks[MMPFN_MAX_SEGMENTS];
+    for (int i = 0; i < n_seg; ++i) {
+      ks[i] = mmpfn_kv_segment{};
+      ks[i].B = segs[i].B; ks[i].T = segs[i].T; ks[i].kv = kv[i];
+    }
+    return layers_run(g, w, state, state_b, ks, n_seg, S, n_train, train, 0, g->nlayers, 0, workspace, workspace_bytes,
+                      st, n_rows, n_ctx);
+  }
+  if (precision != MMPFN_F32 || !w || !w->layers_f32 || !state) { set_error("layers_ragged: bad arguments"); return MMPFN_EINVAL; }
+  if (workspace_bytes < mmpfn_layers_ragged_ws_bytes(g, segs, n_seg, S, precision) || !workspace) {
+    set_error("layers_ragged: workspace %zu bytes too small", workspace_bytes);
+    return MMPFN_EINVAL;
+  }
+  long long off = 0, entry = 0;
+  for (int i = 0; i < n_seg; ++i) {
+    const int B = segs[i].B, T = segs[i].T;
+    if (!train && !kv[i]) { set_error("layers_ragged: the test pass needs every segment's context"); return MMPFN_EINVAL; }
+    const LayerWs ws = carve(workspace, (long long)B * S * T, B, S, T, MMPFN_F32);
+    MMPFN_TRY(layers_f32(g, w, state + off * kE, B, S, T, n_train, train, kv[i], n_rows ? n_rows + entry : nullptr,
+                         n_ctx ? n_ctx + entry : nullptr, ws, st));
+    off += (long long)B * S * T;
+    entry += B;
+  }
+  return MMPFN_OK;
+}
+
+int mmpfn_layers_train_ragged(const mmpfn_geometry* g, const mmpfn_weights* w, float* state_f32, uint16_t* state_bf16,
+                              const mmpfn_segment* segs, int n_seg, int S, const int32_t* n_rows, int precision,
+                              void* const* kv, void* workspace, size_t workspace_bytes, void* stream) {
+  return layers_ragged(g, w, state_f32, state_bf16, segs, n_seg, S, 0, 1, n_rows, nullptr, precision, kv, workspace,
+                       workspace_bytes, (cudaStream_t)stream);
+}
+
+int mmpfn_layers_test_ragged(const mmpfn_geometry* g, const mmpfn_weights* w, float* state_f32, uint16_t* state_bf16,
+                             const mmpfn_segment* segs, int n_seg, int S, int n_train, const int32_t* n_rows,
+                             const int32_t* n_ctx, int precision, void* const* kv, void* workspace,
+                             size_t workspace_bytes, void* stream) {
+  return layers_ragged(g, w, state_f32, state_bf16, segs, n_seg, S, n_train, 0, n_rows, n_ctx, precision, kv, workspace,
+                       workspace_bytes, (cudaStream_t)stream);
 }
 
 int mmpfn_decode(const mmpfn_geometry* g, const mmpfn_weights* w, const float* state, int B, int S, int T,
@@ -797,6 +897,42 @@ int mmpfn_item_attention_bf16(const uint16_t* q, const uint16_t* k, const uint16
   a.q = q; a.k = k; a.vt = vt; a.out = out; a.B = B; a.T = T; a.n_q = n_q; a.Sq_pad = Sq_pad; a.n_kv = n_kv;
   a.Skv_pad = Skv_pad; a.shared_kv = shared_kv;
   return launch_tc_item_attn(a, (cudaStream_t)stream);
+}
+
+int mmpfn_item_attention_bf16_ragged(const uint16_t* q, const uint16_t* k, const uint16_t* vt, int B, int T, int n_q,
+                                     int Sq_pad, int n_kv, int Skv_pad, int shared_kv, const int32_t* q_len,
+                                     const int32_t* kv_len, uint16_t* out, void* stream) {
+  MMPFN_TRY(require_device());
+  if (!q || !k || !vt || !out || !q_len || !kv_len || B < 1 || T < 1 || n_q < 1 || n_kv < 1 || Sq_pad < n_q ||
+      Skv_pad < n_kv || Sq_pad % 8 || Skv_pad % 8) {
+    set_error("item_attention_bf16_ragged: bad arguments");
+    return MMPFN_EINVAL;
+  }
+  TcItemAttn a{};
+  a.q = q; a.k = k; a.vt = vt; a.out = out; a.B = B; a.T = T; a.n_q = n_q; a.Sq_pad = Sq_pad; a.n_kv = n_kv;
+  a.Skv_pad = Skv_pad; a.shared_kv = shared_kv; a.q_len = q_len; a.kv_len = kv_len;
+  return launch_tc_item_attn(a, (cudaStream_t)stream);
+}
+
+int mmpfn_item_attention_f32(const float* q, const float* k, const float* v, int B, int T, int n_q, int n_kv,
+                             int shared_kv, const int32_t* q_len, const int32_t* kv_len, float* out, void* stream) {
+  MMPFN_TRY(require_device());
+  if (!q || !k || !v || !out || B < 1 || T < 1 || n_q < 1 || n_kv < 1) {
+    set_error("item_attention_f32: bad arguments");
+    return MMPFN_EINVAL;
+  }
+  ItemAttnF32 a{};
+  a.q = q; a.k = k; a.v = v; a.out = out;
+  a.q_outer = (long long)n_q * T * kE; a.q_inner = kE; a.q_row = (long long)T * kE;
+  a.o_outer = a.q_outer; a.o_inner = kE; a.o_row = a.q_row;
+  if (shared_kv) {
+    a.kv_outer = (long long)T * n_kv * kD; a.kv_inner = (long long)n_kv * kD; a.kv_row = kD;
+  } else {
+    a.kv_outer = (long long)n_kv * T * kE; a.kv_inner = kE; a.kv_row = (long long)T * kE;
+  }
+  a.planes = B * T; a.inner = T; a.n_q = n_q; a.n_kv = n_kv; a.shared_kv = shared_kv ? 1 : 0;
+  a.q_len = q_len; a.kv_len = kv_len;
+  return launch_item_attn_f32(a, (cudaStream_t)stream);
 }
 
 int mmpfn_feature_attention_bf16(const uint16_t* qkv, uint16_t* att, long long n_rows, int T, void* stream) {

@@ -118,8 +118,9 @@ int launch_sgemm(const SgemmParams& p, int epi, cudaStream_t st);
 // x_stride: elements between consecutive input rows (0 = width).
 int launch_layernorm(const float* x, const float* res, const float* gamma, const float* beta, long long rows,
                      int width, float* y_f32, uint16_t* y_bf16, cudaStream_t st, long long x_stride = 0);
-// copy head-0 k|v of the item-attention qkv buffer [B][S][T][3E] into the fp32 context [B][T][S][2][kD]
-int launch_kv_extract_f32(const float* qkv, float* kv, int B, int S, int T, cudaStream_t st);
+// copy head-0 k|v of the item-attention qkv buffer [B][S][T][3E] into the fp32 context [B][T][S][2][kD]; with
+// n_rows (device [B]) the rows s >= n_rows[b] are written as zeros instead
+int launch_kv_extract_f32(const float* qkv, float* kv, int B, int S, int T, cudaStream_t st, const int* n_rows = nullptr);
 
 // attention between features: qkv [rows = n_seq*T][3*kE] (q|k|v, head-major) -> att [rows][kE]
 int launch_feat_attn_f32(const float* qkv, float* att, long long n_seq, int T, cudaStream_t st);
@@ -138,6 +139,9 @@ struct ItemAttnF32 {
   float* out;
   long long q_outer, q_inner, q_row, kv_outer, kv_inner, kv_row, o_outer, o_inner, o_row;
   int planes, inner, n_q, n_kv, shared_kv;
+  // per-entry counts (device int32 [planes / inner], or NULL): entry b attends over its first kv_len[b] keys, its
+  // query rows q_len[b] .. n_q-1 are written as zeros; rows past an entry's counts are never read
+  const int *q_len, *kv_len;
 };
 int launch_item_attn_f32(const ItemAttnF32& p, cudaStream_t st);
 
@@ -197,6 +201,11 @@ struct TcItemAttn {
   // planes are laid out as usual with Skv_pad allocated rows.  0 = one contiguous row range.
   int kv_seg_rows;
   long long kv_seg_stride;
+  // per-entry counts (device int32 [B], or NULL = n_q / n_kv for every entry): entry b attends over its first
+  // kv_len[b] keys (1..n_kv); its output rows q_len[b] .. n_q-1 are written as zeros.  Key rows between an entry's
+  // count and n_kv that its last tile covers must be zero (what the TMA out-of-bounds fill gives an entry run alone).
+  const int* q_len;
+  const int* kv_len;
 };
 int launch_tc_item_attn(const TcItemAttn& p, cudaStream_t st);
 
@@ -214,12 +223,17 @@ struct TabStatsLayout {
   __host__ __device__ int scale() const { return 6 * Fp; }
   __host__ __device__ int total() const { return 6 * Fp + G; }
 };
+// n_rows / n_train_b (device [B], or NULL = S / n_train): entry b's statistics over its first n_rows[b] rows, of
+// which the first n_train_b[b] are train rows
 int launch_tab_fit(const float* x, int B, int S, int F, int fpg, int n_train, float n_sigma, float* stats,
-                   cudaStream_t st);
+                   cudaStream_t st, const int* n_rows = nullptr, const int* n_train_b = nullptr);
+// img_off (device [B], elements, or NULL = b * img_bstride): where entry b's image tokens start;
+// n_rows (device [B], or NULL = S): rows s >= n_rows[b] are written as zeros
 int launch_stem_tokens(const mmpfn_geometry* g, const mmpfn_weights* w, const float* x, const float* stats,
                        const float* img_tok, const float* y, const float* y_mean, const uint64_t* y_mask,
                        const float* pos_emb, int B, int S, int F, int H_img, long long x_bstride, long long y_bstride,
-                       long long img_bstride, float* state_f32, uint16_t* state_bf16, int32_t* nan_flag, cudaStream_t st);
+                       long long img_bstride, float* state_f32, uint16_t* state_bf16, int32_t* nan_flag, cudaStream_t st,
+                       const long long* img_off = nullptr, const int* n_rows = nullptr);
 int launch_cap_attn(const float* kv, const float* q, int S, int n_kv, int Hc, float* out, cudaStream_t st);
 int launch_cap_combine(const float* o, const float* ffn, const float* gamma, const float* beta, long long rows,
                        float* out, cudaStream_t st);

@@ -80,6 +80,9 @@ struct AttnArgs {
   int stack_rows;   // > 0: the six query heads of a (b, t) column are stacked on the tile's row axis, Sq_pad rows each
   int kv_slots;     // shared_kv: estimators per rank chunk of the K/V context (>= 1; B when the context is dense)
   int tiles_per_seg;   // key tiles per row segment (row-sharded context: keys stored in per-rank chunks); 2^30 = one range
+  // per-entry counts (the RAGGED instantiation only; entry = bt / T): query rows and keys of entry b, or NULL = n_q / n_kv
+  const int* q_len;
+  const int* kv_len;
 };
 
 #ifdef MMPFN_DEBUG
@@ -249,7 +252,10 @@ __device__ __forceinline__ void tmem_st_cols(uint32_t taddr, const uint32_t* v) 
 //   warps 0-3  softmax, thread = query row (TMEM lane quarter = warp)
 //   warp 4     TMA producer + TMEM allocation
 //   warp 5     MMA issue
-template <int BK, int PP>
+// RAGGED: entry b has its own key count kv_len[b] (tiles past it are not visited; its last tile is masked like the
+// tail tile) and query count q_len[b] (output rows from there up to n_q are written as zeros; a tile holding only
+// such rows stores its zeros and issues nothing else).  The other instantiation is the one the layer passes use.
+template <int BK, int PP, bool RAGGED>
 __global__ void __launch_bounds__(A_THREADS, AttnCfg<BK>::kMinCtas)
     tc_item_attn_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                         const __grid_constant__ CUtensorMap map_vt, const AttnArgs p) {
@@ -276,7 +282,33 @@ __global__ void __launch_bounds__(A_THREADS, AttnCfg<BK>::kMinCtas)
   const int kc2 = p.shared_kv ? bt - kb * p.T : plane;
   const int kc3 = p.shared_kv ? kb % p.kv_slots : 0;
   const int kc4 = p.shared_kv ? kb / p.kv_slots : 0;
-  const int nkt = (p.n_kv + BK - 1) / BK;
+  int n_kv = p.n_kv, n_q = p.n_q;
+  if constexpr (RAGGED) {
+    if (p.kv_len) n_kv = min(max(p.kv_len[kb], 1), p.n_kv);
+    if (p.q_len) n_q = min(max(p.q_len[kb], 0), p.n_q);
+    // does the tile hold a row of this entry (stacked: of any head)?
+    bool live = q0 < n_q;
+    if (p.stack_rows) {
+      live = false;
+      for (int hh = 0; hh < kH; ++hh) live |= hh * p.stack_rows < q0 + A_BQ && hh * p.stack_rows + n_q > q0;
+    }
+    if (!live) {
+      if (threadIdx.x < A_BQ) {
+        int qi = q0 + threadIdx.x, hh = h;
+        if (p.stack_rows) {
+          hh = qi / p.stack_rows;
+          qi = hh < kH ? qi - hh * p.stack_rows : p.n_q;
+        }
+        if (qi < p.n_q) {
+          uint4* d4 = reinterpret_cast<uint4*>(p.out + (((long long)kb * p.n_q + qi) * p.T + (bt - kb * p.T)) * kE + hh * kD);
+#pragma unroll
+          for (int i = 0; i < 4; ++i) d4[i] = make_uint4(0, 0, 0, 0);
+        }
+      }
+      return;
+    }
+  }
+  const int nkt = (n_kv + BK - 1) / BK;
 
   if (threadIdx.x == 0) {
     prefetch_tmap(&map_q);
@@ -387,7 +419,7 @@ __global__ void __launch_bounds__(A_THREADS, AttnCfg<BK>::kMinCtas)
     for (int j = 0; j < nkt; ++j) {
       const int sb = j & 1;
       const uint32_t tmem_s = tmem + sb * BK + lane_off;
-      const int valid = p.n_kv - j * BK;         // keys of this tile that exist
+      const int valid = n_kv - j * BK;           // keys of this tile that exist
       // S(j) is in TMEM (and P V(j-2) has drained buffer sb).  Usually the probe made at the end of the
       // previous tile has already said so.
       if (threadIdx.x == 0) ATTN_TRACE(j * 8 + 0);
@@ -528,7 +560,14 @@ __global__ void __launch_bounds__(A_THREADS, AttnCfg<BK>::kMinCtas)
       qi = hh < kH ? qi - hh * p.stack_rows : p.n_q;      // rows past the last head: nothing to store
     }
     if (qi < p.n_q) {
-      const float inv = 1.0f / l_run;
+      float inv = 1.0f / l_run;
+      if constexpr (RAGGED) {
+        if (qi >= n_q) {                         // a pad row of this entry
+          inv = 0.f;
+#pragma unroll
+          for (int i = 0; i < 32; ++i) v[i] = 0u;
+        }
+      }
       const int b = bt / p.T, t = bt % p.T;
       uint16_t* dst = p.out + (((long long)b * p.n_q + qi) * p.T + t) * kE + hh * kD;
       uint4* d4 = reinterpret_cast<uint4*>(dst);
@@ -548,12 +587,12 @@ __global__ void __launch_bounds__(A_THREADS, AttnCfg<BK>::kMinCtas)
   }
 }
 
-template <int BK, int PP>
+template <int BK, int PP, bool RAGGED = false>
 int launch_attn_t(const CUtensorMap& mq, const CUtensorMap& mk, const CUtensorMap& mvt, const AttnArgs& a, dim3 grid,
                   cudaStream_t st) {
   using C = AttnCfg<BK>;
-  MMPFN_OPT_IN_SMEM((tc_item_attn_kernel<BK, PP>), C::kSmem);
-  tc_item_attn_kernel<BK, PP><<<grid, A_THREADS, C::kSmem, st>>>(mq, mk, mvt, a);
+  MMPFN_OPT_IN_SMEM((tc_item_attn_kernel<BK, PP, RAGGED>), C::kSmem);
+  tc_item_attn_kernel<BK, PP, RAGGED><<<grid, A_THREADS, C::kSmem, st>>>(mq, mk, mvt, a);
   return count_launch();
 }
 
@@ -617,8 +656,9 @@ int launch_tc_item_attn(const TcItemAttn& p, cudaStream_t st) {
     const cuuint32_t box[5] = {64, kD, 1, 1, 1};
     MMPFN_TRY(encode_map(&mvt, p.vt, 5, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B));
   }
-  AttnArgs a{p.out, p.T, p.n_q, p.n_kv, p.shared_kv, q_tiles, stack ? p.Sq_pad : 0, slots, tiles_per_seg};
+  AttnArgs a{p.out, p.T, p.n_q, p.n_kv, p.shared_kv, q_tiles, stack ? p.Sq_pad : 0, slots, tiles_per_seg, p.q_len, p.kv_len};
   const dim3 grid((unsigned)(grid_planes * q_tiles));
+  if (p.q_len || p.kv_len) return launch_attn_t<BK, kPolyPairsDefault, true>(mq, mk, mvt, a, grid, st);
 #ifdef MMPFN_DEBUG
   // tuning builds only (-DMMPFN_DEBUG): MMPFN_ATTN_PP = polynomial pairs of every 24.  The product
   // library has exactly one variant and reads no environment variable.

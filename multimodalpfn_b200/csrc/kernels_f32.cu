@@ -409,13 +409,25 @@ __global__ void __launch_bounds__(128) item_attn_f32_kernel(ItemAttnF32 p) {
   const int hk = p.shared_kv ? 0 : h;
   const float* kb = p.k + pb * p.kv_outer + pt * p.kv_inner + hk * kD;
   const float* vb = p.v + pb * p.kv_outer + pt * p.kv_inner + hk * kD;
+  // this entry's own counts: its keys past n_kv are never read, its query rows from n_q on are written as zeros
+  const int n_q = p.q_len ? min(max(p.q_len[pb], 0), p.n_q) : p.n_q;
+  const int n_kv = p.kv_len ? min(max(p.kv_len[pb], 1), p.n_kv) : p.n_kv;
+  if (q0 >= n_q) {
+    for (int i = tid; i < IQ * (kD / 4); i += 128) {
+      const int r = q0 + (i >> 3), c4 = (i & 7) * 4;
+      if (r < p.n_q)
+        *reinterpret_cast<float4*>(p.out + pb * p.o_outer + pt * p.o_inner + (long long)r * p.o_row + h * kD + c4) =
+            make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+    return;
+  }
 
   // Q tile -> Qt (transposed), pre-scaled by 1/sqrt(d)
   const float scale = 0.17677669529663687f;
   for (int i = tid; i < IQ * (kD / 4); i += 128) {
     const int r = i >> 3, c4 = (i & 7) * 4;
     float4 v = make_float4(0, 0, 0, 0);
-    if (q0 + r < p.n_q) v = *reinterpret_cast<const float4*>(qb + (long long)(q0 + r) * p.q_row + c4);
+    if (q0 + r < n_q) v = *reinterpret_cast<const float4*>(qb + (long long)(q0 + r) * p.q_row + c4);
     Qt[c4 + 0][r] = v.x * scale; Qt[c4 + 1][r] = v.y * scale; Qt[c4 + 2][r] = v.z * scale; Qt[c4 + 3][r] = v.w * scale;
   }
   float m[4], l[4], o[4][4];
@@ -427,12 +439,12 @@ __global__ void __launch_bounds__(128) item_attn_f32_kernel(ItemAttnF32 p) {
     for (int j = 0; j < 4; ++j) o[i][j] = 0.f;
   }
 
-  for (int k0 = 0; k0 < p.n_kv; k0 += IK) {
+  for (int k0 = 0; k0 < n_kv; k0 += IK) {
     __syncthreads();   // previous tile fully consumed (also orders the Qt stores the first time)
     for (int i = tid; i < IK * (kD / 4); i += 128) {
       const int r = i >> 3, c4 = (i & 7) * 4;
       float4 kv = make_float4(0, 0, 0, 0), vv = kv;
-      if (k0 + r < p.n_kv) {
+      if (k0 + r < n_kv) {
         kv = *reinterpret_cast<const float4*>(kb + (long long)(k0 + r) * p.kv_row + c4);
         vv = *reinterpret_cast<const float4*>(vb + (long long)(k0 + r) * p.kv_row + c4);
       }
@@ -464,7 +476,7 @@ __global__ void __launch_bounds__(128) item_attn_f32_kernel(ItemAttnF32 p) {
       float mx = -INFINITY;
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
-        if (k0 + tx * 8 + j >= p.n_kv) s[i][j] = -INFINITY;
+        if (k0 + tx * 8 + j >= n_kv) s[i][j] = -INFINITY;
         mx = fmaxf(mx, s[i][j]);
       }
       mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 1));
@@ -510,14 +522,15 @@ __global__ void __launch_bounds__(128) item_attn_f32_kernel(ItemAttnF32 p) {
     if (r >= p.n_q) continue;
     const float inv = 1.0f / l[i];
     float* dst = p.out + pb * p.o_outer + pt * p.o_inner + (long long)r * p.o_row + h * kD + tx * 4;
-    *reinterpret_cast<float4*>(dst) = make_float4(o[i][0] * inv, o[i][1] * inv, o[i][2] * inv, o[i][3] * inv);
+    *reinterpret_cast<float4*>(dst) = r < n_q ? make_float4(o[i][0] * inv, o[i][1] * inv, o[i][2] * inv, o[i][3] * inv)
+                                              : make_float4(0.f, 0.f, 0.f, 0.f);
   }
 }
 }  // namespace
 
 namespace {
 __global__ void kv_extract_f32_kernel(const float* __restrict__ qkv, float* __restrict__ kv, int S, int T,
-                                      long long n) {
+                                      long long n, const int* __restrict__ n_rows) {
   // one thread per (b, t, s, 64 floats): k (32) | v (32) of head 0
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
@@ -525,15 +538,19 @@ __global__ void kv_extract_f32_kernel(const float* __restrict__ qkv, float* __re
   const long long r = i >> 6;           // (b*T + t)*S + s
   const long long s = r % S, bt = r / S;
   const long long t = bt % T, b = bt / T;
+  if (n_rows && s >= n_rows[b]) {                 // a pad row of entry b: not read
+    kv[i] = 0.f;
+    return;
+  }
   const float* src = qkv + ((b * S + s) * T + t) * (3 * kE) + (c < 32 ? kE + c : 2 * kE + (c - 32));
   kv[i] = *src;
 }
 }  // namespace
 
-int launch_kv_extract_f32(const float* qkv, float* kv, int B, int S, int T, cudaStream_t st) {
+int launch_kv_extract_f32(const float* qkv, float* kv, int B, int S, int T, cudaStream_t st, const int* n_rows) {
   const long long n = (long long)B * T * S * 64;
   if (n <= 0) return MMPFN_OK;
-  kv_extract_f32_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(qkv, kv, S, T, n);
+  kv_extract_f32_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(qkv, kv, S, T, n, n_rows);
   return count_launch();
 }
 

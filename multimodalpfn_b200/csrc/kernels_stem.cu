@@ -81,15 +81,19 @@ __device__ void nan_mean_std(Fn value, int n, float& mean_clip, float& stdv, dou
 // One CTA per (group g, estimator b).  Reference: RemoveEmptyFeaturesEncoderStep (encoders.py:496-527),
 // NanHandlingEncoderStep._fit (:453-461), InputNormalizationEncoderStep._fit (:702-735),
 // VariableNumFeaturesEncoderStep._fit (:608-619).
-__global__ void __launch_bounds__(256) tab_fit_kernel(const float* __restrict__ x, int S, int F, int fpg,
-                                                      int n_train, float n_sigma, float* __restrict__ stats_all,
-                                                      int G) {
+// n_rows / n_train_b (or NULL): entry b's own row counts; its rows are the first n_rows[b] of its S-row block.
+__global__ void __launch_bounds__(256) tab_fit_kernel(const float* __restrict__ x, int S_alloc, int F, int fpg,
+                                                      int n_train_all, float n_sigma, float* __restrict__ stats_all,
+                                                      int G, const int* __restrict__ n_rows,
+                                                      const int* __restrict__ n_train_b) {
   __shared__ double sh[16];
   __shared__ int s_flag;
   const int b = blockIdx.y, g = blockIdx.x;
   const TabStatsLayout L{G * fpg, G};
   float* st = stats_all + (long long)b * L.total();
-  const float* xb = x + (long long)b * S * F;
+  const float* xb = x + (long long)b * S_alloc * F;
+  const int S = n_rows ? n_rows[b] : S_alloc;
+  const int n_train = n_train_b ? n_train_b[b] : n_train_all;
 
   // 1. which source columns of this group vary over ALL rows (encoders.py:515)
   int kept[8];
@@ -172,7 +176,7 @@ __global__ void __launch_bounds__(kE) stem_tokens_kernel(
     const float* __restrict__ pos_emb, const float* __restrict__ enc_w, const float* __restrict__ yenc_w,
     const float* __restrict__ yenc_b, int S, int F, int fpg, int G, int H_img, long long x_bstride,
     long long y_bstride, long long img_bstride, float* __restrict__ state, uint16_t* __restrict__ state_bf,
-    int32_t* __restrict__ nan_flag) {
+    int32_t* __restrict__ nan_flag, const long long* __restrict__ img_off, const int* __restrict__ n_rows) {
   const int e = threadIdx.x;
   const long long s = blockIdx.x;
   const int b = blockIdx.y;
@@ -182,6 +186,13 @@ __global__ void __launch_bounds__(kE) stem_tokens_kernel(
   const long long row = (long long)b * S + s;
   float* out = state + row * T * kE;
   uint16_t* outb = state_bf ? state_bf + row * T * kE : nullptr;
+  if (n_rows && s >= n_rows[b]) {          // a pad row of entry b: all zeros (no positional embedding, no NaN test)
+    for (int t = 0; t < T; ++t) {
+      out[(long long)t * kE + e] = 0.f;
+      if (outb) outb[(long long)t * kE + e] = 0;
+    }
+    return;
+  }
   bool bad = false;
   auto emit = [&](int t, float v) {
     out[(long long)t * kE + e] = v;
@@ -223,7 +234,8 @@ __global__ void __launch_bounds__(kE) stem_tokens_kernel(
   // image / text tokens appended after the tabular ones (transformer.py:768, :1038)
   // (img_bstride = 0: one set of tokens shared by the B estimators of a task; otherwise one per batch entry)
   for (int h = 0; h < H_img; ++h)
-    emit(G + h, img_tok[b * img_bstride + ((long long)s * H_img + h) * kE + e] + pos_emb[(G + h) * kE + e]);
+    emit(G + h, img_tok[(img_off ? img_off[b] : b * img_bstride) + ((long long)s * H_img + h) * kE + e] +
+                    pos_emb[(G + h) * kE + e]);
   // y token, last (encoders.py:480-493 indicator/fill, :961-964 ordinal rank, :422-425 Linear(2 -> E) + b)
   {
     float yy = y[b * y_bstride + s];
@@ -376,25 +388,26 @@ __global__ void proba_tail_kernel(const float* __restrict__ logits, const int32_
 }  // namespace
 
 int launch_tab_fit(const float* x, int B, int S, int F, int fpg, int n_train, float n_sigma, float* stats,
-                   cudaStream_t st) {
+                   cudaStream_t st, const int* n_rows, const int* n_train_b) {
   const int G = (F + fpg - 1) / fpg;
   if (G <= 0 || B <= 0) return MMPFN_OK;
   if (fpg > 8) { set_error("features_per_group %d > 8", fpg); return MMPFN_EUNSUPPORTED; }
-  tab_fit_kernel<<<dim3(G, B), 256, 0, st>>>(x, S, F, fpg, n_train, n_sigma, stats, G);
+  tab_fit_kernel<<<dim3(G, B), 256, 0, st>>>(x, S, F, fpg, n_train, n_sigma, stats, G, n_rows, n_train_b);
   return count_launch();
 }
 
 int launch_stem_tokens(const mmpfn_geometry* g, const mmpfn_weights* w, const float* x, const float* stats,
                        const float* img_tok, const float* y, const float* y_mean, const uint64_t* y_mask,
                        const float* pos_emb, int B, int S, int F, int H_img, long long x_bstride, long long y_bstride,
-                       long long img_bstride, float* state_f32, uint16_t* state_bf16, int32_t* nan_flag, cudaStream_t st) {
+                       long long img_bstride, float* state_f32, uint16_t* state_bf16, int32_t* nan_flag, cudaStream_t st,
+                       const long long* img_off, const int* n_rows) {
   const int fpg = g->features_per_group;
   const int G = x ? (F + fpg - 1) / fpg : 0;
   if (fpg > 4) { set_error("features_per_group %d > 4", fpg); return MMPFN_EUNSUPPORTED; }
   if (G * fpg > 1024) { set_error("stem_tokens: %d feature cells per row exceed the 1024 the kernel stages", G * fpg); return MMPFN_EUNSUPPORTED; }
   stem_tokens_kernel<<<dim3(S, B), kE, 0, st>>>(x, stats, img_tok, y, y_mean, y_mask, pos_emb, w->enc_w, w->yenc_w,
                                                w->yenc_b, S, F, fpg, G, H_img, x_bstride, y_bstride, img_bstride, state_f32, state_bf16,
-                                               nan_flag);
+                                               nan_flag, img_off, n_rows);
   return count_launch();
 }
 

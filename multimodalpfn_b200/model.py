@@ -22,13 +22,21 @@ import ctypes as C
 import dataclasses
 from typing import Optional
 
+import numpy as np
 import torch
 
 from . import _lib
 from .synth import Geometry
 from .weights import PackedWeights
 
-__all__ = ["B200PerFeatureTransformer", "TrainContext"]
+__all__ = ["B200PerFeatureTransformer", "TrainContext", "entry_counts"]
+
+
+def entry_counts(counts, capacity: int):
+    """Per-entry row counts of a pass (int32), or None when every entry fills the capacity: such a pass passes no
+    count arrays, i.e. runs the kernels of the equal-shape passes."""
+    counts = np.asarray(counts, dtype=np.int32)
+    return None if bool((counts == capacity).all()) else counts
 
 
 def _ptr(t: Optional[torch.Tensor]):
@@ -407,18 +415,196 @@ class B200PerFeatureTransformer:
             return logits
 
     # ---- several estimator groups at once (bf16): one launch per flat sublayer for all of them ----------
-    def _group_buffers(self, shapes):
+    def _group_buffers(self, shapes, with_bf16: bool = True):
         """One fp32 + one bf16 buffer for states of the given [(B, S, T)] shapes, and the per-group views."""
         E = self.geom.emsize
         total = sum(b * s * t for b, s, t in shapes)
         st = torch.empty((total, E), dtype=torch.float32, device=self.device)
-        stb = torch.empty((total, E), dtype=torch.bfloat16, device=self.device)
+        stb = torch.empty((total, E), dtype=torch.bfloat16, device=self.device) if with_bf16 else None
         views, off = [], 0
         for b, s, t in shapes:
             n = b * s * t
-            views.append((st[off:off + n].view(b, s, t, E), stb[off:off + n].view(b, s, t, E)))
+            views.append((st[off:off + n].view(b, s, t, E), None if stb is None else stb[off:off + n].view(b, s, t, E)))
             off += n
         return st, stb, views
+
+    # ---- entries of different sizes in one pass (tasks.py) ------------------------------------------------
+    def entry_tokens(self, F: Optional[int], n_tok: int) -> int:
+        """Token count T of an entry with ``F`` preprocessed features (None: no table) and ``n_tok`` embeddings."""
+        return (0 if F is None else self._n_groups(F)) + self.n_image_tokens(n_tok) + 1
+
+    def forward_ragged(self, entries, *, final_states: Optional[list] = None):
+        """One train pass and one test pass over batch entries of any sizes -> [logits [n_test, n_out]] in entry order.
+
+        An entry is one (task, estimator) pair: a dict with ``X`` (float32 [n_train + n_test, F], train rows first, or
+        None), ``y`` (class ids [n_train]), ``n_train``, ``n_test`` and ``tok`` / ``tok_row`` / ``n_tok`` (image
+        tokens [rows, H, E] from ``stem_image`` of ``n_tok`` embeddings per row and the row of the entry's first
+        train row in it, or ``tok`` None).  The pass
+        has the row capacity of its largest entry; the other entries' rows up to it are pad rows, kept exactly zero
+        (include/mmpfn_b200.h, "ragged" passes), so every entry's logits are bit-identical to ``fit_context`` +
+        ``predict_with_context`` over that entry alone (the stem statistics see its train and test rows).  Entries of
+        equal T form one segment (at most ``MMPFN_MAX_SEGMENTS``); a pass whose entries all have the capacity passes
+        no count arrays, i.e. runs the kernels of the equal-shape passes.  ``final_states`` (a list) receives, for the
+        train pass and then the test pass, ``(state [B_i, S, T_i, E], [entry index])`` per segment after the layers."""
+        if getattr(self.w, "regression", False):
+            raise ValueError("ragged passes serve classification entries (class-id labels)")
+        dev = self.device
+        T_of = [self.entry_tokens(None if e["X"] is None else e["X"].shape[1],
+                                  0 if e["tok"] is None else e["n_tok"]) for e in entries]
+        seg_T = list(dict.fromkeys(sorted(T_of)))
+        if len(seg_T) > _lib.MAX_SEGMENTS:
+            raise ValueError(f"{len(seg_T)} token counts in one pass (at most {_lib.MAX_SEGMENTS})")
+        # pass order: segments by T; inside a segment, blocks of one (feature count, embedding) kind
+        def block_key(j):
+            e = entries[j]
+            return (-1 if e["X"] is None else e["X"].shape[1], -1 if e["tok"] is None else id(e["tok"]))
+        order = sorted(range(len(entries)), key=lambda j: (T_of[j], block_key(j)))
+        segs = [(T, [j for j in order if T_of[j] == T]) for T in seg_T]
+        n_tr = np.array([entries[j]["n_train"] for j in order], dtype=np.int32)
+        n_te = np.array([entries[j]["n_test"] for j in order], dtype=np.int32)
+        S_tr, S_te = int(n_tr.max()), int(n_te.max())
+        c_tr, c_te = entry_counts(n_tr, S_tr), entry_counts(n_te, S_te)
+        c_all = entry_counts(n_tr + n_te, S_tr + S_te)
+        dev_i32 = lambda a: None if a is None else torch.from_numpy(np.ascontiguousarray(a, dtype=np.int32)).to(dev)
+        d_tr, d_te = dev_i32(c_tr), dev_i32(c_te)
+        pos_in_pass = {j: k for k, j in enumerate(order)}
+        with torch.cuda.device(dev):
+            # stem statistics: one call per feature count over the entries' train + test rows
+            Sa = S_tr + S_te
+            stats_of = {}
+            X_all = {}
+            by_F = {}
+            for j in order:
+                if entries[j]["X"] is not None:
+                    by_F.setdefault(entries[j]["X"].shape[1], []).append(j)
+            for F, js in by_F.items():
+                xa = np.zeros((len(js), Sa, F), dtype=np.float32)
+                for k, j in enumerate(js):
+                    xa[k, :len(entries[j]["X"])] = entries[j]["X"]
+                xa = torch.from_numpy(xa).to(dev)
+                if c_all is None:
+                    stats = self.stem_tab_fit(xa, S_tr)
+                else:
+                    idx = np.array([pos_in_pass[j] for j in js])
+                    stats = self._stem_tab_fit_ragged(xa, dev_i32(n_tr[idx] + n_te[idx]), dev_i32(n_tr[idx]))
+                for k, j in enumerate(js):
+                    stats_of[j] = (stats, k)
+                    X_all[j] = (xa, k)
+            # label statistics per entry on its own labels (torch's mean over a [k, n] block is per row; the
+            # presence mask is exact integer work)
+            y_mean = torch.empty(len(order), dtype=torch.float32, device=dev)
+            by_n = {}
+            for k, j in enumerate(order):
+                by_n.setdefault(entries[j]["n_train"], []).append(k)
+            ys = [np.asarray(entries[j]["y"]) for j in order]
+            for n, ks in by_n.items():
+                y_blk = torch.from_numpy(np.stack([ys[k] for k in ks]).astype(np.float32)).to(dev)
+                y_mean[torch.tensor(ks, device=dev)] = y_blk.mean(dim=1)
+            masks = []
+            for y in ys:
+                yl = y.astype(np.int64)
+                if not np.array_equal(yl, y) or yl.min() < 0 or yl.max() > 62:
+                    raise ValueError("labels must be integer class ids in [0, 62]")
+                masks.append(int(np.bitwise_or.reduce(np.left_shift(np.int64(1), np.unique(yl)))))
+            y_mask = torch.tensor(masks, dtype=torch.int64, device=dev)
+            y_tr = np.zeros((len(order), S_tr), dtype=np.float32)
+            for k, y in enumerate(ys):
+                y_tr[k, :len(y)] = y
+            y_tr = torch.from_numpy(y_tr).to(dev)
+            y_nan = torch.full((S_te,), float("nan"), dtype=torch.float32, device=dev)
+            flag = torch.zeros(1, dtype=torch.int32, device=dev)
+            bf16 = self.precision == _lib.BF16
+            shapes = [(len(js), T) for T, js in segs]
+            kvs = [self.alloc_kv(b, S_tr, T) for b, T in shapes]
+            logits = [None] * len(entries)
+            for train in (True, False):
+                S = S_tr if train else S_te
+                st, stb, views = self._group_buffers([(b, S, T) for b, T in shapes], with_bf16=bf16)
+                k0 = 0
+                for (T, js), (v, vb) in zip(segs, views):
+                    pos = self.positional_embeddings(T - 1)
+                    i0 = 0
+                    while i0 < len(js):          # blocks: entries of one feature count and one embedding kind
+                        i1 = i0 + 1
+                        while i1 < len(js) and block_key(js[i1]) == block_key(js[i0]):
+                            i1 += 1
+                        blk = js[i0:i1]
+                        self._embed_block([entries[j] for j in blk], blk, stats_of, X_all, train, S_tr, S_te,
+                                          y_tr[k0 + i0:k0 + i1], y_nan, y_mean[k0 + i0:k0 + i1],
+                                          y_mask[k0 + i0:k0 + i1], pos, v[i0:i1], None if vb is None else vb[i0:i1],
+                                          (d_tr if train else d_te), k0 + i0, flag)
+                        i0 = i1
+                    k0 += len(js)
+                seg_arr = (_lib.Segment * len(shapes))(*[_lib.Segment(b, T) for b, T in shapes])
+                kvp = (C.c_void_p * len(kvs))(*[kv.data_ptr() for kv in kvs])
+                nbytes = self.lib.mmpfn_layers_ragged_ws_bytes(self._g, seg_arr, len(shapes), S, self.precision)
+                ws = self._scratch("layers", nbytes)
+                if train:
+                    _lib.check(self.lib.mmpfn_layers_train_ragged(
+                        self._g, self._w, st.data_ptr(), _ptr(stb), seg_arr, len(shapes), S, _ptr(d_tr),
+                        self.precision, kvp, ws.data_ptr(), nbytes, self._stream()), "mmpfn_layers_train_ragged")
+                    if final_states is not None:
+                        final_states.extend(zip([v for v, _ in views], [js for _, js in segs]))
+                else:
+                    _lib.check(self.lib.mmpfn_layers_test_ragged(
+                        self._g, self._w_test, st.data_ptr(), _ptr(stb), seg_arr, len(shapes), S, S_tr, _ptr(d_te),
+                        _ptr(d_tr), self.precision, kvp, ws.data_ptr(), nbytes, self._stream()),
+                        "mmpfn_layers_test_ragged")
+                    for (T, js), (v, _) in zip(segs, views):
+                        lg = self.decode(v)
+                        if final_states is not None:
+                            final_states.append((v, js))
+                        for k, j in enumerate(js):
+                            logits[j] = lg[k, :entries[j]["n_test"]]
+                del st, stb, views
+            self._check_nan(flag)
+            return logits
+
+    def _stem_tab_fit_ragged(self, X, n_rows, n_train):
+        B, S, F = X.shape
+        n = self.lib.mmpfn_tab_stats_elems(self._g, self._n_groups(F))
+        stats = torch.empty((B, n), dtype=torch.float32, device=self.device)
+        sigma = float(self.outlier_std) if self.outlier_std is not None else float("inf")
+        _lib.check(self.lib.mmpfn_stem_tab_fit_ragged(self._g, X.data_ptr(), B, S, F, n_rows.data_ptr(),
+                                                      n_train.data_ptr(), sigma, stats.data_ptr(), self._stream()),
+                   "mmpfn_stem_tab_fit_ragged")
+        return stats
+
+    def _embed_block(self, ents, js, stats_of, X_all, train, S_tr, S_te, y_tr, y_nan, y_mean, y_mask, pos, out,
+                     out_b, counts, k0, flag):
+        """Token assembly of one block (same feature count and embeddings) of a ragged pass into its views."""
+        dev, B = self.device, len(ents)
+        S = S_tr if train else S_te
+        x = stats = None
+        F = 0
+        if ents[0]["X"] is not None:
+            xa, _ = X_all[js[0]]
+            F = xa.shape[2]
+            rows = torch.tensor([X_all[j][1] for j in js], device=dev)
+            stats = stats_of[js[0]][0][rows].contiguous()
+            if train:
+                x = xa[rows].contiguous()                     # train rows first: rows [0, n_train) of each block
+                x_bstride = x.shape[1] * F
+            else:
+                xt = np.zeros((B, S_te, F), dtype=np.float32)
+                for k, e in enumerate(ents):
+                    xt[k, :e["n_test"]] = e["X"][e["n_train"]:]
+                x = torch.from_numpy(xt).to(dev)
+                x_bstride = S_te * F
+        else:
+            x_bstride = 0
+        tok = ents[0]["tok"]
+        H = 0 if tok is None else tok.shape[1]
+        off = None
+        if tok is not None:
+            off = torch.tensor([(e["tok_row"] + (0 if train else e["n_train"])) * H * tok.shape[2] for e in ents],
+                               dtype=torch.int64, device=dev)
+        cnt = None if counts is None else counts[k0:k0 + B]
+        _lib.check(self.lib.mmpfn_stem_tokens_ragged(
+            self._g, self._w, _ptr(x), _ptr(stats), _ptr(tok), y_tr.data_ptr() if train else y_nan.data_ptr(),
+            y_mean.data_ptr(), y_mask.data_ptr(), pos.data_ptr(), B, S, F, H, x_bstride, S_tr if train else 0,
+            _ptr(off), _ptr(cnt), out.data_ptr(), _ptr(out_b), flag.data_ptr(), self._stream()),
+            "mmpfn_stem_tokens_ragged")
 
     def fit_contexts(self, specs, *, nan_flag=None):
         """``fit_context`` for several estimator groups that share the train rows (same n_train) — specs:

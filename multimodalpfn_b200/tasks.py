@@ -3,9 +3,19 @@
 The reference has a batch axis in the transformer (``x [S, B, F]``, state ``[B, S, T, E]``,
 ``layer.py:284-285``) but its engines always pass ``B = 1`` (``inference.py:305``) and the CAP stem
 hard-codes it (``transformer.py:78-79``): 256 small datasets mean 256 x n_estimators sequential
-forwards there.  Here the batch axis of every kernel carries *tasks*: all tasks with the same shape
-run as ONE batched forward per estimator slot (their image tokens ride along per batch entry,
-``mmpfn_stem_tokens(img_bstride)``), so the launches see ``B x S x T`` tokens instead of ``S x T``.
+forwards there.  Here the batch axis of every kernel carries *entries*, one per (task, estimator)
+pair, and tasks of ANY sizes share launches:
+
+* ``plan_passes`` splits the entries into passes.  A pass has the row capacity of its largest entry
+  (train rows and test rows); the other entries' rows up to it are pad rows.  Entries are sorted by
+  row count and a pass is closed before it would hold more than ``MAX_SEGMENTS`` distinct token
+  counts T, more than ``token_budget`` tokens, or a padded share of its tokens above
+  ``MAX_PAD_FRACTION``.  Tasks of equal shape pad nothing: their passes pass no count arrays.
+* ``B200PerFeatureTransformer.forward_ragged`` runs one train pass and one test pass per pass
+  (entries of equal T form one segment); the kernels keep every pad row exactly zero, so each
+  entry's arithmetic is that of a forward over the entry alone (include/mmpfn_b200.h).
+* The image stem runs once per embedding-token count over the rows of all its tasks.
+
 Tasks are independent until the end, so a multi-GPU run just deals them out round-robin and gathers
 the probabilities — no collective on the data path.
 
@@ -25,7 +35,42 @@ from .engine import proba_from_logits
 from .model import B200PerFeatureTransformer
 from .preprocessing import RECIPES, fit_transform_all, make_members, transform_all
 
-__all__ = ["predict_proba_tasks", "shard_tasks", "gather_task_results"]
+__all__ = ["predict_proba_tasks", "plan_passes", "shard_tasks", "gather_task_results"]
+
+MAX_SEGMENTS = 8              # distinct token counts per pass (MMPFN_MAX_SEGMENTS)
+MAX_PAD_FRACTION = 0.25       # padded tokens of a pass over all its tokens
+TOKEN_BUDGET = 1 << 21        # train + test tokens per pass (~10 GB of state and bf16 workspace)
+
+
+def plan_passes(shapes: Sequence[tuple], *, token_budget: int = TOKEN_BUDGET) -> list:
+    """Split entries of shapes ``(n_train, n_test, T)`` into passes -> [[entry index]].
+
+    A pass's tokens are ``(S_train + S_test) * sum T`` (its capacities times its entries' token counts).  Entries
+    are taken in descending row count; an entry joins the open pass unless that pass would then hold more than
+    ``MAX_SEGMENTS`` distinct T, more than ``token_budget`` tokens, or more than ``MAX_PAD_FRACTION`` of its tokens
+    on pad rows; then it opens the next pass (alone, an entry pads nothing, whatever its size)."""
+    order = sorted(range(len(shapes)), key=lambda i: (-shapes[i][0], -shapes[i][1], shapes[i][2], i))
+    passes, cur = [], []
+    S_tr = S_te = sum_T = useful = 0
+    Ts = set()
+    for i in order:
+        n_tr, n_te, T = (int(v) for v in shapes[i])
+        if cur:
+            s_tr, s_te, s_T = max(S_tr, n_tr), max(S_te, n_te), sum_T + T
+            tokens = (s_tr + s_te) * s_T
+            if (len(Ts | {T}) <= MAX_SEGMENTS and tokens <= token_budget
+                    and tokens - (useful + (n_tr + n_te) * T) <= MAX_PAD_FRACTION * tokens):
+                cur.append(i)
+                S_tr, S_te, sum_T = s_tr, s_te, s_T
+                useful += (n_tr + n_te) * T
+                Ts.add(T)
+                continue
+            passes.append(cur)
+        cur = [i]
+        S_tr, S_te, sum_T, useful, Ts = n_tr, n_te, T, (n_tr + n_te) * T, {T}
+    if cur:
+        passes.append(cur)
+    return passes
 
 
 def shard_tasks(n_tasks: int, rank: int, world: int) -> list:
@@ -66,9 +111,8 @@ def _prepare(task: dict, n_estimators: int, random_state, recipes):
         return a[:, None] if a.ndim == 2 else a
     itr, ite = img(task.get("img_train")), img(task.get("img_test"))
     n_te = len(Xte) if Xte is not None else len(ite)
-    key = (len(y), n_te, None if itr is None else itr.shape[1:], tuple(None if t[0] is None else t[0].shape[1] for t in train))
     return dict(members=members, train=train, test=test, img_train=itr, img_test=ite, n_classes=n_cls, counts=counts,
-                classes=enc.classes_, key=key)
+                classes=enc.classes_, n_train=len(y), n_test=n_te)
 
 
 def predict_proba_tasks(model: B200PerFeatureTransformer, tasks: Sequence[dict], *, n_estimators: int = 4,
@@ -77,7 +121,7 @@ def predict_proba_tasks(model: B200PerFeatureTransformer, tasks: Sequence[dict],
                         n_jobs: int = 1, timings: Optional[dict] = None):
     """``tasks``: dicts with ``X_train, img_train, y_train, X_test, img_test`` (tables or embeddings may be
     ``None`` like in ``MMPFNClassifier.fit``).  Returns ``{task index: float32 [Nte, n_classes]}`` for the
-    tasks in ``indices`` (default: all).  Tasks of equal shape share launches.  The per-task host work
+    tasks in ``indices`` (default: all).  Tasks of any shapes share launches (``plan_passes``).  The per-task host work
     (fitting the members' quantile / SVD transforms) can run in ``n_jobs`` threads (it is mostly GIL-bound
     sklearn glue: 16 threads measured slower than 1); ``timings`` (a dict) receives
     the seconds spent in ``host_prepare`` and ``device``."""
@@ -96,34 +140,37 @@ def predict_proba_tasks(model: B200PerFeatureTransformer, tasks: Sequence[dict],
     else:
         prepared = {i: _prepare(tasks[i], n_estimators, random_state, recipes) for i in indices}
     t1 = time.perf_counter()
-    groups = {}
+    # one image-stem pass per embedding-token count over the rows of all its tasks
+    tok_of = {}
+    by_ntok = {}
     for i in indices:
-        groups.setdefault(prepared[i]["key"], []).append(i)
-    logits = {i: [None] * n_estimators for i in indices}
-    for key, idx in groups.items():
-        n_tr, n_te, img_shape, widths = key
-        tok_tr = tok_te = None
-        if img_shape is not None:
-            # one image-stem pass over the embeddings of every task of the group: [Bt * S, n_tok, I] -> [Bt, S, H, E]
-            img_all = np.concatenate([np.concatenate([prepared[i]["img_train"], prepared[i]["img_test"]]) for i in idx])
-            tok = model.stem_image(torch.from_numpy(img_all).to(dev))
-            tok = tok.view(len(idx), n_tr + n_te, tok.shape[1], tok.shape[2])
-            tok_tr, tok_te = tok[:, :n_tr].contiguous(), tok[:, n_tr:].contiguous()
+        if prepared[i]["img_train"] is not None:
+            by_ntok.setdefault(prepared[i]["img_train"].shape[1], []).append(i)
+    for n_tok, idx in by_ntok.items():
+        img_all = np.concatenate([np.concatenate([prepared[i]["img_train"], prepared[i]["img_test"]]) for i in idx])
+        tok = model.stem_image(torch.from_numpy(img_all).to(dev))
+        row = 0
+        for i in idx:
+            tok_of[i] = (tok, row, n_tok)
+            row += prepared[i]["n_train"] + prepared[i]["n_test"]
+    entries, owner = [], []
+    for i in indices:
+        pr = prepared[i]
+        tok, row, n_tok = tok_of.get(i, (None, 0, 0))
         for e in range(n_estimators):
-            ytr = torch.from_numpy(np.stack([prepared[i]["train"][e][1] for i in idx])).to(dev)
-            if widths[e] is None:
-                Xtr = Xte = X_full = None
-            else:
-                Xtr = torch.from_numpy(np.stack([prepared[i]["train"][e][0] for i in idx])).to(dev)
-                Xte = torch.from_numpy(np.stack([prepared[i]["test"][e] for i in idx])).to(dev)
-                X_full = torch.cat([Xtr, Xte], dim=1)
-            # reference-equivalent joint forward (the stem's constant-column tests see train and test rows)
-            flag = torch.zeros(1, dtype=torch.int32, device=dev)      # one NaN flag for train and test rows
-            ctx = model.fit_context(Xtr, None, ytr, X_all=X_full, img_tok_train=tok_tr, check=False, nan_flag=flag)
-            lg = model.predict_with_context(ctx, Xte, None, img_tok_test=tok_te, nan_flag=flag)
-            for k, i in enumerate(idx):
-                logits[i][e] = lg[k]
-            del ctx
+            X = pr["train"][e][0]
+            # the stem statistics see train and test rows (the reference's joint forward, encoders.py:515, :615)
+            X_all = None if X is None else np.concatenate([X, pr["test"][e]]).astype(np.float32, copy=False)
+            entries.append(dict(X=X_all, y=pr["train"][e][1], n_train=pr["n_train"], n_test=pr["n_test"], tok=tok,
+                                tok_row=row, n_tok=n_tok))
+            owner.append((i, e))
+    shapes = [(en["n_train"], en["n_test"],
+               model.entry_tokens(None if en["X"] is None else en["X"].shape[1], en["n_tok"])) for en in entries]
+    logits = {i: [None] * n_estimators for i in indices}
+    for ps in plan_passes(shapes):
+        for k, lg in zip(ps, model.forward_ragged([entries[k] for k in ps])):
+            i, e = owner[k]
+            logits[i][e] = lg
     out = {}
     for i in indices:
         pr = prepared[i]
