@@ -277,6 +277,35 @@ int mmpfn_proba_tail(const float* logits, const int32_t* class_perm, const float
                      int n_out, int n_classes, float temperature, int average_before_softmax, float* proba,
                      void* stream);
 
+/* Bar-distribution tail of the regressor (the reference's regressor.py predict: translate_probs_across_borders +
+ * FullSupportBarDistribution mean / icdf / mode), one CTA per test row; only the requested outputs leave the row.
+ *   logits     [n_est][S][K]   per-estimator logits over K buckets (what the decoder writes)
+ *   src_bucket [n_est][K+1]    int32: for common border g_j, the bucket i of estimator e's own borders f_e with
+ *                              f_e[i] <= g_j < f_e[i+1]; -1 below f_e[0], K at or above f_e[K]
+ *   src_share  [n_est][K+1]    (g_j - f_e[i]) / (f_e[i+1] - f_e[i]) clamped to [0, 1] (unused for i = -1, K)
+ *   cancel     [n_est][K]      uint8, nonzero = that bucket's logit is -inf; may be NULL
+ *   borders    [K+1]           common borders G in target units, increasing
+ *   quantiles  [n_q]           in (0, 1)
+ *   mean, median, mode [S]; quant [n_q][S]; log_prob [S][K].  Every output may be NULL (not computed).
+ * Per row s:
+ *  1. z_e = logits[e][s] / temperature (as is when temperature == 1); cancelled buckets -inf; p_e = softmax(z_e);
+ *     P_e(i) = sum_{k<i} p_e[k].
+ *  2. C_e(j) = 0 for i = -1, 1 for i = K, else P_e(i) + p_e[i] * src_share[e][j] (i = src_bucket[e][j]);
+ *     C_e(0) = 0, C_e(K) = 1; q_e[j] = max(C_e(j+1) - C_e(j), 0): estimator e's piecewise-linear CDF at G.
+ *  3. P = mean_e q_e (average_before_softmax = 0) or softmax(mean_e log q_e) (= 1); log_prob = log P.
+ *  4. w_j = G_{j+1} - G_j.  mean = sum_j P_j m_j, m_j = (G_j + G_{j+1}) / 2 inside, half-normal tails outside:
+ *     m_0 = G_1 - w_0 sqrt(2/pi), m_{K-1} = G_{K-1} + w_{K-1} sqrt(2/pi).
+ *  5. quantile q: c_j = sum_{i<=j} P_i, j = first index with c_j >= q (clamped to K-1), r = (q - c_{j-1}) / P_j
+ *     clamped to [0, 1]: G_j + r w_j inside, G_1 - w_0 sqrt(2) erfinv(1 - r) in the left tail,
+ *     G_{K-1} + w_{K-1} sqrt(2) erfinv(r) in the right tail.  median = the quantile at 0.5.
+ *  6. mode = midpoint of the bucket with the largest P_j / w_j (lowest j on ties).
+ * Prefix sums run in float64 (a bucket mass is a difference of two).  2 <= K <= 8192 (MMPFN_EUNSUPPORTED beyond:
+ * the row's working set lives in shared memory). */
+int mmpfn_bar_tail(const float* logits, int n_est, int S, int K, const int32_t* src_bucket, const float* src_share,
+                   const uint8_t* cancel, const float* borders, float temperature, int average_before_softmax,
+                   const float* quantiles, int n_q, float* mean, float* median, float* mode, float* quant,
+                   float* log_prob, void* stream);
+
 /* ---- building blocks exported for unit tests and profiling ---------------------------------- */
 /* y = LayerNorm(x (+ res)) over `width` (192 or 768), eps 1e-5, optional affine (layer.py:40-64). */
 int mmpfn_layernorm(const float* x, const float* res, const float* gamma, const float* beta, int rows, int width,

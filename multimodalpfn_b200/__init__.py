@@ -4,13 +4,16 @@ Importing the package does not need a GPU; constructing a model or classifier do
 """
 from .synth import Geometry  # noqa: F401
 
-__all__ = ["Geometry", "MMPFNClassifier", "B200PerFeatureTransformer", "B200InferenceEngine"]
+__all__ = ["Geometry", "MMPFNClassifier", "MMPFNRegressor", "B200PerFeatureTransformer", "B200InferenceEngine"]
 
 
 def __getattr__(name):
     if name == "MMPFNClassifier":
         from .classifier import MMPFNClassifier
         return MMPFNClassifier
+    if name == "MMPFNRegressor":
+        from .regressor import MMPFNRegressor
+        return MMPFNRegressor
     if name == "B200PerFeatureTransformer":
         from .model import B200PerFeatureTransformer
         return B200PerFeatureTransformer

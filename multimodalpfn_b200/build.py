@@ -19,7 +19,7 @@ INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 DEBUG = os.environ.get("MMPFN_DEBUG_LIB", "0") == "1"
 LIB = os.path.join(HERE, "libmmpfn_b200_dbg.so" if DEBUG else "libmmpfn_b200.so")
 STAMP = os.path.join(HERE, ".libmmpfn_b200_dbg.stamp" if DEBUG else ".libmmpfn_b200.stamp")
-SOURCES = ["api.cu", "kernels_f32.cu", "kernels_stem.cu", "kernels_tc.cu", "kernels_attn.cu", "kernels_mlp.cu", "kernels_rowgemm.cu", "kernels_featfused.cu"]
+SOURCES = ["api.cu", "kernels_f32.cu", "kernels_stem.cu", "kernels_tc.cu", "kernels_attn.cu", "kernels_mlp.cu", "kernels_rowgemm.cu", "kernels_featfused.cu", "kernels_tail.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "--expt-relaxed-constexpr", "-Xcompiler", "-fPIC", "-shared", "-cudart", "static",

@@ -241,4 +241,10 @@ int launch_moe_gate_scale(const float* gate_logits, float* tok, int S, int Hm, c
 int launch_proba_tail(const float* logits, const int32_t* perm, const float* prior, int n_est, int S, int n_out,
                       int n_classes, float temperature, int avg_before, float* proba, cudaStream_t st);
 
+// ---- bar-distribution tail (kernels_tail.cu) ------------------------------------------------------------------
+int launch_bar_tail(const float* logits, int n_est, int S, int K, const int32_t* src_bucket, const float* src_share,
+                    const uint8_t* cancel, const float* borders, float temperature, int avg_before,
+                    const float* quantiles, int n_q, float* mean, float* median, float* mode, float* quant,
+                    float* log_prob, cudaStream_t st);
+
 }  // namespace mmpfn

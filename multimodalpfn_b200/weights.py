@@ -19,7 +19,7 @@ import torch
 from . import _lib
 from .synth import Geometry
 
-__all__ = ["PackedWeights", "load_checkpoint"]
+__all__ = ["PackedWeights", "load_checkpoint", "load_borders"]
 
 
 def _np(v) -> np.ndarray:
@@ -202,3 +202,12 @@ def load_checkpoint(path, *, mixer_type="MGM+CAP", mgm_heads=8, cap_heads=8, fea
     geom = geometry_from_checkpoint(ckpt.get("config", {}), sd, mixer_type=mixer_type, mgm_heads=mgm_heads,
                                     cap_heads=cap_heads, features_per_group=features_per_group)
     return sd, geom
+
+
+def load_borders(path) -> np.ndarray:
+    """The bar-distribution borders ``criterion.borders`` [n_out + 1] of a regression checkpoint (float64, over the
+    standardised target); ValueError when the checkpoint has none."""
+    sd = torch.load(path, map_location="cpu", weights_only=False)["state_dict"]
+    if "criterion.borders" not in sd:
+        raise ValueError("checkpoint has no criterion.borders (not a regression checkpoint)")
+    return _np(sd["criterion.borders"]).astype(np.float64).ravel()
