@@ -306,6 +306,22 @@ int mmpfn_bar_tail(const float* logits, int n_est, int S, int K, const int32_t* 
                    const float* quantiles, int n_q, float* mean, float* median, float* mode, float* quant,
                    float* log_prob, void* stream);
 
+/* mmpfn_bar_tail over the rows of many tasks in one launch, one CTA per global row; steps 1-6 per row exactly as
+ * mmpfn_bar_tail, with task t's own maps and borders (each task's G is in its own target units):
+ *   logits     [n_tasks * n_est]  device array of pointers: logits[t * n_est + e] points to row 0 of task t's rows
+ *                                 for estimator e, rows K floats apart (the decoder's per-entry outputs, in place)
+ *   row_offset [n_tasks + 1]      int32 on the device: task t owns global rows [row_offset[t], row_offset[t+1])
+ *   src_bucket, src_share [n_tasks][n_est][K+1];  cancel [n_tasks][n_est][K] or NULL;  borders [n_tasks][K+1]
+ *   mean, median, mode [S_total]; quant [n_q][S_total]; log_prob [S_total][K], indexed by global row; any may be NULL.
+ * K, n_est, the temperature, the averaging mode and the quantiles are shared by all tasks.  Preconditions the call
+ * cannot check without a host sync: row_offset[0] == 0, row_offset is nondecreasing (a task may own no rows) and
+ * row_offset[n_tasks] == S_total.  MMPFN_EINVAL / MMPFN_EUNSUPPORTED as mmpfn_bar_tail. */
+int mmpfn_bar_tail_tasks(const float* const* logits, int n_tasks, int n_est, const int32_t* row_offset, int S_total,
+                         int K, const int32_t* src_bucket, const float* src_share, const uint8_t* cancel,
+                         const float* borders, float temperature, int average_before_softmax, const float* quantiles,
+                         int n_q, float* mean, float* median, float* mode, float* quant, float* log_prob,
+                         void* stream);
+
 /* ---- building blocks exported for unit tests and profiling ---------------------------------- */
 /* y = LayerNorm(x (+ res)) over `width` (192 or 768), eps 1e-5, optional affine (layer.py:40-64). */
 int mmpfn_layernorm(const float* x, const float* res, const float* gamma, const float* beta, int rows, int width,

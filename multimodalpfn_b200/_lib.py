@@ -80,6 +80,9 @@ SIGNATURES = {
                                  c_void_p]),
     "mmpfn_bar_tail": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_int,
                                c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "mmpfn_bar_tail_tasks": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p,
+                                     c_void_p, c_float, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
+                                     c_void_p, c_void_p]),
     "mmpfn_layernorm": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "mmpfn_linear_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),
     "mmpfn_linear_bf16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p]),

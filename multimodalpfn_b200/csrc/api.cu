@@ -837,9 +837,27 @@ int mmpfn_bar_tail(const float* logits, int n_est, int S, int K, const int32_t* 
     return MMPFN_EINVAL;
   }
   if (!mean && !median && !mode && !quant && !log_prob) return MMPFN_OK;
-  return launch_bar_tail(logits, n_est, S, K, src_bucket, src_share, cancel, borders, temperature,
+  return launch_bar_tail(logits, nullptr, nullptr, 1, n_est, S, K, src_bucket, src_share, cancel, borders, temperature,
                          average_before_softmax, quantiles, n_q, mean, median, mode, quant, log_prob,
                          (cudaStream_t)stream);
+}
+
+int mmpfn_bar_tail_tasks(const float* const* logits, int n_tasks, int n_est, const int32_t* row_offset, int S_total,
+                         int K, const int32_t* src_bucket, const float* src_share, const uint8_t* cancel,
+                         const float* borders, float temperature, int average_before_softmax, const float* quantiles,
+                         int n_q, float* mean, float* median, float* mode, float* quant, float* log_prob,
+                         void* stream) {
+  MMPFN_TRY(require_device());
+  if (!logits || !row_offset || !src_bucket || !src_share || !borders || n_tasks < 1 || n_est < 1 || S_total < 1 ||
+      K < 2 || n_q < 0 || !(temperature > 0.f) || (quant && (!quantiles || n_q < 1))) {
+    set_error("bar_tail_tasks: bad arguments (n_tasks %d n_est %d S_total %d K %d n_q %d temperature %g)", n_tasks,
+              n_est, S_total, K, n_q, temperature);
+    return MMPFN_EINVAL;
+  }
+  if (!mean && !median && !mode && !quant && !log_prob) return MMPFN_OK;
+  return launch_bar_tail(nullptr, logits, row_offset, n_tasks, n_est, S_total, K, src_bucket, src_share, cancel,
+                         borders, temperature, average_before_softmax, quantiles, n_q, mean, median, mode, quant,
+                         log_prob, (cudaStream_t)stream);
 }
 
 int mmpfn_layernorm(const float* x, const float* res, const float* gamma, const float* beta, int rows, int width,

@@ -242,9 +242,10 @@ int launch_proba_tail(const float* logits, const int32_t* perm, const float* pri
                       int n_classes, float temperature, int avg_before, float* proba, cudaStream_t st);
 
 // ---- bar-distribution tail (kernels_tail.cu) ------------------------------------------------------------------
-int launch_bar_tail(const float* logits, int n_est, int S, int K, const int32_t* src_bucket, const float* src_share,
-                    const uint8_t* cancel, const float* borders, float temperature, int avg_before,
-                    const float* quantiles, int n_q, float* mean, float* median, float* mode, float* quant,
-                    float* log_prob, cudaStream_t st);
+// task_logits NULL: one task, logits [n_est][S][K]; else the many-task form (row_offset, n_tasks; logits unused)
+int launch_bar_tail(const float* logits, const float* const* task_logits, const int32_t* row_offset, int n_tasks,
+                    int n_est, int S, int K, const int32_t* src_bucket, const float* src_share, const uint8_t* cancel,
+                    const float* borders, float temperature, int avg_before, const float* quantiles, int n_q,
+                    float* mean, float* median, float* mode, float* quant, float* log_prob, cudaStream_t st);
 
 }  // namespace mmpfn

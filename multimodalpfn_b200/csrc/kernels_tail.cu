@@ -1,4 +1,5 @@
-// kernels_tail.cu — the bar-distribution tail of the regressor (mmpfn_bar_tail, include/mmpfn_b200.h).
+// kernels_tail.cu — the bar-distribution tail of the regressor (mmpfn_bar_tail and its many-task form
+// mmpfn_bar_tail_tasks, include/mmpfn_b200.h).
 //
 // One CTA per test row.  Per estimator: load the row's K logits (float4 when aligned), temperature and cancel
 // mask, block max / sum -> p_e in shared memory, exclusive prefix sum of p_e in float64, then the translated
@@ -93,11 +94,17 @@ __device__ __forceinline__ void border_pos(const int32_t* sb, const float* ss, i
   s = __ldg(ss + j);
 }
 
+// kTasks = false: one task, logits [n_est][S][K] (mmpfn_bar_tail).  kTasks = true: row s belongs to the task tk with
+// row_offset[tk] <= s < row_offset[tk + 1]; its logits for estimator e start at task_logits[tk * n_est + e] (row
+// stride K) and its maps and borders at task tk's slices (mmpfn_bar_tail_tasks).  S is the total row count.
+// The tasks-only parameters come last: the one-task form keeps its parameter offsets, 32 registers and SASS.
+template <bool kTasks>
 __global__ void __launch_bounds__(512) bar_tail_kernel(
     const float* __restrict__ logits, int n_est, int S, int K, const int32_t* __restrict__ src_bucket,
     const float* __restrict__ src_share, const uint8_t* __restrict__ cancel, const float* __restrict__ borders,
     float temperature, int avg_before, const float* __restrict__ quantiles, int n_q, float* __restrict__ mean,
-    float* __restrict__ median, float* __restrict__ mode, float* __restrict__ quant, float* __restrict__ log_prob) {
+    float* __restrict__ median, float* __restrict__ mode, float* __restrict__ quant, float* __restrict__ log_prob,
+    const float* const* __restrict__ task_logits, const int32_t* __restrict__ row_offset, int n_tasks) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double* pre = reinterpret_cast<double*>(smem_raw);                        // [K+1]
   float* p = reinterpret_cast<float*>(pre + K + 1);                         // [K]
@@ -105,10 +112,25 @@ __global__ void __launch_bounds__(512) bar_tail_kernel(
   TailScratch* sc = reinterpret_cast<TailScratch*>(acc + K);
   const int s = blockIdx.x, t = threadIdx.x, nt = blockDim.x;
   const bool vec4 = (K % 4) == 0;
+  int tk = 0;
+  long long row = s;                                   // the row within its task
+  if constexpr (kTasks) {
+    int lo = 0, hi = n_tasks - 1;                      // last task whose first row is <= s (skips empty tasks)
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) >> 1;
+      if (__ldg(row_offset + mid) <= s) lo = mid; else hi = mid - 1;
+    }
+    tk = lo;
+    row = s - __ldg(row_offset + tk);
+    src_bucket += (long long)tk * n_est * (K + 1);
+    src_share += (long long)tk * n_est * (K + 1);
+    if (cancel) cancel += (long long)tk * n_est * K;
+    borders += (long long)tk * (K + 1);
+  }
 
   for (int j = t; j < K; j += nt) acc[j] = 0.f;
   for (int e = 0; e < n_est; ++e) {
-    const float* lg = logits + ((long long)e * S + s) * K;
+    const float* lg = kTasks ? task_logits[(long long)tk * n_est + e] + row * K : logits + ((long long)e * S + s) * K;
     const uint8_t* cm = cancel ? cancel + (long long)e * K : nullptr;
     float mx = -INFINITY;
     if (vec4) {
@@ -238,22 +260,33 @@ __global__ void __launch_bounds__(512) bar_tail_kernel(
   }
 }
 
+// one instantiation each: MMPFN_OPT_IN_SMEM keeps its "done" flag per expansion
+template <bool kTasks>
+int launch_tail(const float* logits, const float* const* task_logits, const int32_t* row_offset, int n_tasks,
+                int n_est, int S, int K, const int32_t* src_bucket, const float* src_share, const uint8_t* cancel,
+                const float* borders, float temperature, int avg_before, const float* quantiles, int n_q, float* mean,
+                float* median, float* mode, float* quant, float* log_prob, cudaStream_t st) {
+  MMPFN_OPT_IN_SMEM(bar_tail_kernel<kTasks>, tail_smem_bytes(kTailMaxK));
+  const int threads = K <= 1024 ? 128 : 512;
+  bar_tail_kernel<kTasks><<<S, threads, tail_smem_bytes(K), st>>>(
+      logits, n_est, S, K, src_bucket, src_share, cancel, borders, temperature,
+      avg_before, quantiles, n_q, mean, median, mode, quant, log_prob, task_logits, row_offset, n_tasks);
+  return count_launch();
+}
+
 }  // namespace
 
-int launch_bar_tail(const float* logits, int n_est, int S, int K, const int32_t* src_bucket, const float* src_share,
-                    const uint8_t* cancel, const float* borders, float temperature, int avg_before,
-                    const float* quantiles, int n_q, float* mean, float* median, float* mode, float* quant,
-                    float* log_prob, cudaStream_t st) {
+int launch_bar_tail(const float* logits, const float* const* task_logits, const int32_t* row_offset, int n_tasks,
+                    int n_est, int S, int K, const int32_t* src_bucket, const float* src_share, const uint8_t* cancel,
+                    const float* borders, float temperature, int avg_before, const float* quantiles, int n_q,
+                    float* mean, float* median, float* mode, float* quant, float* log_prob, cudaStream_t st) {
   if (K > kTailMaxK) {
     set_error("bar_tail: %d buckets exceed the %d the shared-memory layout holds", K, kTailMaxK);
     return MMPFN_EUNSUPPORTED;
   }
-  MMPFN_OPT_IN_SMEM(bar_tail_kernel, tail_smem_bytes(kTailMaxK));
-  const int threads = K <= 1024 ? 128 : 512;
-  bar_tail_kernel<<<S, threads, tail_smem_bytes(K), st>>>(logits, n_est, S, K, src_bucket, src_share, cancel, borders,
-                                                          temperature, avg_before, quantiles, n_q, mean, median, mode,
-                                                          quant, log_prob);
-  return count_launch();
+  return (task_logits ? launch_tail<true> : launch_tail<false>)(
+      logits, task_logits, row_offset, n_tasks, n_est, S, K, src_bucket, src_share, cancel, borders, temperature,
+      avg_before, quantiles, n_q, mean, median, mode, quant, log_prob, st);
 }
 
 }  // namespace mmpfn

@@ -21,7 +21,7 @@ import torch
 from . import _lib
 from .model import B200PerFeatureTransformer, TrainContext
 
-__all__ = ["proba_device", "proba_from_logits", "B200InferenceEngine"]
+__all__ = ["proba_device", "proba_from_logits", "estimator_groups", "B200InferenceEngine"]
 
 
 def proba_device(logits: torch.Tensor, class_perms: Sequence[Optional[np.ndarray]], *, n_classes: int,
@@ -62,6 +62,16 @@ def proba_from_logits(logits: torch.Tensor, class_perms: Sequence[Optional[np.nd
     return out / out.sum(axis=1, keepdims=True)      # classifier.py:576 (after the D2H copy, like the reference)
 
 
+def estimator_groups(members) -> list:
+    """Estimators grouped by preprocessed width (-1: no table), widths ascending -> [(F, [member index])]: one
+    batched forward per group, whose label statistics are taken over the group's [len(idx), Ntr] block."""
+    groups = {}
+    for i, m in enumerate(members):
+        F = -1 if m["X_train"] is None else m["X_train"].shape[1]
+        groups.setdefault(F, []).append(i)
+    return sorted(groups.items())
+
+
 class B200InferenceEngine:
     """Holds the per-estimator preprocessed training tables and runs all estimators per call.
 
@@ -78,13 +88,8 @@ class B200InferenceEngine:
         self.image_train = None if image_train is None else np.asarray(image_train, dtype=np.float32)
         self.cache_context = cache_context
         dev = model.device
-        # group estimators by preprocessed width: one batched forward per group
-        groups = {}
-        for i, m in enumerate(self.members):
-            F = -1 if m["X_train"] is None else m["X_train"].shape[1]
-            groups.setdefault(F, []).append(i)
         self.groups = []
-        for F, idx in sorted(groups.items()):
+        for F, idx in estimator_groups(self.members):
             Xtr = None
             if F >= 0:
                 Xtr = torch.from_numpy(np.stack([np.asarray(self.members[i]["X_train"], dtype=np.float32)

@@ -437,17 +437,20 @@ class B200PerFeatureTransformer:
         """One train pass and one test pass over batch entries of any sizes -> [logits [n_test, n_out]] in entry order.
 
         An entry is one (task, estimator) pair: a dict with ``X`` (float32 [n_train + n_test, F], train rows first, or
-        None), ``y`` (class ids [n_train]), ``n_train``, ``n_test`` and ``tok`` / ``tok_row`` / ``n_tok`` (image
-        tokens [rows, H, E] from ``stem_image`` of ``n_tok`` embeddings per row and the row of the entry's first
-        train row in it, or ``tok`` None).  The pass
+        None), ``y`` (class ids [n_train], or float targets for a regression checkpoint), ``n_train``, ``n_test`` and
+        ``tok`` / ``tok_row`` / ``n_tok`` (image tokens [rows, H, E] from ``stem_image`` of ``n_tok`` embeddings per
+        row and the row of the entry's first train row in it, or ``tok`` None), and optionally ``y_mean`` (a float32
+        device tensor of one element: the label mean to use, as ``fit_context(label_stats=...)`` takes it).  Without
+        it the mean is that of the entry's own labels; for float targets torch's mean of a [k, n] block can change in
+        the last bit with k, so callers that must match a forward over a group of entries pass the group's means.
+        The pass
         has the row capacity of its largest entry; the other entries' rows up to it are pad rows, kept exactly zero
         (include/mmpfn_b200.h, "ragged" passes), so every entry's logits are bit-identical to ``fit_context`` +
         ``predict_with_context`` over that entry alone (the stem statistics see its train and test rows).  Entries of
         equal T form one segment (at most ``MMPFN_MAX_SEGMENTS``); a pass whose entries all have the capacity passes
         no count arrays, i.e. runs the kernels of the equal-shape passes.  ``final_states`` (a list) receives, for the
         train pass and then the test pass, ``(state [B_i, S, T_i, E], [entry index])`` per segment after the layers."""
-        if getattr(self.w, "regression", False):
-            raise ValueError("ragged passes serve classification entries (class-id labels)")
+        regression = getattr(self.w, "regression", False)
         dev = self.device
         T_of = [self.entry_tokens(None if e["X"] is None else e["X"].shape[1],
                                   0 if e["tok"] is None else e["n_tok"]) for e in entries]
@@ -490,23 +493,33 @@ class B200PerFeatureTransformer:
                 for k, j in enumerate(js):
                     stats_of[j] = (stats, k)
                     X_all[j] = (xa, k)
-            # label statistics per entry on its own labels (torch's mean over a [k, n] block is per row; the
-            # presence mask is exact integer work)
+            # label statistics per entry on its own labels: the mean of class ids over a [k, n] block is exact, so
+            # entries of equal n share a block; float targets are averaged one entry per block (the presence mask
+            # is exact integer work)
             y_mean = torch.empty(len(order), dtype=torch.float32, device=dev)
-            by_n = {}
+            by_n, given = {}, []
             for k, j in enumerate(order):
-                by_n.setdefault(entries[j]["n_train"], []).append(k)
+                if entries[j].get("y_mean") is not None:
+                    given.append(k)
+                else:
+                    by_n.setdefault((entries[j]["n_train"], k if regression else -1), []).append(k)
+            if given:
+                y_mean[torch.tensor(given, device=dev)] = torch.cat([entries[order[k]]["y_mean"].reshape(1)
+                                                                     for k in given])
             ys = [np.asarray(entries[j]["y"]) for j in order]
-            for n, ks in by_n.items():
+            for ks in by_n.values():
                 y_blk = torch.from_numpy(np.stack([ys[k] for k in ks]).astype(np.float32)).to(dev)
                 y_mean[torch.tensor(ks, device=dev)] = y_blk.mean(dim=1)
-            masks = []
-            for y in ys:
-                yl = y.astype(np.int64)
-                if not np.array_equal(yl, y) or yl.min() < 0 or yl.max() > 62:
-                    raise ValueError("labels must be integer class ids in [0, 62]")
-                masks.append(int(np.bitwise_or.reduce(np.left_shift(np.int64(1), np.unique(yl)))))
-            y_mask = torch.tensor(masks, dtype=torch.int64, device=dev)
+            if regression:
+                y_mask = torch.full((len(order),), self.REGRESSION_MASK, dtype=torch.int64, device=dev)
+            else:
+                masks = []
+                for y in ys:
+                    yl = y.astype(np.int64)
+                    if not np.array_equal(yl, y) or yl.min() < 0 or yl.max() > 62:
+                        raise ValueError("labels must be integer class ids in [0, 62]")
+                    masks.append(int(np.bitwise_or.reduce(np.left_shift(np.int64(1), np.unique(yl)))))
+                y_mask = torch.tensor(masks, dtype=torch.int64, device=dev)
             y_tr = np.zeros((len(order), S_tr), dtype=np.float32)
             for k, y in enumerate(ys):
                 y_tr[k, :len(y)] = y

@@ -31,11 +31,12 @@ import numpy as np
 import torch
 from sklearn.preprocessing import LabelEncoder
 
-from .engine import proba_from_logits
+from .engine import estimator_groups, proba_from_logits
 from .model import B200PerFeatureTransformer
 from .preprocessing import RECIPES, fit_transform_all, make_members, transform_all
+from .regressor import bar_tail_tasks_device, check_borders, format_result, output_request, prepare_regression
 
-__all__ = ["predict_proba_tasks", "plan_passes", "shard_tasks", "gather_task_results"]
+__all__ = ["predict_proba_tasks", "predict_regression_tasks", "plan_passes", "shard_tasks", "gather_task_results"]
 
 MAX_SEGMENTS = 8              # distinct token counts per pass (MMPFN_MAX_SEGMENTS)
 MAX_PAD_FRACTION = 0.25       # padded tokens of a pass over all its tokens
@@ -104,42 +105,28 @@ def _prepare(task: dict, n_estimators: int, random_state, recipes):
     train = fit_transform_all(members, X, yi)
     test = transform_all(members, Xte)
 
-    def img(a):
-        if a is None:
-            return None
-        a = np.asarray(a, dtype=np.float32)
-        return a[:, None] if a.ndim == 2 else a
-    itr, ite = img(task.get("img_train")), img(task.get("img_test"))
+    itr, ite = _images(task)
     n_te = len(Xte) if Xte is not None else len(ite)
     return dict(members=members, train=train, test=test, img_train=itr, img_test=ite, n_classes=n_cls, counts=counts,
                 classes=enc.classes_, n_train=len(y), n_test=n_te)
 
 
-def predict_proba_tasks(model: B200PerFeatureTransformer, tasks: Sequence[dict], *, n_estimators: int = 4,
-                        random_state=0, softmax_temperature: float = 0.9, average_before_softmax: bool = False,
-                        balance_probabilities: bool = False, recipes=RECIPES, indices: Optional[Sequence[int]] = None,
-                        n_jobs: int = 1, timings: Optional[dict] = None):
-    """``tasks``: dicts with ``X_train, img_train, y_train, X_test, img_test`` (tables or embeddings may be
-    ``None`` like in ``MMPFNClassifier.fit``).  Returns ``{task index: float32 [Nte, n_classes]}`` for the
-    tasks in ``indices`` (default: all).  Tasks of any shapes share launches (``plan_passes``).  The per-task host work
-    (fitting the members' quantile / SVD transforms) can run in ``n_jobs`` threads (it is mostly GIL-bound
-    sklearn glue: 16 threads measured slower than 1); ``timings`` (a dict) receives
-    the seconds spent in ``host_prepare`` and ``device``."""
+def _prepare_all(indices, prepare, n_jobs):
     import os
-    import time
     from concurrent.futures import ThreadPoolExecutor
-    indices = list(range(len(tasks))) if indices is None else list(indices)
-    dev = model.device
-    t0 = time.perf_counter()
     workers = (os.cpu_count() or 1) if n_jobs in (-1, None) else max(1, int(n_jobs))
     workers = min(workers, max(1, len(indices)))
     if workers > 1:
         with ThreadPoolExecutor(workers) as pool:
-            prepared = dict(zip(indices, pool.map(lambda i: _prepare(tasks[i], n_estimators, random_state, recipes),
-                                                  indices)))
-    else:
-        prepared = {i: _prepare(tasks[i], n_estimators, random_state, recipes) for i in indices}
-    t1 = time.perf_counter()
+            return dict(zip(indices, pool.map(prepare, indices)))
+    return {i: prepare(i) for i in indices}
+
+
+def _task_logits(model: B200PerFeatureTransformer, prepared: dict, indices, n_estimators: int, y_means=None) -> dict:
+    """The device part shared by the task functions: one image-stem pass per embedding-token count, the planned
+    ragged passes -> ``{task index: [logits [n_test, n_out] per estimator]}`` (views into the passes' decoder
+    outputs).  ``y_means``: ``{task index: [label mean per estimator]}`` (one-element device tensors) or None."""
+    dev = model.device
     # one image-stem pass per embedding-token count over the rows of all its tasks
     tok_of = {}
     by_ntok = {}
@@ -162,7 +149,7 @@ def predict_proba_tasks(model: B200PerFeatureTransformer, tasks: Sequence[dict],
             # the stem statistics see train and test rows (the reference's joint forward, encoders.py:515, :615)
             X_all = None if X is None else np.concatenate([X, pr["test"][e]]).astype(np.float32, copy=False)
             entries.append(dict(X=X_all, y=pr["train"][e][1], n_train=pr["n_train"], n_test=pr["n_test"], tok=tok,
-                                tok_row=row, n_tok=n_tok))
+                                tok_row=row, n_tok=n_tok, y_mean=None if y_means is None else y_means[i][e]))
             owner.append((i, e))
     shapes = [(en["n_train"], en["n_test"],
                model.entry_tokens(None if en["X"] is None else en["X"].shape[1], en["n_tok"])) for en in entries]
@@ -171,6 +158,26 @@ def predict_proba_tasks(model: B200PerFeatureTransformer, tasks: Sequence[dict],
         for k, lg in zip(ps, model.forward_ragged([entries[k] for k in ps])):
             i, e = owner[k]
             logits[i][e] = lg
+    return logits
+
+
+def predict_proba_tasks(model: B200PerFeatureTransformer, tasks: Sequence[dict], *, n_estimators: int = 4,
+                        random_state=0, softmax_temperature: float = 0.9, average_before_softmax: bool = False,
+                        balance_probabilities: bool = False, recipes=RECIPES, indices: Optional[Sequence[int]] = None,
+                        n_jobs: int = 1, timings: Optional[dict] = None):
+    """``tasks``: dicts with ``X_train, img_train, y_train, X_test, img_test`` (tables or embeddings may be
+    ``None`` like in ``MMPFNClassifier.fit``).  Returns ``{task index: float32 [Nte, n_classes]}`` for the
+    tasks in ``indices`` (default: all).  Tasks of any shapes share launches (``plan_passes``).  The per-task host work
+    (fitting the members' quantile / SVD transforms) can run in ``n_jobs`` threads (it is mostly GIL-bound
+    sklearn glue: 16 threads measured slower than 1); ``timings`` (a dict) receives
+    the seconds spent in ``host_prepare`` and ``device``."""
+    import time
+    indices = list(range(len(tasks))) if indices is None else list(indices)
+    dev = model.device
+    t0 = time.perf_counter()
+    prepared = _prepare_all(indices, lambda i: _prepare(tasks[i], n_estimators, random_state, recipes), n_jobs)
+    t1 = time.perf_counter()
+    logits = _task_logits(model, prepared, indices, n_estimators)
     out = {}
     for i in indices:
         pr = prepared[i]
@@ -184,3 +191,103 @@ def predict_proba_tasks(model: B200PerFeatureTransformer, tasks: Sequence[dict],
         timings["host_prepare"] = t1 - t0
         timings["device"] = time.perf_counter() - t1
     return out
+
+
+def _images(task: dict):
+    def img(a):
+        if a is None:
+            return None
+        a = np.asarray(a, dtype=np.float32)
+        return a[:, None] if a.ndim == 2 else a
+    return img(task.get("img_train")), img(task.get("img_test"))
+
+
+def _prepare_regression_task(i: int, task: dict, g: np.ndarray, n_estimators: int, random_state) -> dict:
+    """``MMPFNRegressor.fit``'s host work for task ``i`` (``prepare_regression``) plus its test tables."""
+    X = None if task.get("X_train") is None else np.asarray(task["X_train"], dtype=np.float32)
+    Xte = None if task.get("X_test") is None else np.asarray(task["X_test"], dtype=np.float32)
+    itr, ite = _images(task)
+    if X is None and itr is None:
+        raise ValueError(f"task {i}: needs a table X_train, an embedding img_train, or both")
+    try:
+        prep = prepare_regression(X, task["y_train"], g, n_estimators=n_estimators, random_state=random_state)
+    except ValueError as exc:
+        raise ValueError(f"task {i}: {exc}") from exc
+    n_te = len(Xte) if Xte is not None else len(ite)
+    prep.update(train=[(t["X_train"], t["y_train"]) for t in prep["tables"]], test=transform_all(prep["members"], Xte),
+                img_train=itr, img_test=ite, n_train=len(prep["tables"][0]["y_train"]), n_test=n_te)
+    return prep
+
+
+def predict_regression_tasks(model: B200PerFeatureTransformer, borders, tasks: Sequence[dict], *,
+                             n_estimators: int = 4, random_state=0, softmax_temperature: float = 0.9,
+                             average_before_softmax: bool = False, output_type: str = "mean", quantiles=None,
+                             indices: Optional[Sequence[int]] = None, n_jobs: int = 1,
+                             timings: Optional[dict] = None) -> dict:
+    """Many regression tasks in shared passes and ONE bar-distribution tail launch.
+
+    ``model``: a regression checkpoint's ``B200PerFeatureTransformer``; ``borders``: that checkpoint's
+    ``criterion.borders`` (``weights.load_borders``; the model does not hold them).  ``tasks``: the dicts of
+    ``predict_proba_tasks`` with float ``y_train``.  Returns ``{task index: result}`` for the tasks in ``indices``
+    (default: all), each exactly what ``MMPFNRegressor(n_estimators=..., random_state=...).fit(...).predict(...,
+    output_type=..., quantiles=...)`` returns for that task alone when the regressor's model is built like ``model``
+    (its seed ``int(random_state)``, ``outlier_std`` 12): arrays, a list of quantile arrays, or the "main" / "full"
+    dicts with the task's own log P and borders G.
+
+    Each task's host work (``prepare_regression``: target checks, transforms, members, border maps) runs in
+    ``n_jobs`` threads.  The label mean of each entry is taken over the estimator groups the regressor's engine
+    forms (``estimator_groups``), so the target token matches in every bit.  Every pass's logits stay on the device
+    until the tail: sum over tasks of n_estimators * n_test * K * 4 bytes (about 1 GB for 32 tasks x 8 estimators x
+    200 test rows x 5000 buckets).  ``timings`` (a dict) receives the seconds of ``host_prepare``, ``device`` (to
+    the host copies inclusive) and ``tail`` (the tail launch alone, CUDA events)."""
+    import time
+    if not getattr(model.w, "regression", False):
+        raise ValueError("model holds a classification checkpoint; use predict_proba_tasks")
+    g = check_borders(borders, model.geom.n_out)
+    K = len(g) - 1
+    if K > 8192:
+        raise ValueError(f"{K} buckets: the bar-distribution tail supports at most 8192")
+    want, qs = output_request(output_type, quantiles)
+    indices = list(range(len(tasks))) if indices is None else list(indices)
+    dev = model.device
+    t0 = time.perf_counter()
+    prepared = _prepare_all(indices, lambda i: _prepare_regression_task(i, tasks[i], g, n_estimators, random_state),
+                            n_jobs)
+    t1 = time.perf_counter()
+    y_means = {}
+    for i in indices:
+        tables = prepared[i]["tables"]
+        y_means[i] = [None] * n_estimators
+        for _, idx in estimator_groups(tables):
+            ytr = torch.from_numpy(np.stack([np.asarray(tables[e]["y_train"], dtype=np.float32) for e in idx])).to(dev)
+            y_mean, _ = model.label_stats(ytr)
+            for k, e in enumerate(idx):
+                y_means[i][e] = y_mean[k:k + 1]
+    logits = _task_logits(model, prepared, indices, n_estimators, y_means)
+    to_dev = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(dev)       # noqa: E731
+    cancel = np.stack([prepared[i]["cancel"] for i in indices])
+    ev = [torch.cuda.Event(enable_timing=True) for _ in range(2)] if timings is not None else None
+    args = (to_dev(np.stack([prepared[i]["src_bucket"] for i in indices])),
+            to_dev(np.stack([prepared[i]["src_share"] for i in indices])),
+            to_dev(cancel.astype(np.uint8)) if cancel.any() else None,
+            to_dev(np.stack([prepared[i]["target_borders"] for i in indices]).astype(np.float32)))
+    q_dev = to_dev(qs.astype(np.float32)) if "quantiles" in want else None
+    if ev is not None:
+        ev[0].record()
+    out = bar_tail_tasks_device([logits[i] for i in indices], *args, softmax_temperature=softmax_temperature,
+                                average_before_softmax=average_before_softmax, quantiles=q_dev, outputs=want)
+    if ev is not None:
+        ev[1].record()
+    ro = out.pop("row_offset")
+    host = {k: v.cpu().numpy() for k, v in out.items()}
+    res = {}
+    for n, i in enumerate(indices):
+        r0, r1 = int(ro[n]), int(ro[n + 1])
+        part = {k: np.array(v[..., r0:r1] if k == "quantiles" else v[r0:r1]) for k, v in host.items()}
+        res[i] = format_result(part, output_type, prepared[i]["target_borders"])
+    if timings is not None:
+        torch.cuda.synchronize(dev)
+        timings["host_prepare"] = t1 - t0
+        timings["device"] = time.perf_counter() - t1
+        timings["tail"] = ev[0].elapsed_time(ev[1]) / 1e3
+    return res
