@@ -212,6 +212,7 @@ int launch_tc_item_attn(const TcItemAttn& p, cudaStream_t st);
 // ---- stem / tail (kernels_stem.cu) -----------------------------------------------------------
 // Statistics block per estimator, indexed by COMPACTED slot c = g*fpg + j (encoders.py:102-130):
 //   src[Fp] (source column stored as float, -1 = empty slot) | fill | lo | hi | mean | std | scale[G]
+// An empty slot holds the statistics of the zero column the reference pads the group with.
 struct TabStatsLayout {
   int Fp, G;
   __host__ __device__ int src() const { return 0; }

@@ -155,6 +155,19 @@ __global__ void __launch_bounds__(256) tab_fit_kernel(const float* __restrict__ 
       int diff = 0;
       for (int i = 1 + threadIdx.x; i < S; i += blockDim.x) diff |= !(x3(i) == v0);
       slot_varies = block_any(diff, &s_flag);
+    } else {
+      // an empty slot is the zero column select_features pads the group with (encoders.py:113-126), and the steps
+      // above see it as such: fill 0, bounds 0, z-norm mean 0 / std 1e-20 (n_train == 1: std 1 and, with the outlier
+      // step on, NaN bounds from the NaN std of one row).  Its normalised values are 0, or NaN with NaN bounds; NaN
+      // values count as varying (encoders.py:615)
+      if (!(n_sigma > 0.f && !isinf(n_sigma))) {
+        lo = -CUDART_INF_F;
+        hi = CUDART_INF_F;
+      } else if (n_train == 1) {
+        lo = hi = CUDART_NAN_F;
+      }
+      if (n_train == 1) stdv = 1.0f;
+      slot_varies = isnan(lo) && S > 1;
     }
     if (slot_varies) ++n_used;
     if (threadIdx.x == 0) {
@@ -207,16 +220,14 @@ __global__ void __launch_bounds__(kE) stem_tokens_kernel(
     __shared__ float cell_v[1024], cell_i[1024];                 // G * fpg <= 1024 cells per row (checked on launch)
     for (int slot = e; slot < G * fpg; slot += kE) {
       const int col = (int)st[L.src() + slot];
-      float v = 0.f, ind = 0.f;
-      if (col >= 0) {
-        const float raw = x[b * x_bstride + s * F + col];
-        ind = isnan(raw) ? -2.0f : (isinf(raw) ? (raw > 0 ? 2.0f : 4.0f) : 0.0f);
-        float t1 = fill_bad(raw, st[L.fill() + slot]);
-        t1 = soft_clip(t1, st[L.lo() + slot], st[L.hi() + slot]);
-        t1 = clip100((t1 - st[L.mean() + slot]) / st[L.stdv() + slot]);
-        v = t1 * st[L.scale() + slot / fpg];
-      }
-      cell_v[slot] = v;
+      // an empty slot (col < 0) is a zero column with its own statistics (tab_fit_kernel): it transforms to 0, or to
+      // NaN where those statistics are NaN
+      const float raw = col >= 0 ? x[b * x_bstride + s * F + col] : 0.f;
+      const float ind = isnan(raw) ? -2.0f : (isinf(raw) ? (raw > 0 ? 2.0f : 4.0f) : 0.0f);
+      float t1 = fill_bad(raw, st[L.fill() + slot]);
+      t1 = soft_clip(t1, st[L.lo() + slot], st[L.hi() + slot]);
+      t1 = clip100((t1 - st[L.mean() + slot]) / st[L.stdv() + slot]);
+      cell_v[slot] = t1 * st[L.scale() + slot / fpg];
       cell_i[slot] = ind;
     }
     __syncthreads();

@@ -48,6 +48,10 @@ def proba_device(logits: torch.Tensor, class_perms: Sequence[Optional[np.ndarray
     prior_d = None
     if balance_probabilities:
         cc = np.asarray(class_counts, dtype=np.float64)
+        if cc.shape != (width,):
+            # the reference's out * cc/cc.sum() (classifier.py:563-566) fails to broadcast; the kernel would read
+            # past the end of the prior
+            raise ValueError(f"{cc.size} class counts for {width} probability columns")
         prior_d = torch.from_numpy((cc / cc.sum()).astype(np.float32)).to(dev)
     proba = torch.empty((S, width), dtype=torch.float32, device=dev)
     _lib.check(lib.mmpfn_proba_tail(logits.data_ptr(), perm_d.data_ptr(), None if prior_d is None else prior_d.data_ptr(),

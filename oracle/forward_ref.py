@@ -57,6 +57,8 @@ def stem_tab_fit(xg, n_train, *, n_sigma=12.0):
     xg: [S, G, fpg] raw grouped features (NaN allowed).  Returns a dict.
     The "constant column" tests look at ALL rows given (encoders.py:515, :615); the other
     statistics use the first n_train rows (encoders.py:461, :710).
+    n_sigma None or inf: no outlier step (InferenceConfig.remove_outliers False, model/config.py:43, leaves it
+    out of the step list, model/loading.py:308-371); the bounds are -inf / +inf, which the soft clip passes through.
     """
     S = xg.shape[0]
     sel = (xg[1:] == xg[0]).sum(0) != (S - 1)                       # encoders.py:515
@@ -64,12 +66,16 @@ def stem_tab_fit(xg, n_train, *, n_sigma=12.0):
     fill = torch.nanmean(xc[:n_train], dim=0)                       # encoders.py:461
     x1 = _nan_fill(xc, fill)
     d = x1[:n_train]
-    mu, sd_ = _nanmean_clip(d), _nanstd(d)                          # encoders.py:148-150
-    lo, hi = mu - n_sigma * sd_, mu + n_sigma * sd_
-    d2 = d.clone()
-    d2[torch.logical_or(d2 > hi, d2 < lo)] = float("nan")           # encoders.py:152
-    mu, sd_ = _nanmean_clip(d2), _nanstd(d2)
-    lo, hi = mu - n_sigma * sd_, mu + n_sigma * sd_                 # encoders.py:157-158
+    if n_sigma is None or math.isinf(n_sigma):
+        # inf * sd would give NaN bounds wherever sd is 0 or NaN (a constant column, n_train == 1)
+        lo, hi = torch.full_like(fill, -math.inf), torch.full_like(fill, math.inf)
+    else:
+        mu, sd_ = _nanmean_clip(d), _nanstd(d)                      # encoders.py:148-150
+        lo, hi = mu - n_sigma * sd_, mu + n_sigma * sd_
+        d2 = d.clone()
+        d2[torch.logical_or(d2 > hi, d2 < lo)] = float("nan")       # encoders.py:152
+        mu, sd_ = _nanmean_clip(d2), _nanstd(d2)
+        lo, hi = mu - n_sigma * sd_, mu + n_sigma * sd_             # encoders.py:157-158
     x2 = _soft_clip(x1, lo, hi)
     mean = _nanmean_clip(x2[:n_train])                              # encoders.py:81-82
     std = _nanstd(x2[:n_train]) + 1e-20
@@ -153,8 +159,8 @@ def stem_y_apply(yy, st, w_y, b_y, regression=False):
     ind = torch.isnan(yy) * -2.0
     yy = torch.where(torch.isnan(yy), st["mean"], yy)
     if not regression:
-        yy = (yy[:, None] > st["uniq"][None]).sum(-1).to(torch.float32)   # class rank, encoders.py:961-964
-    return torch.stack([yy, ind.to(torch.float32)], dim=-1) @ w_y.T + b_y
+        yy = (yy[:, None] > st["uniq"][None]).sum(-1).to(yy.dtype)         # class rank, encoders.py:961-964
+    return torch.stack([yy, ind.to(yy.dtype)], dim=-1) @ w_y.T + b_y
 
 
 # ---------------------------------------------------------------------------------------------
