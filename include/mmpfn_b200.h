@@ -36,7 +36,7 @@
 extern "C" {
 #endif
 
-#define MMPFN_ABI_VERSION 1
+#define MMPFN_ABI_VERSION 2
 
 enum { MMPFN_OK = 0, MMPFN_EINVAL = -1, MMPFN_ENODEVICE = -2, MMPFN_ECUDA = -3, MMPFN_EUNSUPPORTED = -4 };
 enum { MMPFN_F32 = 0, MMPFN_BF16 = 1 };
@@ -148,41 +148,38 @@ int mmpfn_stem_tokens(const mmpfn_geometry* g, const mmpfn_weights* w, const flo
                       float* state_f32, uint16_t* state_bf16, int32_t* nan_flag, void* stream);
 
 /* ---- the 12 layers ------------------------------------------------------------------------- */
-/* Bytes of scratch mmpfn_layers_* need for a [B][S][T][E] state. */
-size_t mmpfn_layers_ws_bytes(const mmpfn_geometry* g, int B, int S, int T, int precision);
 /* Bytes of the K/V context of n_train rows: per layer, head-0 keys and values of the item
  * attention for every (estimator, token column) — the reference's "first head only" cache
  * (multi_head_attention.py:328-336, :467-470) with a layer axis in front. */
 size_t mmpfn_kv_bytes(const mmpfn_geometry* g, int B, int n_train, int T, int precision);
 
-/* Train rows: layer.py:272-457 with every row a train row (self-attention over items, all heads,
- * layer.py:363-372); writes the head-0 K/V context when kv != NULL.  state is updated in place. */
-int mmpfn_layers_train(const mmpfn_geometry* g, const mmpfn_weights* w, float* state_f32, uint16_t* state_bf16,
-                       int B, int S, int T, int precision, void* kv, void* workspace, size_t workspace_bytes,
-                       void* stream);
-/* Test rows: item attention reads the cached head-0 K/V of the n_train train rows for all six
- * query heads (layer.py:346-358, multi_head_attention.py:436-445). */
-int mmpfn_layers_test(const mmpfn_geometry* g, const mmpfn_weights* w, float* state_f32, uint16_t* state_bf16,
-                      int B, int S, int T, int n_train, int precision, const void* kv, void* workspace,
-                      size_t workspace_bytes, void* stream);
-
-/* Several estimator groups ("segments": same row count S, own batch B and token count T) through the layers
- * in one call, bf16 mode.  Their states are laid back to back in one buffer — segment i occupies
- * B_i*S*T_i token rows of 192, in list order — so the sublayers that work on the flat token axis (QKV and
- * output projections + LayerNorm, MLP) launch once for all segments; the attentions launch per segment.
- * kv[i]: segment i's context (mmpfn_kv_bytes(B_i, n_train, T_i)); written by the train pass (may be NULL
- * there), read by the test pass.  Same results as one mmpfn_layers_train / _test call per segment. */
+/* Whole passes through the 12 layers (layer.py:272-457), both precisions; state is updated in place.
+ *  - Train pass: every row is a train row (self-attention over items, all heads, layer.py:363-372); writes the
+ *    head-0 K/V context of segment i to kv[i] when kv[i] != NULL.
+ *  - Test pass: the item attention reads the cached head-0 K/V of the n_train train rows for all six query heads
+ *    (layer.py:346-358, multi_head_attention.py:436-445); every kv[i] is required.
+ * A call takes a list of estimator groups ("segments": same row count S, own batch B_i and token count T_i).  Their
+ * states are laid back to back in one buffer — segment i occupies B_i*S*T_i token rows of 192, in list order —
+ * and kv[i] is segment i's context, mmpfn_kv_bytes(B_i, n_train, T_i, precision).  One segment {B, T} is the plain
+ * pass over a [B][S][T][E] state.  bf16: the sublayers that work on the flat token axis (QKV and output projections
+ * + LayerNorm, MLP) launch once for all segments, the attentions per segment; fp32: one segment after another.
+ * Every segment's result is that of a call over that segment alone.  state_bf16 is unused (may be NULL) in
+ * MMPFN_F32.
+ * n_rows / n_ctx: per-entry row counts (device int32, see "per-entry row counts" below), or NULL = every entry
+ * uses all S rows (and all n_train context rows).  With counts, entry b's item attention (layer.py:341-379) runs
+ * over its own rows only. */
 #define MMPFN_MAX_SEGMENTS 8
 typedef struct mmpfn_segment {
   int32_t B, T;
 } mmpfn_segment;
-size_t mmpfn_layers_multi_ws_bytes(const mmpfn_geometry* g, const mmpfn_segment* segs, int n_seg, int S);
-int mmpfn_layers_train_multi(const mmpfn_geometry* g, const mmpfn_weights* w, float* state_f32, uint16_t* state_bf16,
-                             const mmpfn_segment* segs, int n_seg, int S, void* const* kv, void* workspace,
+size_t mmpfn_layers_ragged_ws_bytes(const mmpfn_geometry* g, const mmpfn_segment* segs, int n_seg, int S, int precision);
+int mmpfn_layers_train_ragged(const mmpfn_geometry* g, const mmpfn_weights* w, float* state_f32, uint16_t* state_bf16,
+                              const mmpfn_segment* segs, int n_seg, int S, const int32_t* n_rows, int precision,
+                              void* const* kv, void* workspace, size_t workspace_bytes, void* stream);
+int mmpfn_layers_test_ragged(const mmpfn_geometry* g, const mmpfn_weights* w, float* state_f32, uint16_t* state_bf16,
+                             const mmpfn_segment* segs, int n_seg, int S, int n_train, const int32_t* n_rows,
+                             const int32_t* n_ctx, int precision, void* const* kv, void* workspace,
                              size_t workspace_bytes, void* stream);
-int mmpfn_layers_test_multi(const mmpfn_geometry* g, const mmpfn_weights* w, float* state_f32, uint16_t* state_bf16,
-                            const mmpfn_segment* segs, int n_seg, int S, int n_train, void* const* kv, void* workspace,
-                            size_t workspace_bytes, void* stream);
 
 /* The same passes over a RANGE of layers and with the K/V context addressed explicitly: what the multi-GPU
  * engine (multimodalpfn_b200/dist.py) needs to all-gather layer l's K/V under layers l+1.. and to let the test
@@ -191,7 +188,8 @@ int mmpfn_layers_test_multi(const mmpfn_geometry* g, const mmpfn_weights* w, flo
  * with c estimators back to back.  Train pass (train != 0): c = B, block of layer l written at
  * kv + l * layer_stride.  Test pass: estimator b of the segment = (rank b / slots, slot b % slots) lives in the block at
  * kv + l * layer_stride + rank * rank_stride with c = slots.  layer_stride 0 = blocks of consecutive layers are
- * adjacent; slots 0 = all B estimators in one block (rank_stride unused): then this is mmpfn_layers_*_multi.
+ * adjacent; slots 0 = all B estimators in one block (rank_stride unused): then this is the bf16 pass of
+ * mmpfn_layers_train_ragged / _test_ragged without counts.
  * Layers [layer_begin, layer_end) run; the state is carried in state_f32 / state_bf16 between calls. */
 typedef struct mmpfn_kv_segment {
   int32_t B, T;
@@ -227,8 +225,7 @@ int mmpfn_layers_run(const mmpfn_geometry* g, const mmpfn_weights* w, float* sta
  * Independent tasks of different sizes share one pass.  A batch ENTRY is one (task, estimator) pair; a pass has a
  * row capacity S (train pass: S train rows; test pass: S test rows against n_train context rows) and entry b uses
  * its first n_rows[b] rows (test pass: attends to its first n_ctx[b] context rows).  The counts are device int32
- * arrays with one element per entry (over all segments, in list order); NULL = every entry uses all rows, which runs
- * exactly the kernels of mmpfn_layers_*_multi / mmpfn_layers_train / _test.
+ * arrays with one element per entry (over all segments, in list order); NULL = every entry uses all rows.
  *
  * Pad-row contract: the rows between an entry's count and the capacity must be ZERO when a kernel reads them.
  * mmpfn_stem_tokens_ragged writes them as zeros, and the layers keep them exactly zero (no biases; LayerNorm of a
@@ -249,19 +246,6 @@ int mmpfn_stem_tokens_ragged(const mmpfn_geometry* g, const mmpfn_weights* w, co
                              const float* pos_emb, int B, int S, int F, int H_img, long long x_bstride,
                              long long y_bstride, const int64_t* img_offset, const int32_t* n_rows, float* state_f32,
                              uint16_t* state_bf16, int32_t* nan_flag, void* stream);
-/* The 12 layers over segments (layout of mmpfn_layers_train_multi: same S, own B_i and T_i, states back to back;
- * kv[i] = segment i's context, mmpfn_kv_bytes(B_i, n_train, T_i, precision)) with per-entry counts, both precisions:
- * layer.py:272-457 with the item attention (layer.py:341-379, multi_head_attention.py:436-445) of entry b over its
- * own rows only.  bf16: the segments share the row-wise launches; fp32: one segment after another.
- * state_bf16 is unused (may be NULL) in MMPFN_F32. */
-size_t mmpfn_layers_ragged_ws_bytes(const mmpfn_geometry* g, const mmpfn_segment* segs, int n_seg, int S, int precision);
-int mmpfn_layers_train_ragged(const mmpfn_geometry* g, const mmpfn_weights* w, float* state_f32, uint16_t* state_bf16,
-                              const mmpfn_segment* segs, int n_seg, int S, const int32_t* n_rows, int precision,
-                              void* const* kv, void* workspace, size_t workspace_bytes, void* stream);
-int mmpfn_layers_test_ragged(const mmpfn_geometry* g, const mmpfn_weights* w, float* state_f32, uint16_t* state_bf16,
-                             const mmpfn_segment* segs, int n_seg, int S, int n_train, const int32_t* n_rows,
-                             const int32_t* n_ctx, int precision, void* const* kv, void* workspace,
-                             size_t workspace_bytes, void* stream);
 
 /* ---- decoder + probability tail ------------------------------------------------------------ */
 /* transformer.py:392-396, :850-853: logits[b][s][:] = W2 gelu(W1 state[b][s][T-1] + b1) + b2.

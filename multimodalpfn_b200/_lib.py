@@ -63,18 +63,9 @@ SIGNATURES = {
     "mmpfn_stem_image": (c_int, [PG, PW, c_void_p, c_int, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
     "mmpfn_stem_tokens": (c_int, [PG, PW, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                   c_int, c_int, c_int, c_int, c_ll, c_ll, c_ll, c_void_p, c_void_p, c_void_p, c_void_p]),
-    "mmpfn_layers_ws_bytes": (c_size_t, [PG, c_int, c_int, c_int, c_int]),
     "mmpfn_kv_bytes": (c_size_t, [PG, c_int, c_int, c_int, c_int]),
-    "mmpfn_layers_multi_ws_bytes": (c_size_t, [PG, PS, c_int, c_int]),
-    "mmpfn_layers_train_multi": (c_int, [PG, PW, c_void_p, c_void_p, PS, c_int, c_int, PVP, c_void_p, c_size_t, c_void_p]),
-    "mmpfn_layers_test_multi": (c_int, [PG, PW, c_void_p, c_void_p, PS, c_int, c_int, c_int, PVP, c_void_p, c_size_t,
-                                        c_void_p]),
     "mmpfn_layers_run": (c_int, [PG, PW, c_void_p, c_void_p, PKS, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
                                  c_void_p, c_size_t, c_void_p]),
-    "mmpfn_layers_train": (c_int, [PG, PW, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
-                                   c_size_t, c_void_p]),
-    "mmpfn_layers_test": (c_int, [PG, PW, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
-                                  c_size_t, c_void_p]),
     "mmpfn_decode": (c_int, [PG, PW, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "mmpfn_proba_tail": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_float, c_int, c_void_p,
                                  c_void_p]),
@@ -139,7 +130,7 @@ def load(build_if_missing: bool = True):
         fn = getattr(lib, name)   # AttributeError here = header and library out of sync
         fn.restype = res
         fn.argtypes = args
-    if lib.mmpfn_abi_version() != 1:
+    if lib.mmpfn_abi_version() != 2:
         raise RuntimeError("libmmpfn_b200.so ABI version mismatch")
     _lib = lib
     return lib

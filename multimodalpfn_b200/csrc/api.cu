@@ -105,37 +105,26 @@ static int proj_gemm(const TcGemm& g, cudaStream_t st) {
   return launch_tc_rowgemm(g, st);
 }
 
-// workspace carving for the layers
+// scratch of the row-wise sublayers: the fp32 buffers are carved by carve(); in bf16 mode layers_run points
+// att_b / hid_b into its own workspace (carve_multi)
 struct LayerWs {
-  // fp32 mode
   float *qkv, *att, *hid, *tmp;
-  // bf16 mode
-  uint16_t *qkv_b, *att_b, *hid_b, *qi, *ki, *vti;
+  uint16_t *att_b, *hid_b;
   size_t bytes;
 };
-static LayerWs carve(void* base, long long M, int B, int S, int T, int precision) {
+// the fp32 workspace of a pass over M tokens
+static LayerWs carve(void* base, long long M) {
   LayerWs w{};
   size_t off = 0;
   auto take = [&](size_t bytes) {
     char* p = base ? (char*)base + off : nullptr;
     off += align_up(bytes, 1024);
-    return (void*)p;
+    return (float*)p;
   };
-  if (precision == MMPFN_F32) {
-    w.qkv = (float*)take((size_t)M * 3 * kE * 4);
-    w.att = (float*)take((size_t)M * kE * 4);
-    w.hid = (float*)take((size_t)M * kHid * 4);
-    w.tmp = (float*)take((size_t)M * kE * 4);
-  } else {
-    const size_t plane = (size_t)B * T * kH * kv_pad(S) * kD * 2;
-    // qkv (features) and hid (MLP) are never live together: share one buffer
-    w.hid_b = (uint16_t*)take((size_t)M * kHid * 2);
-    w.qkv_b = w.hid_b;
-    w.att_b = (uint16_t*)take((size_t)M * kE * 2);
-    w.qi = (uint16_t*)take(plane);
-    w.ki = (uint16_t*)take(plane);
-    w.vti = (uint16_t*)take(plane);
-  }
+  w.qkv = take((size_t)M * 3 * kE * 4);
+  w.att = take((size_t)M * kE * 4);
+  w.hid = take((size_t)M * kHid * 4);
+  w.tmp = take((size_t)M * kE * 4);
   w.bytes = off;
   return w;
 }
@@ -345,36 +334,22 @@ int mmpfn_stem_tokens_ragged(const mmpfn_geometry* g, const mmpfn_weights* w, co
                             (const long long*)img_offset, n_rows);
 }
 
-size_t mmpfn_layers_ws_bytes(const mmpfn_geometry* g, int B, int S, int T, int precision) {
-  if (check_geometry(g) != MMPFN_OK) return 0;
-  return carve(nullptr, (long long)B * S * T, B, S, T, precision).bytes;
-}
-
 size_t mmpfn_kv_bytes(const mmpfn_geometry* g, int B, int n_train, int T, int precision) {
   if (check_geometry(g) != MMPFN_OK) return 0;
   if (precision == MMPFN_F32) return (size_t)g->nlayers * B * T * n_train * 2 * kD * 4;
   return (size_t)g->nlayers * B * T * kv_pad(n_train) * 2 * kD * 2;
 }
 
-// One layer's two row-wise sublayers shared by the train and the test pass.
-static int feature_attention(const LayerW& lw, float* state, uint16_t* state_b, long long M, long long n_seq, int T,
-                             int precision, const LayerWs& ws, cudaStream_t st) {
-  if (precision == MMPFN_F32) {
-    MMPFN_TRY(launch_sgemm(gemm(state, kE, lw.fqkv, kE, nullptr, ws.qkv, 3 * kE, (int)M, 3 * kE, kE), EPI_NONE, st));
-    MMPFN_TRY(launch_feat_attn_f32(ws.qkv, ws.att, n_seq, T, st));
-    MMPFN_TRY(launch_sgemm(gemm(ws.att, kE, lw.fout, kE, nullptr, ws.tmp, kE, (int)M, kE, kE), EPI_NONE, st));
-    return launch_layernorm(ws.tmp, state, nullptr, nullptr, M, kE, state, nullptr, st);
-  }
-  TcGemm a{};
-  a.A = state_b; a.W = lw.fqkv_b; a.M = (int)M; a.N = 3 * kE; a.K = kE; a.epi = TC_EPI_BF16; a.out_bf16 = ws.qkv_b;
-  MMPFN_TRY(proj_gemm(a, st));
-  MMPFN_TRY(launch_feat_attn_bf16(ws.qkv_b, ws.att_b, n_seq, T, st));
-  TcGemm o{};
-  o.A = ws.att_b; o.W = lw.fout_b; o.M = (int)M; o.N = kE; o.K = kE; o.epi = TC_EPI_RESID_LN;
-  o.resid_f32 = state; o.ln_bf16 = state_b;
-  return proj_gemm(o, st);
+// The feature sublayer of the fp32 passes (layers_f32); layers_run has its own, per segment.
+static int feature_attention(const LayerW& lw, float* state, long long M, long long n_seq, int T, const LayerWs& ws,
+                             cudaStream_t st) {
+  MMPFN_TRY(launch_sgemm(gemm(state, kE, lw.fqkv, kE, nullptr, ws.qkv, 3 * kE, (int)M, 3 * kE, kE), EPI_NONE, st));
+  MMPFN_TRY(launch_feat_attn_f32(ws.qkv, ws.att, n_seq, T, st));
+  MMPFN_TRY(launch_sgemm(gemm(ws.att, kE, lw.fout, kE, nullptr, ws.tmp, kE, (int)M, kE, kE), EPI_NONE, st));
+  return launch_layernorm(ws.tmp, state, nullptr, nullptr, M, kE, state, nullptr, st);
 }
 
+// The MLP and the item attention's out-projection + LN, shared by the fp32 and the bf16 passes.
 static int mlp(const LayerW& lw, float* state, uint16_t* state_b, long long M, int precision, const LayerWs& ws,
                cudaStream_t st) {
   if (precision == MMPFN_F32) {
@@ -418,34 +393,6 @@ static int out_proj_ln(const LayerW& lw, float* state, uint16_t* state_b, long l
   return proj_gemm(o, st);
 }
 
-static int check_layers_args(const mmpfn_geometry* g, const mmpfn_weights* w, float* state, uint16_t* state_b, int B,
-                             int S, int T, int precision, void* workspace, size_t workspace_bytes, LayerWs* ws) {
-  MMPFN_TRY(check_geometry(g));
-  MMPFN_TRY(require_device());
-  if (!w || !w->layers_f32 || !state || B < 1 || S < 1 || T < 2 ||
-      (precision != MMPFN_F32 && precision != MMPFN_BF16)) {
-    set_error("layers: bad arguments (B %d S %d T %d precision %d)", B, S, T, precision);
-    return MMPFN_EINVAL;
-  }
-  if (precision == MMPFN_BF16 && (!state_b || !w->layers_bf16)) {
-    set_error("layers: bf16 mode needs the bf16 state shadow and bf16 weights");
-    return MMPFN_EINVAL;
-  }
-  // row counts are passed as int to the GEMM tiles
-  if ((long long)B * S * T > 2147483647LL) { set_error("layers: too many tokens"); return MMPFN_EUNSUPPORTED; }
-  *ws = carve(workspace, (long long)B * S * T, B, S, T, precision);
-  if (!workspace || workspace_bytes < ws->bytes) {
-    set_error("layers: workspace %zu < %zu bytes", workspace_bytes, ws->bytes);
-    return MMPFN_EINVAL;
-  }
-  return MMPFN_OK;
-}
-
-static int layers_run(const mmpfn_geometry* g, const mmpfn_weights* w, float* state, uint16_t* state_b,
-                      const mmpfn_kv_segment* ks, int n_seg, int S, int n_train, int train, int layer_begin,
-                      int layer_end, int phase, void* workspace, size_t workspace_bytes, cudaStream_t st,
-                      const int* n_rows = nullptr, const int* n_ctx = nullptr);
-
 // The fp32 (parity mode) passes over one [B][S][T] state.  train != 0: self-attention over the S rows, head-0 K/V
 // written to kv (may be NULL); else the S rows attend to the n_train rows of the context kv.  n_rows / n_ctx (device
 // [B], or NULL = S / n_train): entry b's own row count in this pass and context rows of the test pass.
@@ -454,7 +401,7 @@ static int layers_f32(const mmpfn_geometry* g, const mmpfn_weights* w, float* st
   const long long M = (long long)B * S * T;
   for (int l = 0; l < g->nlayers; ++l) {
     const LayerW lw = layer_w(w, l);
-    MMPFN_TRY(feature_attention(lw, state, nullptr, M, (long long)B * S, T, MMPFN_F32, ws, st));
+    MMPFN_TRY(feature_attention(lw, state, M, (long long)B * S, T, ws, st));
     ItemAttnF32 a{};
     a.out = ws.att;
     a.o_outer = (long long)S * T * kE; a.o_inner = kE; a.o_row = (long long)T * kE;
@@ -483,34 +430,6 @@ static int layers_f32(const mmpfn_geometry* g, const mmpfn_weights* w, float* st
     MMPFN_TRY(mlp(lw, state, nullptr, M, MMPFN_F32, ws, st));
   }
   return MMPFN_OK;
-}
-
-int mmpfn_layers_train(const mmpfn_geometry* g, const mmpfn_weights* w, float* state, uint16_t* state_b, int B, int S,
-                       int T, int precision, void* kv, void* workspace, size_t workspace_bytes, void* stream) {
-  LayerWs ws;
-  MMPFN_TRY(check_layers_args(g, w, state, state_b, B, S, T, precision, workspace, workspace_bytes, &ws));
-  cudaStream_t st = (cudaStream_t)stream;
-  if (precision == MMPFN_BF16) {      // one segment of the general bf16 pass (same workspace layout)
-    mmpfn_kv_segment k{};
-    k.B = B; k.T = T; k.kv = kv;
-    return layers_run(g, w, state, state_b, &k, 1, S, 0, 1, 0, g->nlayers, 0, workspace, workspace_bytes, st);
-  }
-  return layers_f32(g, w, state, B, S, T, 0, 1, kv, nullptr, nullptr, ws, st);
-}
-
-int mmpfn_layers_test(const mmpfn_geometry* g, const mmpfn_weights* w, float* state, uint16_t* state_b, int B, int S,
-                      int T, int n_train, int precision, const void* kv, void* workspace, size_t workspace_bytes,
-                      void* stream) {
-  LayerWs ws;
-  MMPFN_TRY(check_layers_args(g, w, state, state_b, B, S, T, precision, workspace, workspace_bytes, &ws));
-  if (!kv || n_train < 1) { set_error("layers_test: needs the K/V context of the train rows"); return MMPFN_EINVAL; }
-  cudaStream_t st = (cudaStream_t)stream;
-  if (precision == MMPFN_BF16) {
-    mmpfn_kv_segment k{};
-    k.B = B; k.T = T; k.kv = const_cast<void*>(kv);
-    return layers_run(g, w, state, state_b, &k, 1, S, n_train, 0, 0, g->nlayers, 0, workspace, workspace_bytes, st);
-  }
-  return layers_f32(g, w, state, B, S, T, n_train, 0, const_cast<void*>(kv), nullptr, nullptr, ws, st);
 }
 
 // ---- several estimator groups (segments) in one call -------------------------------------------------
@@ -547,21 +466,15 @@ static MultiWs carve_multi(void* base, const mmpfn_segment* segs, int n_seg, int
   return w;
 }
 static int check_segments(const mmpfn_segment* segs, int n_seg, int S, long long* M_total) {
-  if (!segs || n_seg < 1 || n_seg > MMPFN_MAX_SEGMENTS || S < 1) { set_error("layers_multi: bad segment list"); return MMPFN_EINVAL; }
+  if (!segs || n_seg < 1 || n_seg > MMPFN_MAX_SEGMENTS || S < 1) { set_error("layers: bad segment list"); return MMPFN_EINVAL; }
   long long m = 0;
   for (int i = 0; i < n_seg; ++i) {
-    if (segs[i].B < 1 || segs[i].T < 2) { set_error("layers_multi: bad segment %d (B %d T %d)", i, segs[i].B, segs[i].T); return MMPFN_EINVAL; }
+    if (segs[i].B < 1 || segs[i].T < 2) { set_error("layers: bad segment %d (B %d T %d)", i, segs[i].B, segs[i].T); return MMPFN_EINVAL; }
     m += (long long)segs[i].B * S * segs[i].T;
   }
-  if (m > 2147483647LL) { set_error("layers_multi: too many tokens"); return MMPFN_EUNSUPPORTED; }
+  if (m > 2147483647LL) { set_error("layers: too many tokens"); return MMPFN_EUNSUPPORTED; }
   *M_total = m;
   return MMPFN_OK;
-}
-
-size_t mmpfn_layers_multi_ws_bytes(const mmpfn_geometry* g, const mmpfn_segment* segs, int n_seg, int S) {
-  long long M = 0;
-  if (check_geometry(g) != MMPFN_OK || check_segments(segs, n_seg, S, &M) != MMPFN_OK) return 0;
-  return carve_multi(nullptr, segs, n_seg, S, M).bytes;
 }
 
 // One K/V context block per segment and layer: K0 [c][T][Np][32] then V0^T [c][T][32][Np] (bf16), c = the
@@ -603,7 +516,7 @@ static int layers_run(const mmpfn_geometry* g, const mmpfn_weights* w, float* st
   if (!workspace || workspace_bytes < ws.bytes) { set_error("layers_run: workspace %zu < %zu bytes", workspace_bytes, ws.bytes); return MMPFN_EINVAL; }
   const int Sp = kv_pad(Sa), Np = kv_pad(n_train);
   LayerWs flat{};
-  flat.hid_b = ws.hid_b; flat.qkv_b = ws.hid_b; flat.att_b = ws.att_b;
+  flat.hid_b = ws.hid_b; flat.att_b = ws.att_b;
 #ifdef MMPFN_DEBUG
   // tuning build only: MMPFN_FEAT_FUSED=0 takes the two-kernel form of the feature sublayer's first half
   static int feat_fused = -1;
@@ -703,35 +616,11 @@ static int layers_run(const mmpfn_geometry* g, const mmpfn_weights* w, float* st
   return MMPFN_OK;
 }
 
-static int layers_multi(const mmpfn_geometry* g, const mmpfn_weights* w, float* state, uint16_t* state_b,
-                        const mmpfn_segment* segs, int n_seg, int S, int n_train, int train, void* const* kv,
-                        void* workspace, size_t workspace_bytes, cudaStream_t st) {
-  if (!segs || !kv || n_seg < 1 || n_seg > MMPFN_MAX_SEGMENTS || !g) { set_error("layers_multi: bad segment list"); return MMPFN_EINVAL; }
-  mmpfn_kv_segment ks[MMPFN_MAX_SEGMENTS];
-  for (int i = 0; i < n_seg; ++i) {
-    ks[i] = mmpfn_kv_segment{};
-    ks[i].B = segs[i].B; ks[i].T = segs[i].T; ks[i].kv = kv[i];
-  }
-  return layers_run(g, w, state, state_b, ks, n_seg, S, n_train, train, 0, g->nlayers, 0, workspace, workspace_bytes, st);
-}
-
-int mmpfn_layers_train_multi(const mmpfn_geometry* g, const mmpfn_weights* w, float* state_f32, uint16_t* state_bf16,
-                             const mmpfn_segment* segs, int n_seg, int S, void* const* kv, void* workspace,
-                             size_t workspace_bytes, void* stream) {
-  return layers_multi(g, w, state_f32, state_bf16, segs, n_seg, S, 0, 1, kv, workspace, workspace_bytes, (cudaStream_t)stream);
-}
-
-int mmpfn_layers_test_multi(const mmpfn_geometry* g, const mmpfn_weights* w, float* state_f32, uint16_t* state_bf16,
-                            const mmpfn_segment* segs, int n_seg, int S, int n_train, void* const* kv, void* workspace,
-                            size_t workspace_bytes, void* stream) {
-  return layers_multi(g, w, state_f32, state_bf16, segs, n_seg, S, n_train, 0, kv, workspace, workspace_bytes, (cudaStream_t)stream);
-}
-
 int mmpfn_layers_run(const mmpfn_geometry* g, const mmpfn_weights* w, float* state_f32, uint16_t* state_bf16,
                      const mmpfn_kv_segment* segs, int n_seg, int S, int n_train, int train, int layer_begin,
                      int layer_end, int phase, void* workspace, size_t workspace_bytes, void* stream) {
   return layers_run(g, w, state_f32, state_bf16, segs, n_seg, S, n_train, train, layer_begin, layer_end, phase, workspace,
-                    workspace_bytes, (cudaStream_t)stream);
+                    workspace_bytes, (cudaStream_t)stream, nullptr, nullptr);
 }
 
 // ---- per-entry row counts ----------------------------------------------------------------------------
@@ -745,7 +634,7 @@ size_t mmpfn_layers_ragged_ws_bytes(const mmpfn_geometry* g, const mmpfn_segment
     const long long m = (long long)segs[i].B * S * segs[i].T;
     if (m > m_max) m_max = m;
   }
-  return carve(nullptr, m_max, 1, S, 2, MMPFN_F32).bytes;
+  return carve(nullptr, m_max).bytes;
 }
 
 static int layers_ragged(const mmpfn_geometry* g, const mmpfn_weights* w, float* state, uint16_t* state_b,
@@ -776,7 +665,7 @@ static int layers_ragged(const mmpfn_geometry* g, const mmpfn_weights* w, float*
   for (int i = 0; i < n_seg; ++i) {
     const int B = segs[i].B, T = segs[i].T;
     if (!train && !kv[i]) { set_error("layers_ragged: the test pass needs every segment's context"); return MMPFN_EINVAL; }
-    const LayerWs ws = carve(workspace, (long long)B * S * T, B, S, T, MMPFN_F32);
+    const LayerWs ws = carve(workspace, (long long)B * S * T);
     MMPFN_TRY(layers_f32(g, w, state + off * kE, B, S, T, n_train, train, kv[i], n_rows ? n_rows + entry : nullptr,
                          n_ctx ? n_ctx + entry : nullptr, ws, st));
     off += (long long)B * S * T;

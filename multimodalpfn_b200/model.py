@@ -211,7 +211,7 @@ class B200PerFeatureTransformer:
             img_bstride = img_tok.shape[1] * img_tok.shape[2] * img_tok.shape[3]
         T = G + H_img + 1
         E = self.geom.emsize
-        if out is not None:          # views into a buffer shared by several estimator groups (layers_*_multi)
+        if out is not None:          # views into a buffer shared by several estimator groups (``layers``)
             state, state_b = out
             assert tuple(state.shape) == (B, S, T, E) and state.is_contiguous()
         else:
@@ -225,38 +225,26 @@ class B200PerFeatureTransformer:
         return state, state_b
 
     # ------------------------------------------------------------------ layers / decoder
-    def layers_train(self, state, state_b, kv: Optional[torch.Tensor]):
-        B, S, T, _ = state.shape
-        nbytes = self.lib.mmpfn_layers_ws_bytes(self._g, B, S, T, self.precision)
-        ws = self._scratch("layers", nbytes)
-        _lib.check(self.lib.mmpfn_layers_train(self._g, self._w, state.data_ptr(), _ptr(state_b), B, S, T,
-                                               self.precision, _ptr(kv), ws.data_ptr(), nbytes, self._stream()),
-                   "mmpfn_layers_train")
-
-    def layers_test(self, state, state_b, kv: torch.Tensor, n_train: int):
-        B, S, T, _ = state.shape
-        nbytes = self.lib.mmpfn_layers_ws_bytes(self._g, B, S, T, self.precision)
-        ws = self._scratch("layers", nbytes)
-        _lib.check(self.lib.mmpfn_layers_test(self._g, self._w_test, state.data_ptr(), _ptr(state_b), B, S, T, n_train,
-                                              self.precision, kv.data_ptr(), ws.data_ptr(), nbytes, self._stream()),
-                   "mmpfn_layers_test")
-
-    def _layers_multi(self, state, state_b, segs, S: int, kvs, n_train: Optional[int]):
-        """``state`` / ``state_b``: flat [M_total, E] buffers holding the segments' [B_i, S, T_i, E] states back
-        to back; ``segs``: [(B_i, T_i)]; ``kvs``: one context tensor per segment."""
+    def layers(self, state, state_b, segs, S: int, kvs, *, n_train: Optional[int] = None, n_rows=None, n_ctx=None):
+        """The 12 layers, in place, over the states of ``segs`` ([(B_i, T_i)]) held back to back in ``state`` /
+        ``state_b`` (one segment: a [B, S, T, E] state).  ``kvs``: one K/V context per segment (None on the train pass:
+        not kept).  ``n_train=None``: the train pass, which writes the contexts; else the test pass against
+        ``n_train`` context rows.  ``n_rows`` / ``n_ctx``: per-entry counts (int32 device tensors) or None
+        (``mmpfn_layers_train_ragged`` / ``_test_ragged``)."""
         n = len(segs)
         arr = (_lib.Segment * n)(*[_lib.Segment(int(b), int(t)) for b, t in segs])
-        kvp = (C.c_void_p * n)(*[kv.data_ptr() for kv in kvs])
-        nbytes = self.lib.mmpfn_layers_multi_ws_bytes(self._g, arr, n, S)
+        kvp = (C.c_void_p * n)(*[_ptr(kv) for kv in kvs])
+        nbytes = self.lib.mmpfn_layers_ragged_ws_bytes(self._g, arr, n, S, self.precision)
         ws = self._scratch("layers", nbytes)
         if n_train is None:
-            _lib.check(self.lib.mmpfn_layers_train_multi(self._g, self._w, state.data_ptr(), state_b.data_ptr(), arr, n, S,
-                                                         kvp, ws.data_ptr(), nbytes, self._stream()),
-                       "mmpfn_layers_train_multi")
+            _lib.check(self.lib.mmpfn_layers_train_ragged(self._g, self._w, state.data_ptr(), _ptr(state_b), arr, n, S,
+                                                          _ptr(n_rows), self.precision, kvp, ws.data_ptr(), nbytes,
+                                                          self._stream()), "mmpfn_layers_train_ragged")
         else:
-            _lib.check(self.lib.mmpfn_layers_test_multi(self._g, self._w_test, state.data_ptr(), state_b.data_ptr(), arr, n, S,
-                                                        n_train, kvp, ws.data_ptr(), nbytes, self._stream()),
-                       "mmpfn_layers_test_multi")
+            _lib.check(self.lib.mmpfn_layers_test_ragged(self._g, self._w_test, state.data_ptr(), _ptr(state_b), arr, n,
+                                                         S, int(n_train), _ptr(n_rows), _ptr(n_ctx), self.precision,
+                                                         kvp, ws.data_ptr(), nbytes, self._stream()),
+                       "mmpfn_layers_test_ragged")
 
     def layers_run(self, state, state_b, segs, S: int, n_train: Optional[int], layer_begin: int, layer_end: int,
                    phase: int = 0, ws_key: str = ""):
@@ -280,7 +268,7 @@ class B200PerFeatureTransformer:
         arr = (_lib.KvSegment * n)(*[seg(s) for s in segs])
         plain = (_lib.Segment * n)(*[_lib.Segment(int(s["B"]), int(s["T"])) for s in segs])
         S_alloc = max([S] + [int(s.get("seg_rows", 0)) for s in segs]) if n_train is None else S
-        nbytes = self.lib.mmpfn_layers_multi_ws_bytes(self._g, plain, n, S_alloc)
+        nbytes = self.lib.mmpfn_layers_ragged_ws_bytes(self._g, plain, n, S_alloc, _lib.BF16)
         ws = self._scratch("layers" + ws_key, nbytes)
         _lib.check(self.lib.mmpfn_layers_run(self._g, self._w if n_train is None else self._w_test, state.data_ptr(),
                                              state_b.data_ptr(), arr, n, S,
@@ -381,7 +369,7 @@ class B200PerFeatureTransformer:
             state, state_b = self.embed(X_train, stats, img_tok_train, y_train, y_mean, y_mask, pos, B=B, S=n_train,
                                         F=F, x_bstride=n_train * F, y_bstride=n_train, nan_flag=flag)
             kv = self.alloc_kv(B, n_train, T)
-            self.layers_train(state, state_b, kv)
+            self.layers(state, state_b, [(B, T)], n_train, [kv])
             if check:
                 self._check_nan(flag)
             return TrainContext(B=B, n_train=n_train, F=F, T=T, n_tok=n_tok, kv=kv, tab_stats=stats, y_mean=y_mean,
@@ -406,7 +394,7 @@ class B200PerFeatureTransformer:
                                         nan_flag=flag)
             if state.shape[2] != ctx.T:
                 raise ValueError("test rows produce a different number of tokens than the context")
-            self.layers_test(state, state_b, ctx.kv, ctx.n_train)
+            self.layers(state, state_b, [(ctx.B, ctx.T)], n_test, [ctx.kv], n_train=ctx.n_train)
             logits = self.decode(state)
             if check:
                 self._check_nan(flag)
@@ -548,21 +536,12 @@ class B200PerFeatureTransformer:
                                           (d_tr if train else d_te), k0 + i0, flag)
                         i0 = i1
                     k0 += len(js)
-                seg_arr = (_lib.Segment * len(shapes))(*[_lib.Segment(b, T) for b, T in shapes])
-                kvp = (C.c_void_p * len(kvs))(*[kv.data_ptr() for kv in kvs])
-                nbytes = self.lib.mmpfn_layers_ragged_ws_bytes(self._g, seg_arr, len(shapes), S, self.precision)
-                ws = self._scratch("layers", nbytes)
                 if train:
-                    _lib.check(self.lib.mmpfn_layers_train_ragged(
-                        self._g, self._w, st.data_ptr(), _ptr(stb), seg_arr, len(shapes), S, _ptr(d_tr),
-                        self.precision, kvp, ws.data_ptr(), nbytes, self._stream()), "mmpfn_layers_train_ragged")
+                    self.layers(st, stb, shapes, S, kvs, n_rows=d_tr)
                     if final_states is not None:
                         final_states.extend(zip([v for v, _ in views], [js for _, js in segs]))
                 else:
-                    _lib.check(self.lib.mmpfn_layers_test_ragged(
-                        self._g, self._w_test, st.data_ptr(), _ptr(stb), seg_arr, len(shapes), S, S_tr, _ptr(d_te),
-                        _ptr(d_tr), self.precision, kvp, ws.data_ptr(), nbytes, self._stream()),
-                        "mmpfn_layers_test_ragged")
+                    self.layers(st, stb, shapes, S, kvs, n_train=S_tr, n_rows=d_te, n_ctx=d_tr)
                     for (T, js), (v, _) in zip(segs, views):
                         lg = self.decode(v)
                         if final_states is not None:
@@ -622,8 +601,8 @@ class B200PerFeatureTransformer:
     def fit_contexts(self, specs, *, nan_flag=None):
         """``fit_context`` for several estimator groups that share the train rows (same n_train) — specs:
         dicts with ``X_train [B, Ntr, F]``, ``y_train [B, Ntr]``, optional ``X_all``, ``img_tok_train``,
-        ``label_stats``.  Same results as one ``fit_context`` per group; the layers run as
-        ``mmpfn_layers_train_multi``."""
+        ``label_stats``.  Same results as one ``fit_context`` per group; the layers run as one pass over all
+        groups (``layers``)."""
         assert self.precision == _lib.BF16
         with torch.cuda.device(self.device):
             flag = nan_flag if nan_flag is not None else torch.zeros(1, dtype=torch.int32, device=self.device)
@@ -649,7 +628,7 @@ class B200PerFeatureTransformer:
                 self.embed(p["X"], p["stats"], p["tok"], p["y"], p["y_mean"], p["y_mask"], p["pos"], B=p["B"], S=n_train,
                            F=p["F"], x_bstride=n_train * p["F"], y_bstride=n_train, nan_flag=flag, out=v)
             kvs = [self.alloc_kv(p["B"], n_train, p["T"]) for p in prep]
-            self._layers_multi(st, stb, [(p["B"], p["T"]) for p in prep], n_train, kvs, None)
+            self.layers(st, stb, [(p["B"], p["T"]) for p in prep], n_train, kvs)
             return [TrainContext(B=p["B"], n_train=n_train, F=p["F"], T=p["T"], n_tok=0, kv=kv, tab_stats=p["stats"],
                                  y_mean=p["y_mean"], y_mask=p["y_mask"], pos_emb=p["pos"], precision=self.precision)
                     for p, kv in zip(prep, kvs)]
@@ -668,7 +647,7 @@ class B200PerFeatureTransformer:
                     raise ValueError("test tables do not match their contexts")
                 self.embed(X, c.tab_stats, img_tok_test, y_nan, c.y_mean, c.y_mask, c.pos_emb, B=c.B, S=n_test, F=c.F,
                            x_bstride=n_test * c.F, y_bstride=0, nan_flag=flag, out=v)
-            self._layers_multi(st, stb, [(c.B, c.T) for c in ctxs], n_test, [c.kv for c in ctxs], ctxs[0].n_train)
+            self.layers(st, stb, [(c.B, c.T) for c in ctxs], n_test, [c.kv for c in ctxs], n_train=ctxs[0].n_train)
             return [self.decode(v[0]) for v in views]
 
     def forward_batch(self, X_full, img_full, y_train, *, check=True, return_embeddings=False):

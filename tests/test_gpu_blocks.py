@@ -261,8 +261,8 @@ def _one_layer_model(precision, seed=3):
 
 @pytest.mark.parametrize("precision,tol", [("fp32", 2e-5), ("bf16", 0.06)])
 @pytest.mark.parametrize("B,S,T,n_test", [(1, 200, 7, 60), (2, 333, 12, 130), (1, 1100, 5, 257)])
-def test_single_layer_vs_oracle(precision, tol, B, S, T, n_test):
-    """layers_train (writes the K/V context) then layers_test on random O(1) states vs the
+def test_single_layer_pass_vs_oracle(precision, tol, B, S, T, n_test):
+    """The train pass (writes the K/V context) then the test pass on random O(1) states vs the
     oracle's layer_forward (layer.py:272-457)."""
     from oracle import forward_ref as R
     model, sd, geom = _one_layer_model(precision)
@@ -273,10 +273,10 @@ def test_single_layer_vs_oracle(precision, tol, B, S, T, n_test):
     st = tr.cuda().contiguous()
     stb = st.to(torch.bfloat16) if precision == "bf16" else None
     kv = model.alloc_kv(B, S, T)
-    model.layers_train(st, stb, kv)
+    model.layers(st, stb, [(B, T)], S, [kv])
     se = te.cuda().contiguous()
     seb = se.to(torch.bfloat16) if precision == "bf16" else None
-    model.layers_test(se, seb, kv, S)
+    model.layers(se, seb, [(B, T)], n_test, [kv], n_train=S)
     torch.cuda.synchronize()
     for b in range(B):
         ref_tr, kvr = R.layer_forward(tr[b], S, tsd, 0, want_kv=True)
@@ -289,8 +289,8 @@ def test_single_layer_vs_oracle(precision, tol, B, S, T, n_test):
 
 
 @pytest.mark.parametrize("seed", list(range(10)))
-def test_single_layer_random_shapes(seed):
-    """layers_train + layers_test at random ragged shapes (1-700 rows, 2-140 tokens, 1-3 estimators): tiles
+def test_single_layer_pass_random_shapes(seed):
+    """Train + test pass at random ragged shapes (1-700 rows, 2-140 tokens, 1-3 estimators): tiles
     that are mostly padding, key sets shorter than one 48-key tile, token counts that switch the feature
     attention between its register-tile sizes — bf16 path vs the oracle's layer_forward."""
     from oracle import forward_ref as R
@@ -309,8 +309,8 @@ def test_single_layer_random_shapes(seed):
     st, se = tr.cuda().contiguous(), te.cuda().contiguous()
     stb, seb = st.to(torch.bfloat16), se.to(torch.bfloat16)
     kv = model.alloc_kv(B, S, T)
-    model.layers_train(st, stb, kv)
-    model.layers_test(se, seb, kv, S)
+    model.layers(st, stb, [(B, T)], S, [kv])
+    model.layers(se, seb, [(B, T)], n_test, [kv], n_train=S)
     torch.cuda.synchronize()
     assert torch.isfinite(st).all() and torch.isfinite(se).all()
     for b in range(B):

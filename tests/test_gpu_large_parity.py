@@ -57,7 +57,7 @@ def test_ctx10k_vs_reference(precision):
 
 @pytest.mark.parametrize("gain", ["g1", "g3"])
 @pytest.mark.parametrize("precision", ["bf16", "fp32"])
-def test_layer50k_vs_reference(precision, gain):
+def test_layer50k_pass_vs_reference(precision, gain):
     """The 50 000-key axis of configs[3]: ONE layer (feature attention, item attention with 50 000 train
     rows as keys, MLP) on a [50 128 rows, T = 3] state; 64 train rows and 64 test rows of the output against
     the reference's own ``PerFeatureEncoderLayer`` modules (1042 key tiles accumulate per query).
@@ -77,8 +77,8 @@ def test_layer50k_vs_reference(precision, gain):
     tr_b = tr.to(torch.bfloat16) if bf else None
     te_b = te.to(torch.bfloat16) if bf else None
     kv = model.alloc_kv(1, n_tr, T)
-    model.layers_train(tr, tr_b, kv)
-    model.layers_test(te, te_b, kv, n_tr)
+    model.layers(tr, tr_b, [(1, T)], n_tr, [kv])
+    model.layers(te, te_b, [(1, T)], n_te, [kv], n_train=n_tr)
     out = torch.cat([tr[0], te[0]]).cpu().numpy()[cases.LAYER50K_ROWS]
     err = np.abs(out - g["out_rows"])
     print(f"[layer50k {gain} {precision}] max|err| train rows {err[:64].max():.3e}, test rows {err[64:].max():.3e}, "

@@ -212,7 +212,7 @@ def test_model_extreme_shapes_vs_oracle(n_tr, n_te, F, n_tok):
 
 @pytest.mark.parametrize("fit_mode", ["fit_preprocessors", "fit_with_cache"])
 def test_multi_group_pass_equals_per_group(fit_mode):
-    """Estimator groups of different token counts through mmpfn_layers_*_multi (flat sublayers launched once
+    """Estimator groups of different token counts as segments of one layer pass (flat sublayers launched once
     for all groups) vs one pass per group: identical logits, bit for bit."""
     from multimodalpfn_b200.classifier import MMPFNClassifier
     from multimodalpfn_b200.preprocessing import transform_all
