@@ -439,21 +439,19 @@ class ShardedEngine:
         tok_tr = tok_te = None
         if staged["img_test"] is not None:
             tok_tr, tok_te = eng.train_image_tokens(), m.stem_image(staged["img_test"])
-        out = [None] * len(self.members)
-        mine: Dict[int, TrainContext] = {}
-        for si, sub in enumerate(self.subs):
-            if sub.owner != self.rank:
-                continue
+        owned = [si for si, sub in enumerate(self.subs) if sub.owner == self.rank]
+        specs = []
+        for si in owned:
+            sub = self.subs[si]
             g = eng.groups[sub.group]
             Xtr = None if g["X_train"] is None else g["X_train"][sub.pos].contiguous()
             Xte = staged["X_test"][sub.group]
             Xte = None if Xte is None else Xte[sub.pos].contiguous()
             ls = g["label_stats"]
-            mine[si] = m.fit_context(Xtr, None, g["y_train"][sub.pos].contiguous(),
-                                     X_all=None if Xte is None else torch.cat([Xtr, Xte], dim=1),
-                                     img_tok_train=tok_tr, check=False,
-                                     label_stats=(ls[0][sub.pos].contiguous(), ls[1][sub.pos].contiguous()),
-                                     nan_flag=eng.nan_flag)
+            specs.append(dict(X_train=Xtr, y_train=g["y_train"][sub.pos].contiguous(),
+                              X_all=None if Xte is None else torch.cat([Xtr, Xte], dim=1), img_tok_train=tok_tr,
+                              label_stats=(ls[0][sub.pos].contiguous(), ls[1][sub.pos].contiguous())))
+        mine: Dict[int, TrainContext] = dict(zip(owned, m.fit_contexts(specs, nan_flag=eng.nan_flag))) if specs else {}
         ctxs: Dict[int, TrainContext] = {}
         for si, sub in enumerate(self.subs):
             g = eng.groups[sub.group]
@@ -471,9 +469,10 @@ class ShardedEngine:
                 c = mine[si]
                 src = [c.kv, c.y_mean, c.y_mask] + ([c.tab_stats] if G_ else [])
             got = broadcast_bundle(src, shapes, sub.owner, dev, self.group)
-            ctxs[si] = TrainContext(B=B, n_train=n_tr, F=F, T=T, n_tok=0, kv=got[0], tab_stats=got[3] if G_ else None,
+            ctxs[si] = TrainContext(B=B, n_train=n_tr, F=F, T=T, kv=got[0], tab_stats=got[3] if G_ else None,
                                     y_mean=got[1], y_mask=got[2], pos_emb=m.positional_embeddings(T - 1),
                                     precision=m.precision)
+        merged = []
         for gi, g in enumerate(eng.groups):
             subs = [(si, sub) for si, sub in enumerate(self.subs) if sub.group == gi]
             if len(subs) == 1:
@@ -492,10 +491,12 @@ class ShardedEngine:
                     if stats is not None:
                         stats[sub.pos] = c.tab_stats
                 kv = m.merge_kv([(ctxs[si].kv, sub.pos) for si, sub in subs], Bg, c0.n_train, c0.T)
-                ctx = TrainContext(B=Bg, n_train=c0.n_train, F=c0.F, T=c0.T, n_tok=0, kv=kv, tab_stats=stats,
+                ctx = TrainContext(B=Bg, n_train=c0.n_train, F=c0.F, T=c0.T, kv=kv, tab_stats=stats,
                                    y_mean=y_mean, y_mask=y_mask, pos_emb=c0.pos_emb, precision=m.precision)
-            lg = m.predict_with_context(ctx, staged["X_test"][gi], None, img_tok_test=tok_te, check=False,
-                                        nan_flag=eng.nan_flag)
+            merged.append(ctx)
+        lgs = m.predict_with_contexts(merged, staged["X_test"], img_tok_test=tok_te, nan_flag=eng.nan_flag)
+        out = [None] * len(self.members)
+        for g, lg in zip(eng.groups, lgs):
             for k, i in enumerate(g["idx"]):
                 out[i] = lg[k]
         self.exchange = {"collective": "broadcast", "mode": "broadcast"}

@@ -3,9 +3,9 @@
 ``MMPFNClassifier.predict_proba`` (``classifier.py:544-576``).
 
 Differences from the reference, all result-neutral:
-* estimators that share a preprocessed feature count run as ONE batched forward (the reference
-  loops over them serially, ``inference.py:294-349``) and share the image/text stem, which does not
-  depend on the estimator (``inference.py:272, 311-314``);
+* estimators that share a preprocessed feature count form one batch, and all batches go through the
+  layers in ONE pass (the reference loops over the estimators serially, ``inference.py:294-349``);
+  they share the image/text stem, which does not depend on the estimator (``inference.py:272, 311-314``);
 * weights stay resident on the device (the reference moves the model host<->device on every
   ``predict_proba``, ``inference.py:291, 351``);
 * ``fit_mode="fit_with_cache"`` keeps the per-layer K/V context of the train rows from ``fit`` so
@@ -109,7 +109,6 @@ class B200InferenceEngine:
         self._graphs = {}                      # input shapes -> (graph, static inputs, static output, scratch epoch)
         self.max_graphs = 4                    # least recently used beyond that are dropped (each holds a private pool)
         self._pinned_bufs = {}
-        self.multi_group = True                # False: one pass per group (tests compare the two, bit for bit)
         self._stage_event = None
         self._side = None                      # side stream of the test-row image stem
         self.launches_per_call = None
@@ -126,11 +125,12 @@ class B200InferenceEngine:
 
     def _build_contexts(self):
         self.train_image_tokens()
-        for g in self.groups:
-            g["ctx"] = self.model.fit_context(g["X_train"], None, g["y_train"], img_tok_train=self._img_tok_train,
-                                              label_stats=g["label_stats"])
-            if self.img_train_dev is not None:
-                g["ctx"].n_tok = self.img_train_dev.shape[1]
+        self.nan_flag.zero_()
+        ctxs = self.model.fit_contexts([dict(X_train=g["X_train"], y_train=g["y_train"], img_tok_train=self._img_tok_train,
+                                             label_stats=g["label_stats"]) for g in self.groups], nan_flag=self.nan_flag)
+        self.check_nan()
+        for g, ctx in zip(self.groups, ctxs):
+            g["ctx"] = ctx
 
     def _pinned(self, key, shape):
         """A persistent page-locked host buffer per input: the H2D copies of a call are asynchronous
@@ -180,31 +180,23 @@ class B200InferenceEngine:
         """The device-resident part of one call -> [n_est, Nte, n_out], estimator order as given to
         the constructor."""
         m = self.model
-        out = [None] * len(self.members)
         img_test_dev = staged["img_test"]
         flag = self.nan_flag
         flag.zero_()
-        # several groups with tables, bf16: one batched pass over all of them (flat sublayers launch once)
-        multi = (1 < len(self.groups) <= 8 and getattr(m, "precision", None) == _lib.BF16 and hasattr(m, "fit_contexts")
-                 and all(g["F"] >= 0 for g in self.groups) and self.multi_group)
-        if self.cache_context and multi:
-            tok_test = m.stem_image(img_test_dev) if img_test_dev is not None else None
-            lgs = m.predict_with_contexts([g["ctx"] for g in self.groups], staged["X_test"], img_tok_test=tok_test,
-                                          nan_flag=flag)
-            for g, lg in zip(self.groups, lgs):
-                for k, i in enumerate(g["idx"]):
-                    out[i] = lg[k]
-        elif multi:
-            tok_tr = tok_te = None
-            join = None
+        if self.cache_context:
+            ctxs = [g["ctx"] for g in self.groups]
+            tok_te = m.stem_image(img_test_dev) if img_test_dev is not None else None
+        else:
+            # reference-equivalent: the train contexts are rebuilt inside every call (inference.py:302-348)
+            tok_tr = tok_te = join = None
             if img_test_dev is not None:
                 tok_tr = self.train_image_tokens()
                 # the image/text stem of the TEST rows (a dozen small, latency-bound launches) does not depend on the
                 # context build: it runs on a side stream beside the train pass and joins before the test pass
                 # (only the FFMA stem: from 32 MGM heads its gated projection is a TMA / tcgen05 kernel, and layer-type
                 # kernels of two streams must not overlap, include/mmpfn_b200.h)
-                if m.geom.mgm_heads < 32:
-                    dev = m.device
+                dev = m.device
+                if dev.type == "cuda" and m.geom.mgm_heads < 32:
                     main = torch.cuda.current_stream(dev)
                     if self._side is None:
                         self._side = torch.cuda.Stream(device=dev)
@@ -217,34 +209,18 @@ class B200InferenceEngine:
                         tok_te.record_stream(main)
                 else:
                     tok_te = m.stem_image(img_test_dev)
-            specs = [dict(X_train=g["X_train"], y_train=g["y_train"], X_all=torch.cat([g["X_train"], Xte], dim=1),
+            specs = [dict(X_train=g["X_train"], y_train=g["y_train"],
+                          X_all=None if Xte is None else torch.cat([g["X_train"], Xte], dim=1),
                           img_tok_train=tok_tr, label_stats=g["label_stats"])
                      for g, Xte in zip(self.groups, staged["X_test"])]
             ctxs = m.fit_contexts(specs, nan_flag=flag)
             if join is not None:
                 torch.cuda.current_stream(m.device).wait_event(join)
-            lgs = m.predict_with_contexts(ctxs, staged["X_test"], img_tok_test=tok_te, nan_flag=flag)
-            for g, lg in zip(self.groups, lgs):
-                for k, i in enumerate(g["idx"]):
-                    out[i] = lg[k]
-        elif self.cache_context:
-            tok_test = m.stem_image(img_test_dev) if img_test_dev is not None else None
-            for g, Xte in zip(self.groups, staged["X_test"]):
-                lg = m.predict_with_context(g["ctx"], Xte, None, img_tok_test=tok_test, check=False, nan_flag=flag)
-                for k, i in enumerate(g["idx"]):
-                    out[i] = lg[k]
-        else:
-            # reference-equivalent: the train context is rebuilt inside every call (inference.py:302-348)
-            tok_tr = tok_te = None
-            if img_test_dev is not None:
-                tok_tr, tok_te = self.train_image_tokens(), m.stem_image(img_test_dev)
-            for g, Xte in zip(self.groups, staged["X_test"]):
-                X_full = None if Xte is None else torch.cat([g["X_train"], Xte], dim=1)
-                ctx = m.fit_context(g["X_train"], None, g["y_train"], X_all=X_full, img_tok_train=tok_tr, check=False,
-                                    label_stats=g["label_stats"], nan_flag=flag)
-                lg = m.predict_with_context(ctx, Xte, None, img_tok_test=tok_te, check=False, nan_flag=flag)
-                for k, i in enumerate(g["idx"]):
-                    out[i] = lg[k]
+        lgs = m.predict_with_contexts(ctxs, staged["X_test"], img_tok_test=tok_te, nan_flag=flag)
+        out = [None] * len(self.members)
+        for g, lg in zip(self.groups, lgs):
+            for k, i in enumerate(g["idx"]):
+                out[i] = lg[k]
         return torch.stack(out)
 
     def check_nan(self):

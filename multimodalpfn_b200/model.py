@@ -50,7 +50,6 @@ class TrainContext:
     n_train: int
     F: int
     T: int
-    n_tok: int
     kv: torch.Tensor                      # per-layer head-0 K/V of the item attention (layout: include/mmpfn_b200.h)
     tab_stats: Optional[torch.Tensor]     # [B, stats_elems]
     y_mean: torch.Tensor                  # [B]
@@ -230,21 +229,30 @@ class B200PerFeatureTransformer:
         ``state_b`` (one segment: a [B, S, T, E] state).  ``kvs``: one K/V context per segment (None on the train pass:
         not kept).  ``n_train=None``: the train pass, which writes the contexts; else the test pass against
         ``n_train`` context rows.  ``n_rows`` / ``n_ctx``: per-entry counts (int32 device tensors) or None
-        (``mmpfn_layers_train_ragged`` / ``_test_ragged``)."""
-        n = len(segs)
-        arr = (_lib.Segment * n)(*[_lib.Segment(int(b), int(t)) for b, t in segs])
-        kvp = (C.c_void_p * n)(*[_ptr(kv) for kv in kvs])
-        nbytes = self.lib.mmpfn_layers_ragged_ws_bytes(self._g, arr, n, S, self.precision)
-        ws = self._scratch("layers", nbytes)
-        if n_train is None:
-            _lib.check(self.lib.mmpfn_layers_train_ragged(self._g, self._w, state.data_ptr(), _ptr(state_b), arr, n, S,
-                                                          _ptr(n_rows), self.precision, kvp, ws.data_ptr(), nbytes,
-                                                          self._stream()), "mmpfn_layers_train_ragged")
-        else:
-            _lib.check(self.lib.mmpfn_layers_test_ragged(self._g, self._w_test, state.data_ptr(), _ptr(state_b), arr, n,
-                                                         S, int(n_train), _ptr(n_rows), _ptr(n_ctx), self.precision,
-                                                         kvp, ws.data_ptr(), nbytes, self._stream()),
-                       "mmpfn_layers_test_ragged")
+        (``mmpfn_layers_train_ragged`` / ``_test_ragged``).  A list of more than ``MAX_SEGMENTS`` segments runs as
+        consecutive calls; every segment's result is that of a call over that segment alone either way."""
+        off = entry = 0          # state elements and entries of the segments before this call
+        for i in range(0, len(segs), _lib.MAX_SEGMENTS):
+            part = segs[i:i + _lib.MAX_SEGMENTS]
+            n = len(part)
+            arr = (_lib.Segment * n)(*[_lib.Segment(int(b), int(t)) for b, t in part])
+            kvp = (C.c_void_p * n)(*[_ptr(kv) for kv in kvs[i:i + n]])
+            nbytes = self.lib.mmpfn_layers_ragged_ws_bytes(self._g, arr, n, S, self.precision)
+            ws = self._scratch("layers", nbytes)
+            st = state.view(-1)[off:].data_ptr()
+            stb = None if state_b is None else state_b.view(-1)[off:].data_ptr()
+            rows = None if n_rows is None else n_rows[entry:]
+            if n_train is None:
+                _lib.check(self.lib.mmpfn_layers_train_ragged(self._g, self._w, st, stb, arr, n, S, _ptr(rows),
+                                                              self.precision, kvp, ws.data_ptr(), nbytes,
+                                                              self._stream()), "mmpfn_layers_train_ragged")
+            else:
+                ctx = None if n_ctx is None else n_ctx[entry:]
+                _lib.check(self.lib.mmpfn_layers_test_ragged(self._g, self._w_test, st, stb, arr, n, S, int(n_train),
+                                                             _ptr(rows), _ptr(ctx), self.precision, kvp, ws.data_ptr(),
+                                                             nbytes, self._stream()), "mmpfn_layers_test_ragged")
+            off += self.geom.emsize * S * sum(int(b) * int(t) for b, t in part)
+            entry += sum(int(b) for b, _ in part)
 
     def layers_run(self, state, state_b, segs, S: int, n_train: Optional[int], layer_begin: int, layer_end: int,
                    phase: int = 0, ws_key: str = ""):
@@ -341,40 +349,14 @@ class B200PerFeatureTransformer:
         """
         with torch.cuda.device(self.device):
             X_train, img_train = self._prep(X_train, img_train)
-            y_train = y_train.to(self.device, torch.float32)
-            if y_train.dim() == 1:
-                y_train = y_train[None]
-            y_train = y_train.contiguous()
-            B, n_train = y_train.shape
-            F = 0 if X_train is None else X_train.shape[2]
-            n_tok = 0 if img_train is None else img_train.shape[1]
-            if X_train is None and img_train is None and img_tok_train is None:
-                raise ValueError("need tabular features, image embeddings, or both")
-            stats = None
-            if X_train is not None:
-                if X_all is not None:
-                    X_all, _ = self._prep(X_all, None)
-                    stats = self.stem_tab_fit(X_all, n_train)
-                else:
-                    stats = self.stem_tab_fit(X_train, n_train)
             if img_tok_train is None and img_train is not None:
                 img_tok_train = self.stem_image(img_train)
-            # label statistics involve a host sync: callers that replay a CUDA graph pass them in
-            y_mean, y_mask = label_stats if label_stats is not None else self.label_stats(y_train)
-            G = self._n_groups(F) if X_train is not None else 0
-            H_img = 0 if img_tok_train is None else img_tok_train.shape[-2]
-            T = G + H_img + 1
-            pos = self.positional_embeddings(T - 1)
             flag = nan_flag if nan_flag is not None else torch.zeros(1, dtype=torch.int32, device=self.device)
-            state, state_b = self.embed(X_train, stats, img_tok_train, y_train, y_mean, y_mask, pos, B=B, S=n_train,
-                                        F=F, x_bstride=n_train * F, y_bstride=n_train, nan_flag=flag)
-            kv = self.alloc_kv(B, n_train, T)
-            self.layers(state, state_b, [(B, T)], n_train, [kv])
+            ctx, = self.fit_contexts([dict(X_train=X_train, y_train=y_train, X_all=X_all, img_tok_train=img_tok_train,
+                                           label_stats=label_stats)], nan_flag=flag, keep_train_out=keep_train_out)
             if check:
                 self._check_nan(flag)
-            return TrainContext(B=B, n_train=n_train, F=F, T=T, n_tok=n_tok, kv=kv, tab_stats=stats, y_mean=y_mean,
-                                y_mask=y_mask, pos_emb=pos, precision=self.precision,
-                                train_out=state[:, :, T - 1].clone() if keep_train_out else None)
+            return ctx
 
     def predict_with_context(self, ctx: TrainContext, X_test, img_test, *, img_tok_test=None, check=True,
                              nan_flag=None, return_embeddings=False):
@@ -384,37 +366,97 @@ class B200PerFeatureTransformer:
             X_test, img_test = self._prep(X_test, img_test)
             if img_tok_test is None and img_test is not None:
                 img_tok_test = self.stem_image(img_test)
-            n_test = X_test.shape[1] if X_test is not None else img_tok_test.shape[-3]
-            if X_test is not None and (X_test.shape[0] != ctx.B or X_test.shape[2] != ctx.F):
-                raise ValueError(f"test table {tuple(X_test.shape)} does not match the context (B {ctx.B}, F {ctx.F})")
-            y_nan = torch.full((1, n_test), float("nan"), dtype=torch.float32, device=self.device)
             flag = nan_flag if nan_flag is not None else torch.zeros(1, dtype=torch.int32, device=self.device)
-            state, state_b = self.embed(X_test, ctx.tab_stats, img_tok_test, y_nan, ctx.y_mean, ctx.y_mask, ctx.pos_emb,
-                                        B=ctx.B, S=n_test, F=ctx.F, x_bstride=n_test * ctx.F, y_bstride=0,
-                                        nan_flag=flag)
-            if state.shape[2] != ctx.T:
-                raise ValueError("test rows produce a different number of tokens than the context")
-            self.layers(state, state_b, [(ctx.B, ctx.T)], n_test, [ctx.kv], n_train=ctx.n_train)
-            logits = self.decode(state)
+            out, = self.predict_with_contexts([ctx], [X_test], img_tok_test=img_tok_test, nan_flag=flag,
+                                              return_embeddings=return_embeddings)
             if check:
                 self._check_nan(flag)
-            if return_embeddings:
-                return logits, state[:, :, ctx.T - 1].clone()
-            return logits
+            return out
 
-    # ---- several estimator groups at once (bf16): one launch per flat sublayer for all of them ----------
-    def _group_buffers(self, shapes, with_bf16: bool = True):
-        """One fp32 + one bf16 buffer for states of the given [(B, S, T)] shapes, and the per-group views."""
+    # ---- several estimator groups in one layer pass ----------------------------------------------------------
+    def _group_buffers(self, shapes):
+        """One fp32 buffer (and, in bf16, one bf16 shadow) for states of the given [(B, S, T)] shapes, and the
+        per-group views."""
         E = self.geom.emsize
         total = sum(b * s * t for b, s, t in shapes)
         st = torch.empty((total, E), dtype=torch.float32, device=self.device)
-        stb = torch.empty((total, E), dtype=torch.bfloat16, device=self.device) if with_bf16 else None
+        stb = torch.empty((total, E), dtype=torch.bfloat16, device=self.device) if self.precision == _lib.BF16 else None
         views, off = [], 0
         for b, s, t in shapes:
             n = b * s * t
             views.append((st[off:off + n].view(b, s, t, E), None if stb is None else stb[off:off + n].view(b, s, t, E)))
             off += n
         return st, stb, views
+
+    def fit_contexts(self, specs, *, nan_flag=None, keep_train_out=False):
+        """``fit_context`` for estimator groups that share the train rows -> [TrainContext], one per spec.  A spec is a
+        dict with ``X_train`` ([B, Ntr, F], [Ntr, F], or None: no table) and ``y_train`` ([B, Ntr] or [Ntr]), and
+        optionally ``X_all``, ``img_tok_train`` (``stem_image`` of the train rows) and ``label_stats``.  The stem runs
+        per group, the layers as one pass over all groups (``layers``)."""
+        with torch.cuda.device(self.device):
+            flag = nan_flag if nan_flag is not None else torch.zeros(1, dtype=torch.int32, device=self.device)
+            prep = []
+            for sp in specs:
+                X_train, _ = self._prep(sp["X_train"], None)
+                tok = sp.get("img_tok_train")
+                if X_train is None and tok is None:
+                    raise ValueError("need tabular features, image embeddings, or both")
+                y_train = sp["y_train"].to(self.device, torch.float32)
+                y_train = (y_train[None] if y_train.dim() == 1 else y_train).contiguous()
+                B, n_train = y_train.shape
+                F = 0 if X_train is None else X_train.shape[2]
+                stats = None
+                if X_train is not None:
+                    X_all = X_train if sp.get("X_all") is None else self._prep(sp["X_all"], None)[0]
+                    stats = self.stem_tab_fit(X_all, n_train)
+                # label statistics involve a host sync: callers that replay a CUDA graph pass them in
+                ls = sp.get("label_stats")
+                y_mean, y_mask = ls if ls is not None else self.label_stats(y_train)
+                T = self._n_groups(F) + (0 if tok is None else tok.shape[-2]) + 1
+                prep.append(dict(X=X_train, y=y_train, B=B, n_train=n_train, F=F, stats=stats, tok=tok, y_mean=y_mean,
+                                 y_mask=y_mask, T=T, pos=self.positional_embeddings(T - 1)))
+            n_train = prep[0]["n_train"]
+            if any(p["n_train"] != n_train for p in prep):
+                raise ValueError(f"estimator groups with different train row counts {[p['n_train'] for p in prep]}")
+            st, stb, views = self._group_buffers([(p["B"], n_train, p["T"]) for p in prep])
+            for p, v in zip(prep, views):
+                self.embed(p["X"], p["stats"], p["tok"], p["y"], p["y_mean"], p["y_mask"], p["pos"], B=p["B"], S=n_train,
+                           F=p["F"], x_bstride=n_train * p["F"], y_bstride=n_train, nan_flag=flag, out=v)
+            kvs = [self.alloc_kv(p["B"], n_train, p["T"]) for p in prep]
+            self.layers(st, stb, [(p["B"], p["T"]) for p in prep], n_train, kvs)
+            return [TrainContext(B=p["B"], n_train=n_train, F=p["F"], T=p["T"], kv=kv, tab_stats=p["stats"],
+                                 y_mean=p["y_mean"], y_mask=p["y_mask"], pos_emb=p["pos"], precision=self.precision,
+                                 train_out=v[:, :, p["T"] - 1].clone() if keep_train_out else None)
+                    for p, kv, (v, _) in zip(prep, kvs, views)]
+
+    def predict_with_contexts(self, ctxs, X_tests, *, img_tok_test=None, nan_flag=None, return_embeddings=False):
+        """``predict_with_context`` for several contexts and the same test rows -> [logits [B_i, Nte, n_out]] (with
+        ``return_embeddings``: [(logits, y-token)]).  ``X_tests``: each context's test table (None: no table).  One
+        layer pass over all groups, one decode per group."""
+        with torch.cuda.device(self.device):
+            flag = nan_flag if nan_flag is not None else torch.zeros(1, dtype=torch.int32, device=self.device)
+            Xs = [self._prep(X, None)[0] for X in X_tests]
+            n_test = Xs[0].shape[1] if Xs[0] is not None else img_tok_test.shape[-3]
+            H_img = 0 if img_tok_test is None else img_tok_test.shape[-2]
+            n_train = ctxs[0].n_train
+            if any(c.n_train != n_train for c in ctxs):
+                raise ValueError(f"contexts with different train row counts {[c.n_train for c in ctxs]}")
+            for c, X in zip(ctxs, Xs):
+                if X is not None and (X.shape[0] != c.B or X.shape[1] != n_test or X.shape[2] != c.F):
+                    raise ValueError(f"test table {tuple(X.shape)} does not match its context (B {c.B}, F {c.F}) "
+                                     f"and {n_test} test rows")
+                if (0 if X is None else self._n_groups(c.F)) + H_img + 1 != c.T:
+                    raise ValueError("test rows produce a different number of tokens than the context")
+            y_nan = torch.full((1, n_test), float("nan"), dtype=torch.float32, device=self.device)
+            st, stb, views = self._group_buffers([(c.B, n_test, c.T) for c in ctxs])
+            for c, X, v in zip(ctxs, Xs, views):
+                self.embed(X, c.tab_stats, img_tok_test, y_nan, c.y_mean, c.y_mask, c.pos_emb, B=c.B, S=n_test, F=c.F,
+                           x_bstride=n_test * c.F, y_bstride=0, nan_flag=flag, out=v)
+            self.layers(st, stb, [(c.B, c.T) for c in ctxs], n_test, [c.kv for c in ctxs], n_train=n_train)
+            logits = [self.decode(v) for v, _ in views]
+            if return_embeddings:
+                return [(lg, v[:, :, c.T - 1].clone()) for lg, (v, _), c in zip(logits, views, ctxs)]
+            return logits
 
     # ---- entries of different sizes in one pass (tasks.py) ------------------------------------------------
     def entry_tokens(self, F: Optional[int], n_tok: int) -> int:
@@ -514,13 +556,12 @@ class B200PerFeatureTransformer:
             y_tr = torch.from_numpy(y_tr).to(dev)
             y_nan = torch.full((S_te,), float("nan"), dtype=torch.float32, device=dev)
             flag = torch.zeros(1, dtype=torch.int32, device=dev)
-            bf16 = self.precision == _lib.BF16
             shapes = [(len(js), T) for T, js in segs]
             kvs = [self.alloc_kv(b, S_tr, T) for b, T in shapes]
             logits = [None] * len(entries)
             for train in (True, False):
                 S = S_tr if train else S_te
-                st, stb, views = self._group_buffers([(b, S, T) for b, T in shapes], with_bf16=bf16)
+                st, stb, views = self._group_buffers([(b, S, T) for b, T in shapes])
                 k0 = 0
                 for (T, js), (v, vb) in zip(segs, views):
                     pos = self.positional_embeddings(T - 1)
@@ -598,58 +639,6 @@ class B200PerFeatureTransformer:
             _ptr(off), _ptr(cnt), out.data_ptr(), _ptr(out_b), flag.data_ptr(), self._stream()),
             "mmpfn_stem_tokens_ragged")
 
-    def fit_contexts(self, specs, *, nan_flag=None):
-        """``fit_context`` for several estimator groups that share the train rows (same n_train) — specs:
-        dicts with ``X_train [B, Ntr, F]``, ``y_train [B, Ntr]``, optional ``X_all``, ``img_tok_train``,
-        ``label_stats``.  Same results as one ``fit_context`` per group; the layers run as one pass over all
-        groups (``layers``)."""
-        assert self.precision == _lib.BF16
-        with torch.cuda.device(self.device):
-            flag = nan_flag if nan_flag is not None else torch.zeros(1, dtype=torch.int32, device=self.device)
-            prep = []
-            for sp in specs:
-                X_train, _ = self._prep(sp["X_train"], None)
-                y_train = sp["y_train"].to(self.device, torch.float32).contiguous()
-                B, n_train = y_train.shape
-                F = X_train.shape[2]
-                X_all = sp.get("X_all")
-                if X_all is not None:
-                    X_all, _ = self._prep(X_all, None)
-                stats = self.stem_tab_fit(X_all if X_all is not None else X_train, n_train)
-                tok = sp.get("img_tok_train")
-                y_mean, y_mask = sp["label_stats"] if sp.get("label_stats") is not None else self.label_stats(y_train)
-                T = self._n_groups(F) + (0 if tok is None else tok.shape[-2]) + 1
-                prep.append(dict(X=X_train, y=y_train, B=B, n_train=n_train, F=F, stats=stats, tok=tok, y_mean=y_mean,
-                                 y_mask=y_mask, T=T, pos=self.positional_embeddings(T - 1)))
-            n_train = prep[0]["n_train"]
-            assert all(p["n_train"] == n_train for p in prep)
-            st, stb, views = self._group_buffers([(p["B"], n_train, p["T"]) for p in prep])
-            for p, v in zip(prep, views):
-                self.embed(p["X"], p["stats"], p["tok"], p["y"], p["y_mean"], p["y_mask"], p["pos"], B=p["B"], S=n_train,
-                           F=p["F"], x_bstride=n_train * p["F"], y_bstride=n_train, nan_flag=flag, out=v)
-            kvs = [self.alloc_kv(p["B"], n_train, p["T"]) for p in prep]
-            self.layers(st, stb, [(p["B"], p["T"]) for p in prep], n_train, kvs)
-            return [TrainContext(B=p["B"], n_train=n_train, F=p["F"], T=p["T"], n_tok=0, kv=kv, tab_stats=p["stats"],
-                                 y_mean=p["y_mean"], y_mask=p["y_mask"], pos_emb=p["pos"], precision=self.precision)
-                    for p, kv in zip(prep, kvs)]
-
-    def predict_with_contexts(self, ctxs, X_tests, *, img_tok_test=None, nan_flag=None):
-        """``predict_with_context`` for several groups at once (same test rows) -> [logits [B_i, Nte, n_out]]."""
-        assert self.precision == _lib.BF16
-        with torch.cuda.device(self.device):
-            flag = nan_flag if nan_flag is not None else torch.zeros(1, dtype=torch.int32, device=self.device)
-            Xs = [self._prep(X, None)[0] for X in X_tests]
-            n_test = Xs[0].shape[1]
-            y_nan = torch.full((1, n_test), float("nan"), dtype=torch.float32, device=self.device)
-            st, stb, views = self._group_buffers([(c.B, n_test, c.T) for c in ctxs])
-            for c, X, v in zip(ctxs, Xs, views):
-                if X.shape[0] != c.B or X.shape[2] != c.F or X.shape[1] != n_test:
-                    raise ValueError("test tables do not match their contexts")
-                self.embed(X, c.tab_stats, img_tok_test, y_nan, c.y_mean, c.y_mask, c.pos_emb, B=c.B, S=n_test, F=c.F,
-                           x_bstride=n_test * c.F, y_bstride=0, nan_flag=flag, out=v)
-            self.layers(st, stb, [(c.B, c.T) for c in ctxs], n_test, [c.kv for c in ctxs], n_train=ctxs[0].n_train)
-            return [self.decode(v[0]) for v in views]
-
     def forward_batch(self, X_full, img_full, y_train, *, check=True, return_embeddings=False):
         """Reference-equivalent joint forward for B estimators sharing the image embeddings:
         X_full [B, S, F] (train rows first), img_full [S, n_tok, img_dim], y_train [B, Ntr]
@@ -673,8 +662,6 @@ class B200PerFeatureTransformer:
             ctx = self.fit_context(X_tr, None, y_train, X_all=X_full,
                                    img_tok_train=None if img_tok is None else img_tok[:n_train].contiguous(),
                                    check=False, nan_flag=flag, keep_train_out=return_embeddings)
-            if img_full is not None:
-                ctx.n_tok = img_full.shape[1]
             out = self.predict_with_context(ctx, X_te, None,
                                             img_tok_test=None if img_tok is None else img_tok[n_train:].contiguous(),
                                             check=check, nan_flag=flag, return_embeddings=return_embeddings)

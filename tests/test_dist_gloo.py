@@ -2,7 +2,7 @@
 ownership, the layout of the per-layer all-gather buffer (``KvPlan``), that every estimator's K/V block of every
 layer arrives where the test pass reads it, and that the sharded engine returns what the unsharded engine returns
 for each rank's test chunk.  The CUDA model is replaced by an arithmetic stand-in with the same host interface
-(embed / layers_run / decode; fit_context / predict_with_context built from the same arithmetic), so only the
+(embed / layers_run / decode; fit_contexts / predict_with_contexts built from the same arithmetic), so only the
 plumbing is tested."""
 import os
 import socket
@@ -158,20 +158,23 @@ class FakeModel:
         return state[:, :, -1, :1].repeat(1, 1, 10) + state.mean((2, 3))[..., None]
 
     # ---- the unsharded engine's entry points, from the same arithmetic -------------------------------------
-    def fit_context(self, X_train, img, y_train, *, X_all=None, img_tok_train=None, check=True, label_stats=None,
-                    nan_flag=None):
-        B, n_tr, F = X_train.shape
-        stats = self.stem_tab_fit(X_all if X_all is not None else X_train, n_tr)
-        y_mean, y_mask = label_stats if label_stats is not None else self.label_stats(y_train)
-        T = self._n_groups(F) + img_tok_train.shape[1] + 1
-        st, _, views = self._group_buffers([(B, n_tr, T)])
-        self.embed(X_train, stats, img_tok_train, y_train, y_mean, y_mask, None, B=B, S=n_tr, F=F, x_bstride=0, y_bstride=0,
-                   nan_flag=None, out=views[0])
-        kv = torch.zeros(L * B * T * 8, dtype=torch.uint8)
-        self.layers_run(st, None, [dict(B=B, T=T, kv=kv, layer_stride=0, slots=0, rank_stride=0, kv_buffer=kv, kv_offset=0)],
-                        n_tr, None, 0, L)
-        return TrainContext(B=B, n_train=n_tr, F=F, T=T, n_tok=0, kv=kv, tab_stats=stats, y_mean=y_mean, y_mask=y_mask,
-                            pos_emb=None, precision=1)
+    def fit_contexts(self, specs, *, nan_flag=None):
+        ctxs = []
+        for sp in specs:
+            X_train, X_all, img_tok_train = sp["X_train"], sp.get("X_all"), sp["img_tok_train"]
+            B, n_tr, F = X_train.shape
+            stats = self.stem_tab_fit(X_all if X_all is not None else X_train, n_tr)
+            y_mean, y_mask = sp["label_stats"] if sp.get("label_stats") is not None else self.label_stats(sp["y_train"])
+            T = self._n_groups(F) + img_tok_train.shape[1] + 1
+            st, _, views = self._group_buffers([(B, n_tr, T)])
+            self.embed(X_train, stats, img_tok_train, sp["y_train"], y_mean, y_mask, None, B=B, S=n_tr, F=F, x_bstride=0,
+                       y_bstride=0, nan_flag=None, out=views[0])
+            kv = torch.zeros(L * B * T * 8, dtype=torch.uint8)
+            self.layers_run(st, None, [dict(B=B, T=T, kv=kv, layer_stride=0, slots=0, rank_stride=0, kv_buffer=kv,
+                                            kv_offset=0)], n_tr, None, 0, L)
+            ctxs.append(TrainContext(B=B, n_train=n_tr, F=F, T=T, kv=kv, tab_stats=stats, y_mean=y_mean, y_mask=y_mask,
+                                     pos_emb=None, precision=1))
+        return ctxs
 
     def merge_kv(self, parts, B, n_train, T):
         out = torch.zeros(L * B * T * 8, dtype=torch.uint8)
@@ -179,15 +182,18 @@ class FakeModel:
             out.view(torch.float64).view(L, B, T)[:, pos] = kv.view(torch.float64).view(L, len(pos), T)
         return out
 
-    def predict_with_context(self, ctx, X_test, img, *, img_tok_test=None, check=True, nan_flag=None):
-        B, n_te, F = X_test.shape
-        st, _, views = self._group_buffers([(B, n_te, ctx.T)])
-        y_nan = torch.full((1, n_te), float("nan"))
-        self.embed(X_test, ctx.tab_stats, img_tok_test, y_nan, ctx.y_mean, ctx.y_mask, None, B=B, S=n_te, F=F, x_bstride=0,
-                   y_bstride=0, nan_flag=None, out=views[0])
-        self.layers_run(st, None, [dict(B=B, T=ctx.T, kv=ctx.kv, layer_stride=0, slots=0, rank_stride=0, kv_buffer=ctx.kv,
-                                        kv_offset=0)], n_te, ctx.n_train, 0, L)
-        return self.decode(views[0][0])
+    def predict_with_contexts(self, ctxs, X_tests, *, img_tok_test=None, nan_flag=None):
+        logits = []
+        for ctx, X_test in zip(ctxs, X_tests):
+            B, n_te, F = X_test.shape
+            st, _, views = self._group_buffers([(B, n_te, ctx.T)])
+            y_nan = torch.full((1, n_te), float("nan"))
+            self.embed(X_test, ctx.tab_stats, img_tok_test, y_nan, ctx.y_mean, ctx.y_mask, None, B=B, S=n_te, F=F,
+                       x_bstride=0, y_bstride=0, nan_flag=None, out=views[0])
+            self.layers_run(st, None, [dict(B=B, T=ctx.T, kv=ctx.kv, layer_stride=0, slots=0, rank_stride=0,
+                                            kv_buffer=ctx.kv, kv_offset=0)], n_te, ctx.n_train, 0, L)
+            logits.append(self.decode(views[0][0]))
+        return logits
 
 
 def _make_engine(rank_seed, n_a=4, n_b=4, n_train=20):

@@ -143,11 +143,9 @@ def test_packed_tasks_vs_reference(precision):
 def test_clf8_pad_ufes_vs_reference(precision, path):
     """configs[1] in full: the tensors that crossed the model boundary of the reference's 8-estimator
     ``MMPFNClassifier`` run on the PAD-UFES shape (its own preprocessing: 4 x F'=36 -> T=27, 4 x F'=22 ->
-    T=20), through the batched multi-group pass bench.py times (bf16) and through one pass per group;
-    per-estimator logits (fp32) and the final probabilities against the reference's."""
+    T=20), through the multi-group pass bench.py times and through one pass per group; per-estimator logits
+    (fp32) and the final probabilities against the reference's."""
     from multimodalpfn_b200.engine import proba_from_logits
-    if precision == "fp32" and path == "multi_group":
-        pytest.skip("the multi-group pass is the bf16 path")
     g = load_golden("large_clf8_pad_ufes")
     geom = Geometry(mgm_heads=8, cap_heads=8)
     sd = make_state_dict(geom, seed=1)

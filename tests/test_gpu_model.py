@@ -210,28 +210,43 @@ def test_model_extreme_shapes_vs_oracle(n_tr, n_te, F, n_tok):
         assert np.abs(p - pr).max() <= P_TOL[precision], (precision, float(np.abs(p - pr).max()))
 
 
-@pytest.mark.parametrize("fit_mode", ["fit_preprocessors", "fit_with_cache"])
-def test_multi_group_pass_equals_per_group(fit_mode):
-    """Estimator groups of different token counts as segments of one layer pass (flat sublayers launched once
-    for all groups) vs one pass per group: identical logits, bit for bit."""
+@pytest.mark.parametrize("precision", ["fp32", "bf16"])
+@pytest.mark.parametrize("case", ["fit_preprocessors", "fit_with_cache", "nine_groups"])
+def test_multi_group_pass_equals_per_group(case, precision):
+    """Estimator groups of different token counts as segments of one layer pass (bf16: flat sublayers launched once
+    for all groups; fp32: one segment after another; beyond 8 groups: consecutive calls) vs one engine per group with
+    the same ``cache_context``: identical logits, bit for bit."""
     from multimodalpfn_b200.classifier import MMPFNClassifier
+    from multimodalpfn_b200.engine import B200InferenceEngine
     from multimodalpfn_b200.preprocessing import transform_all
     from multimodalpfn_b200.synth import Geometry, make_dataset, make_state_dict
     geom = Geometry(mgm_heads=2, cap_heads=4)
     sd = make_state_dict(geom, seed=3)
     d = make_dataset("pad_ufes_small", 0)
-    clf = MMPFNClassifier(mixer_type="MGM+CAP", mgm_heads=2, cap_heads=4, features_per_group=2, n_estimators=4,
-                          model_path=(sd, geom), device="cuda", inference_precision="bf16",
-                          ignore_pretraining_limits=True, random_state=0, fit_mode=fit_mode)
-    clf.fit(d["X_train"], d["img_train"], d["y_train"])
-    eng = clf.executor_
-    assert len(eng.groups) == 2
-    staged = eng.stage(transform_all(clf.members_, d["X_test"]), d["img_test"])
-    eng.multi_group = True
-    a = eng.logits_staged(staged).clone()
-    eng.multi_group = False
-    b = eng.logits_staged(staged).clone()
-    assert torch.isfinite(a).all() and torch.equal(a, b)
+    if case == "nine_groups":
+        # nine table widths (raw columns 0..F-1): nine groups, more than one layer call takes
+        widths = list(range(2, 20, 2))
+        model = B200PerFeatureTransformer(sd, geom, precision=precision, seed=0)
+        members = [dict(X_train=d["X_train"][:, :F], y_train=d["y_train"].astype(np.float32), class_perm=None)
+                   for F in widths]
+        eng = B200InferenceEngine(model, members, d["img_train"])
+        X_tests = [d["X_test"][:, :F] for F in widths]
+        assert len(eng.groups) == 9
+    else:
+        clf = MMPFNClassifier(mixer_type="MGM+CAP", mgm_heads=2, cap_heads=4, features_per_group=2, n_estimators=4,
+                              model_path=(sd, geom), device="cuda", inference_precision=precision,
+                              ignore_pretraining_limits=True, random_state=0, fit_mode=case)
+        clf.fit(d["X_train"], d["img_train"], d["y_train"])
+        eng = clf.executor_
+        X_tests = transform_all(clf.members_, d["X_test"])
+        assert len(eng.groups) == 2
+    a = eng.logits_staged(eng.stage(X_tests, d["img_test"])).clone()
+    assert torch.isfinite(a).all()
+    for g in eng.groups:
+        one = B200InferenceEngine(eng.model, [eng.members[i] for i in g["idx"]], eng.image_train,
+                                  cache_context=eng.cache_context)
+        b = one.logits_staged(one.stage([X_tests[i] for i in g["idx"]], d["img_test"]))
+        assert torch.equal(a[g["idx"]], b), g["F"]
 
 
 def test_eight_estimators_equal_one_at_a_time():
