@@ -346,7 +346,7 @@ __global__ void __launch_bounds__(F_THREADS, 1) tc_mlp_kernel(const __grid_const
       // pass 1: add the residual chunk (16-byte piece j of row r sits at piece j ^ (r & 7)), keep the
       // sum in TMEM, accumulate the statistics.  The slots of chunks 0-2 go straight back to the
       // producer (chunks 3-5 of this tile); those of chunks 3-5 only after pass 2, which reuses them.
-      float sum = 0.f, sq = 0.f;
+      LnRowStats stats;
 #pragma unroll 1
       for (int c = 0; c < F_NRC; ++c) {
         const int q = i * F_NRC + c;
@@ -362,8 +362,6 @@ __global__ void __launch_bounds__(F_THREADS, 1) tc_mlp_kernel(const __grid_const
         for (int k = 0; k < 8; ++k) {
           const float a0 = __uint_as_float(v[4 * k]) + rr[k].x, a1 = __uint_as_float(v[4 * k + 1]) + rr[k].y,
                       a2 = __uint_as_float(v[4 * k + 2]) + rr[k].z, a3 = __uint_as_float(v[4 * k + 3]) + rr[k].w;
-          sum += (a0 + a1) + (a2 + a3);
-          sq = fmaf(a0, a0, sq); sq = fmaf(a1, a1, sq); sq = fmaf(a2, a2, sq); sq = fmaf(a3, a3, sq);
           v[4 * k] = __float_as_uint(a0); v[4 * k + 1] = __float_as_uint(a1);
           v[4 * k + 2] = __float_as_uint(a2); v[4 * k + 3] = __float_as_uint(a3);
         }
@@ -373,11 +371,11 @@ __global__ void __launch_bounds__(F_THREADS, 1) tc_mlp_kernel(const __grid_const
         // load then overwrites the slot under loads still in flight (a few rows per launch read the wrong chunk when
         // other work delays the warp: profiles/r02_interleaved_test_layers_experiment.txt).
         if (c < F_R_SLOTS) mbar_arrive_warp(&r_empty[slot]);
+        stats.add32(v, c);
       }
       tmem_st_wait();
-      const float mean = sum * (1.0f / kE);
-      const float var = fmaxf(sq * (1.0f / kE) - mean * mean, 0.f);
-      const float rstd = rsqrtf(var + kLnEps);
+      float mean, rstd;
+      stats.finish(mean, rstd);
       epi_bar();      // every row of the ring has been read: its memory becomes the staging area
       // pass 2: chunk c goes through staging slot c & 1 and out by TMA (rows past M are clipped by
       // the tensor maps).  One named barrier per chunk: before it the store leader has waited until

@@ -254,7 +254,7 @@ __global__ void __launch_bounds__(R_THREADS, 1) tc_rowgemm_kernel(const __grid_c
         // state = LN(state + acc).  Pass 1: add the residual chunk (shared memory, 128B swizzle: 16-byte
         // chunk j of row r sits at chunk j ^ (r & 7)), keep the sum in TMEM, accumulate the statistics.
         // Pass 2: normalise, write the fp32 state and its bf16 shadow.
-        float sum = 0.f, sq = 0.f;
+        LnRowStats stats;
 #pragma unroll 1
         for (int c = 0; c < R_NCH; ++c) {
           const int q = i * R_NCH + c;
@@ -270,8 +270,6 @@ __global__ void __launch_bounds__(R_THREADS, 1) tc_rowgemm_kernel(const __grid_c
           for (int k = 0; k < 8; ++k) {
             const float a0 = __uint_as_float(v[4 * k]) + rr[k].x, a1 = __uint_as_float(v[4 * k + 1]) + rr[k].y,
                         a2 = __uint_as_float(v[4 * k + 2]) + rr[k].z, a3 = __uint_as_float(v[4 * k + 3]) + rr[k].w;
-            sum += (a0 + a1) + (a2 + a3);
-            sq = fmaf(a0, a0, sq); sq = fmaf(a1, a1, sq); sq = fmaf(a2, a2, sq); sq = fmaf(a3, a3, sq);
             v[4 * k] = __float_as_uint(a0); v[4 * k + 1] = __float_as_uint(a1);
             v[4 * k + 2] = __float_as_uint(a2); v[4 * k + 3] = __float_as_uint(a3);
           }
@@ -279,11 +277,11 @@ __global__ void __launch_bounds__(R_THREADS, 1) tc_rowgemm_kernel(const __grid_c
           // (released behind the store that consumed the residual values: an arrival issued right after the ld.shared
           // instructions does not wait for their data — see kernels_mlp.cu)
           mbar_arrive_warp(&r_empty[slot]);
+          stats.add32(v, c);
         }
         tmem_st_wait();
-        const float mean = sum * (1.0f / kE);
-        const float var = fmaxf(sq * (1.0f / kE) - mean * mean, 0.f);
-        const float rstd = rsqrtf(var + kLnEps);
+        float mean, rstd;
+        stats.finish(mean, rstd);
         // pass 2: chunk c goes through staging slot c & 1 (fp32 and bf16 halves) and out by TMA.  One
         // named barrier per chunk: before it the store leader has waited until the store of chunk c-1
         // has read its slot, so after it every thread may overwrite that slot with chunk c+1.

@@ -172,7 +172,7 @@ __global__ void __launch_bounds__(G_THREADS) tc_gemm_kernel(const __grid_constan
       const long long m = (long long)m0 + r;
       const bool ok = m < p.M;
       float* res = p.resid + m * kE;
-      float sum = 0.f, sq = 0.f;
+      LnRowStats stats;
 #pragma unroll 1
       for (int c = 0; c < kE / 32; ++c) {
         tmem_ld32(trow + c * 32, v);
@@ -184,18 +184,16 @@ __global__ void __launch_bounds__(G_THREADS) tc_gemm_kernel(const __grid_constan
             const float4 rr = r4[i];
             const float a0 = __uint_as_float(v[4 * i]) + rr.x, a1 = __uint_as_float(v[4 * i + 1]) + rr.y,
                         a2 = __uint_as_float(v[4 * i + 2]) + rr.z, a3 = __uint_as_float(v[4 * i + 3]) + rr.w;
-            sum += (a0 + a1) + (a2 + a3);
-            sq = fmaf(a0, a0, sq); sq = fmaf(a1, a1, sq); sq = fmaf(a2, a2, sq); sq = fmaf(a3, a3, sq);
             v[4 * i] = __float_as_uint(a0); v[4 * i + 1] = __float_as_uint(a1);
             v[4 * i + 2] = __float_as_uint(a2); v[4 * i + 3] = __float_as_uint(a3);
           }
+          stats.add32(v, c);
         }
         tmem_st32(trow + c * 32, v);
       }
       tmem_st_wait();
-      const float mean = sum * (1.0f / kE);
-      const float var = fmaxf(sq * (1.0f / kE) - mean * mean, 0.f);
-      const float rstd = rsqrtf(var + kLnEps);
+      float mean, rstd;
+      stats.finish(mean, rstd);
       uint16_t* lnb = p.ln_bf16 + m * kE;
 #pragma unroll 1
       for (int c = 0; c < kE / 32; ++c) {

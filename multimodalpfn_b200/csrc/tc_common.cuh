@@ -313,6 +313,57 @@ __host__ __device__ constexpr uint32_t make_idesc(int M, int N) {
   return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
+// ---------------------------------------------------------------------------------------------
+// LayerNorm statistics of the residual + LayerNorm epilogues (kernels_mlp.cu, kernels_rowgemm.cu,
+// kernels_tc.cu): one thread owns one kE-wide row, which arrives as six 32-column chunks in order.
+// The variance is taken about the mean, not as sq/kE - mean^2: that one-pass form cancels when a row's
+// |mean| is large against its spread (the error grows with the square of mean/std; past ~1000 the
+// variance comes out 0: a row of mean -4096, std 1.6 came out off by ~2e3).  Every value enters shifted
+// by K = the mean of the row's first chunk, within ~std/sqrt(32) of the row mean, so that
+// var = E[(a-K)^2] - E[a-K]^2 cancels only by (mean - K)^2 / var ~ 1/32, whatever the mean.  The sums are
+// one pass over registers in packed fp32x2 arithmetic; the epilogues take them after a chunk's sum has
+// gone back to TMEM and its residual slot to the producer, off the path of the residual ring.
+// A row of exact zeros gives mean 0, variance 0 and normalises to exact zeros (the pad-row contract).
+// ---------------------------------------------------------------------------------------------
+struct LnRowStats {
+  float k = 0.f;
+  uint64_t s2 = 0ull, q2a = 0ull, q2b = 0ull;     // sum of (a - K) and of (a - K)^2, two lanes each
+  // chunk c (0-based) of the row: 32 fp32 values as bits
+  __device__ __forceinline__ void add32(const uint32_t (&v)[32], int c) {
+    uint64_t a2[16];
+#pragma unroll
+    for (int i = 0; i < 16; ++i) a2[i] = pack_f32x2(__uint_as_float(v[2 * i]), __uint_as_float(v[2 * i + 1]));
+    if (c == 0) {
+      uint64_t t2[4] = {0ull, 0ull, 0ull, 0ull};
+#pragma unroll
+      for (int i = 0; i < 16; ++i) t2[i & 3] = add_f32x2(t2[i & 3], a2[i]);
+      float t0, t1;
+      unpack_f32x2(add_f32x2(add_f32x2(t2[0], t2[1]), add_f32x2(t2[2], t2[3])), t0, t1);
+      k = (t0 + t1) * (1.0f / 32);
+    }
+    const uint64_t nk2 = pack_f32x2(-k, -k);
+    uint64_t sa = 0ull, sb = 0ull;
+#pragma unroll
+    for (int i = 0; i < 16; i += 2) {
+      const uint64_t d0 = add_f32x2(a2[i], nk2), d1 = add_f32x2(a2[i + 1], nk2);
+      sa = add_f32x2(sa, d0);
+      sb = add_f32x2(sb, d1);
+      q2a = fma_f32x2(d0, d0, q2a);
+      q2b = fma_f32x2(d1, d1, q2b);
+    }
+    s2 = add_f32x2(s2, add_f32x2(sa, sb));
+  }
+  // after the last chunk
+  __device__ __forceinline__ void finish(float& mean, float& rstd) const {
+    float s0, s1, q0, q1;
+    unpack_f32x2(s2, s0, s1);
+    unpack_f32x2(add_f32x2(q2a, q2b), q0, q1);
+    const float dm = (s0 + s1) * (1.0f / kE);
+    mean = k + dm;
+    rstd = rsqrtf(fmaxf((q0 + q1) * (1.0f / kE) - dm * dm, 0.f) + kLnEps);
+  }
+};
+
 
 // ---------------------------------------------------------------------------------------------
 // host: tensor maps

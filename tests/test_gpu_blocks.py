@@ -260,10 +260,12 @@ def _one_layer_model(precision, seed=3):
 
 
 @pytest.mark.parametrize("precision,tol", [("fp32", 2e-5), ("bf16", 0.06)])
-@pytest.mark.parametrize("B,S,T,n_test", [(1, 200, 7, 60), (2, 333, 12, 130), (1, 1100, 5, 257)])
+@pytest.mark.parametrize("B,S,T,n_test", [(1, 200, 7, 60), (2, 333, 12, 130), (1, 1100, 5, 257), (1, 40, 120, 9),
+                                          (1, 24, 200, 7)])
 def test_single_layer_pass_vs_oracle(precision, tol, B, S, T, n_test):
     """The train pass (writes the K/V context) then the test pass on random O(1) states vs the
-    oracle's layer_forward (layer.py:272-457)."""
+    oracle's layer_forward (layer.py:272-457).  T = 120 and 200: the fp32 feature attention past 48 KB of shared
+    memory (its opt-in starts at 120 tokens); the bf16 pass takes the CUDA-core feature attention above 192."""
     from oracle import forward_ref as R
     model, sd, geom = _one_layer_model(precision)
     tsd = R.as_torch_state_dict(sd)
