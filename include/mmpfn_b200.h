@@ -22,9 +22,14 @@
  *  - there is NO CPU fallback: on a machine without an sm_100 device every compute entry point
  *    returns MMPFN_ENODEVICE;
  *  - tensors are dense, row-major, innermost dimension last, in the layouts stated per call;
- *  - `precision`: MMPFN_F32 (FFMA kernels, the 1e-5 parity mode) or MMPFN_BF16 (tcgen05/TMEM/TMA
+ *  - `precision`: MMPFN_F32 (FFMA kernels, the 1e-5 parity mode), MMPFN_BF16 (tcgen05/TMEM/TMA
  *    kernels: bf16 MMA operands, fp32 accumulation, fp32 softmax/LayerNorm statistics and an fp32
- *    residual stream).
+ *    residual stream) or MMPFN_F16 (the same kernels with fp16 MMA operands: 3 more significand bits than
+ *    bf16; every fp32 -> fp16 rounding saturates at +-65504 instead of overflowing to inf).  In MMPFN_F16 every
+ *    argument or buffer whose name says bf16 (state_bf16, the K/V context, the layout comments below) holds
+ *    fp16 values instead, in the same layout and size; the weights come from mmpfn_weights.layers_f16.  The stem
+ *    has no fp16 form: the layer passes write the fp16 shadow of the fp32 state themselves.  The *_f16 building
+ *    blocks below are the fp16 twins of the *_bf16 ones.
  */
 #ifndef MMPFN_B200_H
 #define MMPFN_B200_H
@@ -39,7 +44,7 @@ extern "C" {
 #define MMPFN_ABI_VERSION 2
 
 enum { MMPFN_OK = 0, MMPFN_EINVAL = -1, MMPFN_ENODEVICE = -2, MMPFN_ECUDA = -3, MMPFN_EUNSUPPORTED = -4 };
-enum { MMPFN_F32 = 0, MMPFN_BF16 = 1 };
+enum { MMPFN_F32 = 0, MMPFN_BF16 = 1, MMPFN_F16 = 2 };
 enum { MMPFN_MIXER_NONE = 0, MMPFN_MIXER_MGM = 1, MMPFN_MIXER_MGM_CAP = 2, MMPFN_MIXER_MOE = 3 };
 
 /* Geometry of the checkpoint (reference model/config.py:18-83, model/loading.py:470-538).
@@ -53,7 +58,7 @@ typedef struct mmpfn_geometry {
  * reference state_dict (SURVEY.md Appendix B).  All matrices are "W[N][K]" (output-major), so a
  * projection is out[n] = sum_k in[k] * W[n][k].
  *
- * layers_f32 / layers_bf16: nlayers consecutive blocks of
+ * layers_f32 / layers_bf16 / layers_f16: nlayers consecutive blocks of
  *     feat_wqkv [3*E][E] | feat_wout [E][E] | item_wqkv [3*E][E] | item_wout [E][E]
  *     | mlp_w1 [nhid][E] | mlp_w2 [E][nhid]
  * where wqkv rows are ordered (j in q,k,v; head; d) exactly like the reference `_w_qkv [3,H,D,E]`
@@ -94,6 +99,9 @@ typedef struct mmpfn_weights {
    * one large GEMM, M0 x (Hm*img) x img — runs on tcgen05 with bf16 operands and fp32 accumulation; NULL (or fewer
    * heads) keeps it on the fp32 FFMA path (the 1e-5 parity mode) */
   const uint16_t* mgm_w1_bf16;
+  /* fp16 copy of the layer blocks, layout of layers_bf16; read only under MMPFN_F16 (appended: callers that never
+   * pass MMPFN_F16 need not know the field) */
+  const uint16_t* layers_f16;
 } mmpfn_weights;
 
 /* ---- introspection ------------------------------------------------------------------------- */
@@ -153,7 +161,7 @@ int mmpfn_stem_tokens(const mmpfn_geometry* g, const mmpfn_weights* w, const flo
  * (multi_head_attention.py:328-336, :467-470) with a layer axis in front. */
 size_t mmpfn_kv_bytes(const mmpfn_geometry* g, int B, int n_train, int T, int precision);
 
-/* Whole passes through the 12 layers (layer.py:272-457), both precisions; state is updated in place.
+/* Whole passes through the 12 layers (layer.py:272-457), every precision; state is updated in place.
  *  - Train pass: every row is a train row (self-attention over items, all heads, layer.py:363-372); writes the
  *    head-0 K/V context of segment i to kv[i] when kv[i] != NULL.
  *  - Test pass: the item attention reads the cached head-0 K/V of the n_train train rows for all six query heads
@@ -164,7 +172,8 @@ size_t mmpfn_kv_bytes(const mmpfn_geometry* g, int B, int n_train, int T, int pr
  * pass over a [B][S][T][E] state.  bf16: the sublayers that work on the flat token axis (QKV and output projections
  * + LayerNorm, MLP) launch once for all segments, the attentions per segment; fp32: one segment after another.
  * Every segment's result is that of a call over that segment alone.  state_bf16 is unused (may be NULL) in
- * MMPFN_F32.
+ * MMPFN_F32.  MMPFN_F16: the call first writes the fp16 shadow of state_f32 into state_bf16 (an fp16 buffer of the
+ * same size), then runs as MMPFN_BF16 does with fp16 operands; the K/V context is fp16 in the bf16 layout.
  * n_rows / n_ctx: per-entry row counts (device int32, see "per-entry row counts" below), or NULL = every entry
  * uses all S rows (and all n_train context rows).  With counts, entry b's item attention (layer.py:341-379) runs
  * over its own rows only. */
@@ -189,7 +198,7 @@ int mmpfn_layers_test_ragged(const mmpfn_geometry* g, const mmpfn_weights* w, fl
  * kv + l * layer_stride.  Test pass: estimator b of the segment = (rank b / slots, slot b % slots) lives in the block at
  * kv + l * layer_stride + rank * rank_stride with c = slots.  layer_stride 0 = blocks of consecutive layers are
  * adjacent; slots 0 = all B estimators in one block (rank_stride unused): then this is the bf16 pass of
- * mmpfn_layers_train_ragged / _test_ragged without counts.
+ * mmpfn_layers_train_ragged / _test_ragged without counts.  bf16 only (there is no precision argument).
  * Layers [layer_begin, layer_end) run; the state is carried in state_f32 / state_bf16 between calls. */
 typedef struct mmpfn_kv_segment {
   int32_t B, T;
@@ -322,6 +331,9 @@ int mmpfn_linear_bf16(const uint16_t* A, const uint16_t* W, int M, int N, int K,
  *   state_f32 [M][192] <- LayerNorm(state_f32 + A W^T),  state_bf16 <- bf16(state_f32);  A [M][192], W [192][192] bf16. */
 int mmpfn_linear_ln_bf16(const uint16_t* A, const uint16_t* W, int M, float* state_f32, uint16_t* state_bf16,
                          void* stream);
+/* fp16 twin: A, W, state_f16 fp16 */
+int mmpfn_linear_ln_f16(const uint16_t* A, const uint16_t* W, int M, float* state_f32, uint16_t* state_f16,
+                        void* stream);
 
 /* The QKV projection of the attention across items (multi_head_attention.py:430-434) with its scatter into
  * the layouts the item-attention kernel reads: state [B][S][T][192] bf16, w_qkv [n_proj*192][192] bf16
@@ -330,12 +342,17 @@ int mmpfn_linear_ln_bf16(const uint16_t* A, const uint16_t* W, int M, float* sta
  *   k0 [B*T][S_pad][32], vt0 [B*T][32][S_pad] (multi_head_attention.py:328-336).  S_pad % 64 == 0. */
 int mmpfn_item_qkv_bf16(const uint16_t* state_bf16, const uint16_t* w_qkv, int B, int S, int T, int S_pad, int n_proj,
                         uint16_t* q, uint16_t* k, uint16_t* vt, uint16_t* k0, uint16_t* vt0, void* stream);
+/* fp16 twin: every 16-bit buffer fp16 */
+int mmpfn_item_qkv_f16(const uint16_t* state_f16, const uint16_t* w_qkv, int B, int S, int T, int S_pad, int n_proj,
+                       uint16_t* q, uint16_t* k, uint16_t* vt, uint16_t* k0, uint16_t* vt0, void* stream);
 
 /* The MLP sublayer alone (mlp.py:93-138 + layer.py:437-455), one fused tcgen05 kernel, in place:
  *   state_f32 [M][192] <- LayerNorm(state_f32 + W2 gelu(W1 state_bf16)),  state_bf16 <- bf16(state_f32)
  * w1 [768][192], w2 [192][768] bf16 (the reference's linear1.weight / linear2.weight). */
 int mmpfn_mlp_bf16(float* state_f32, uint16_t* state_bf16, const uint16_t* w1, const uint16_t* w2, int M,
                    void* stream);
+/* fp16 twin: state_f16, w1, w2 fp16 */
+int mmpfn_mlp_f16(float* state_f32, uint16_t* state_f16, const uint16_t* w1, const uint16_t* w2, int M, void* stream);
 
 /* Item-axis attention alone (layer.py:341-379), bf16 tcgen05 kernel, for unit tests and roofline timing.
  *   q  [B*T*nhead][Sq_pad][32]   k [planes_kv][Skv_pad][32]   vt [planes_kv][32][Skv_pad]   (bf16)
@@ -352,6 +369,10 @@ int mmpfn_item_attention_bf16(const uint16_t* q, const uint16_t* k, const uint16
 int mmpfn_item_attention_bf16_ragged(const uint16_t* q, const uint16_t* k, const uint16_t* vt, int B, int T, int n_q,
                                      int Sq_pad, int n_kv, int Skv_pad, int shared_kv, const int32_t* q_len,
                                      const int32_t* kv_len, uint16_t* out, void* stream);
+/* fp16 twin of both (q, k, vt, out fp16): q_len / kv_len NULL = the plain form, both set = the per-entry form */
+int mmpfn_item_attention_f16(const uint16_t* q, const uint16_t* k, const uint16_t* vt, int B, int T, int n_q,
+                             int Sq_pad, int n_kv, int Skv_pad, int shared_kv, const int32_t* q_len,
+                             const int32_t* kv_len, uint16_t* out, void* stream);
 /* Item-axis attention of the fp32 parity mode (layer.py:341-379), for unit tests:
  *   q, out [B][n_q][T][nhead*32];  shared_kv = 0: k, v [B][n_kv][T][nhead*32];  shared_kv = 1 (every query head reads
  *   head 0, multi_head_attention.py:436-445): k, v [B][T][n_kv][32].
@@ -363,6 +384,8 @@ int mmpfn_item_attention_f32(const float* q, const float* k, const float* v, int
  * tensor-core kernel, for unit tests and HBM-roofline timing.
  *   qkv [n_rows*T][576] bf16 (q | k | v, head-major inside each third)  ->  att [n_rows*T][192] bf16 */
 int mmpfn_feature_attention_bf16(const uint16_t* qkv, uint16_t* att, long long n_rows, int T, void* stream);
+/* fp16 twin: qkv, att fp16 */
+int mmpfn_feature_attention_f16(const uint16_t* qkv, uint16_t* att, long long n_rows, int T, void* stream);
 
 /* QKV projection + feature-axis attention in ONE kernel (multi_head_attention.py:430-434 + layer.py:332-339 for the
  * feature axis): the [tokens][576] qkv block never leaves the SM.  What the bf16 layer passes run for T <= 64
@@ -371,6 +394,9 @@ int mmpfn_feature_attention_bf16(const uint16_t* qkv, uint16_t* att, long long n
  *   x [n_rows*T][192] bf16, w_qkv [576][192] bf16  ->  att [n_rows*T][192] bf16 */
 int mmpfn_feature_qkv_attention_bf16(const uint16_t* x, const uint16_t* w_qkv, long long n_rows, int T, uint16_t* att,
                                      void* stream);
+/* fp16 twin: x, w_qkv, att fp16 */
+int mmpfn_feature_qkv_attention_f16(const uint16_t* x, const uint16_t* w_qkv, long long n_rows, int T, uint16_t* att,
+                                    void* stream);
 
 #ifdef __cplusplus
 }

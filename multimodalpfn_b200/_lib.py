@@ -12,7 +12,7 @@ from . import build as _build
 
 c_void_p, c_int, c_float, c_size_t, c_int64, c_ll = C.c_void_p, C.c_int, C.c_float, C.c_size_t, C.c_int64, C.c_longlong
 
-F32, BF16 = 0, 1
+F32, BF16, F16 = 0, 1, 2
 MAX_SEGMENTS = 8          # MMPFN_MAX_SEGMENTS
 MIXER = {"none": 0, "MGM": 1, "MGM+CAP": 2, "MoE": 3}
 ERRORS = {-1: "EINVAL", -2: "ENODEVICE", -3: "ECUDA", -4: "EUNSUPPORTED"}
@@ -26,7 +26,7 @@ class Geometry(C.Structure):
 WEIGHT_FIELDS = ("layers_f32", "layers_bf16", "enc_w", "yenc_w", "yenc_b", "dec_w1", "dec_b1", "dec_w2", "dec_b2",
                  "mgm_w1", "mgm_b1", "mgm_w2", "mgm_b2", "moe_gate_w", "moe_gate_b", "cap_knorm_w", "cap_knorm_b",
                  "cap_q", "cap_wkv", "cap_bkv", "cap_wo", "cap_bo", "cap_onorm_w", "cap_onorm_b", "cap_f1_w",
-                 "cap_f1_b", "cap_f2_w", "cap_f2_b", "mgm_w1_bf16")
+                 "cap_f1_b", "cap_f2_w", "cap_f2_b", "mgm_w1_bf16", "layers_f16")
 
 
 class Weights(C.Structure):
@@ -97,6 +97,14 @@ SIGNATURES = {
                                          PVP, c_void_p, c_size_t, c_void_p]),
     "mmpfn_item_attention_bf16_ragged": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int,
                                                  c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "mmpfn_linear_ln_f16": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
+    "mmpfn_item_qkv_f16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,
+                                   c_void_p, c_void_p, c_void_p]),
+    "mmpfn_mlp_f16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
+    "mmpfn_item_attention_f16": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+                                         c_void_p, c_void_p, c_void_p, c_void_p]),
+    "mmpfn_feature_attention_f16": (c_int, [c_void_p, c_void_p, c_ll, c_int, c_void_p]),
+    "mmpfn_feature_qkv_attention_f16": (c_int, [c_void_p, c_void_p, c_ll, c_int, c_void_p, c_void_p]),
     "mmpfn_item_attention_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p,
                                          c_void_p, c_void_p, c_void_p]),
 }

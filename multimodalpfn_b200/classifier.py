@@ -31,6 +31,17 @@ MAX_NUMBER_OF_SAMPLES = 10_000
 MAX_NUMBER_OF_FEATURES = 500
 
 
+def precision_name(p) -> str:
+    """The layer precision ("fp32", "bf16" or "fp16") an ``inference_precision`` value selects."""
+    if p in ("auto", "autocast", torch.bfloat16, "bf16", "bfloat16"):
+        return "bf16"          # the reference autocasts on CUDA (base.py:126-165); bf16 here, SURVEY gotcha 4
+    if p in (torch.float32, "fp32", "float32"):
+        return "fp32"
+    if p in (torch.float16, "fp16", "float16"):
+        return "fp16"          # the reference's own CUDA autocast type (inference.py:339): 3 more bits than bf16
+    raise ValueError(f"unsupported inference_precision {p!r} (fp32, fp16, or bf16/auto)")
+
+
 class MMPFNClassifier(ClassifierMixin, BaseEstimator):
     def __init__(self, *, mixer_type: str = "MGM+CAP", mgm_heads: int = 8, cap_heads: Optional[int] = 8,
                  features_per_group: int = 2, n_estimators: int = 4, categorical_features_indices=None,
@@ -60,12 +71,7 @@ class MMPFNClassifier(ClassifierMixin, BaseEstimator):
 
     # -------------------------------------------------------------------------------------
     def _precision(self) -> str:
-        p = self.inference_precision
-        if p in ("auto", "autocast", torch.bfloat16, "bf16", "bfloat16"):
-            return "bf16"          # the reference autocasts on CUDA (base.py:126-165); bf16 here, SURVEY gotcha 4
-        if p in (torch.float32, "fp32", "float32"):
-            return "fp32"
-        raise ValueError(f"unsupported inference_precision {p!r} (fp32 or bf16/auto)")
+        return precision_name(self.inference_precision)
 
     def _device(self) -> torch.device:
         if self.device in ("auto", "cuda"):

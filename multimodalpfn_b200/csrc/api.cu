@@ -75,14 +75,16 @@ struct LayerW {
   const uint16_t *fqkv_b, *fout_b, *iqkv_b, *iout_b, *w1_b, *w2_b;
 };
 static size_t layer_elems() { return (size_t)2 * (3 * kE * kE + kE * kE) + (size_t)2 * kHid * kE; }
-static LayerW layer_w(const mmpfn_weights* w, int l) {
+// fmt: which 16-bit copy of the layer blocks the tensor-core kernels read (layers_bf16 or layers_f16)
+static LayerW layer_w(const mmpfn_weights* w, int l, int fmt = FMT_BF16) {
   LayerW r{};
   const size_t o0 = 0, o1 = o0 + 3 * kE * kE, o2 = o1 + kE * kE, o3 = o2 + 3 * kE * kE, o4 = o3 + kE * kE,
                o5 = o4 + (size_t)kHid * kE;
   const float* f = w->layers_f32 + l * layer_elems();
   r.fqkv = f + o0; r.fout = f + o1; r.iqkv = f + o2; r.iout = f + o3; r.w1 = f + o4; r.w2 = f + o5;
-  if (w->layers_bf16) {
-    const uint16_t* b = w->layers_bf16 + l * layer_elems();
+  const uint16_t* b16 = fmt == FMT_F16 ? w->layers_f16 : w->layers_bf16;
+  if (b16) {
+    const uint16_t* b = b16 + l * layer_elems();
     r.fqkv_b = b + o0; r.fout_b = b + o1; r.iqkv_b = b + o2; r.iout_b = b + o3; r.w1_b = b + o4; r.w2_b = b + o5;
   }
   return r;
@@ -91,19 +93,24 @@ static LayerW layer_w(const mmpfn_weights* w, int l) {
 static int kv_pad(int n) { return (n + 63) / 64 * 64; }
 
 // K = 192 projections: the persistent kernel (kernels_rowgemm.cu).  In the tuning build (-DMMPFN_DEBUG)
-// MMPFN_ROWGEMM=0 selects the one-tile-per-CTA kernel of kernels_tc.cu instead (A/B timing and bisecting);
-// the product library reads no environment variable.
-static int proj_gemm(const TcGemm& g, cudaStream_t st) {
+// MMPFN_ROWGEMM=0 selects the one-tile-per-CTA kernel of kernels_tc.cu instead (A/B timing and bisecting; bf16
+// only); the product library reads no environment variable.
+static int proj_gemm(const TcGemm& g, cudaStream_t st, int fmt = FMT_BF16) {
 #ifdef MMPFN_DEBUG
   static int persistent = -1;
   if (persistent < 0) {
     const char* e = getenv("MMPFN_ROWGEMM");
     persistent = e ? atoi(e) : 1;
   }
-  if (!persistent) return launch_tc_gemm(g, st);
+  if (!persistent) {
+    if (fmt != FMT_BF16) { set_error("MMPFN_ROWGEMM=0: the one-tile kernel has no fp16 variant"); return MMPFN_EUNSUPPORTED; }
+    return launch_tc_gemm(g, st);
+  }
 #endif
-  return launch_tc_rowgemm(g, st);
+  return launch_tc_rowgemm(g, st, fmt);
 }
+// the 16-bit operand format of a tensor-core precision (MMPFN_BF16 / MMPFN_F16)
+static int fmt_of(int precision) { return precision == MMPFN_F16 ? FMT_F16 : FMT_BF16; }
 
 // scratch of the row-wise sublayers: the fp32 buffers are carved by carve(); in bf16 mode layers_run points
 // att_b / hid_b into its own workspace (carve_multi)
@@ -349,7 +356,7 @@ static int feature_attention(const LayerW& lw, float* state, long long M, long l
   return launch_layernorm(ws.tmp, state, nullptr, nullptr, M, kE, state, nullptr, st);
 }
 
-// The MLP and the item attention's out-projection + LN, shared by the fp32 and the bf16 passes.
+// The MLP and the item attention's out-projection + LN, shared by the fp32 and the 16-bit passes.
 static int mlp(const LayerW& lw, float* state, uint16_t* state_b, long long M, int precision, const LayerWs& ws,
                cudaStream_t st) {
   if (precision == MMPFN_F32) {
@@ -370,8 +377,9 @@ static int mlp(const LayerW& lw, float* state, uint16_t* state_b, long long M, i
   if (fused) {
     TcMlp f{};
     f.state_b = state_b; f.state_b_out = state_b; f.resid_f32 = state; f.w1 = lw.w1_b; f.w2 = lw.w2_b; f.M = (int)M;
-    return launch_tc_mlp(f, st);
+    return launch_tc_mlp(f, st, fmt_of(precision));
   }
+  if (precision != MMPFN_BF16) { set_error("MMPFN_FUSED_MLP=0: the two-GEMM MLP has no fp16 variant"); return MMPFN_EUNSUPPORTED; }
   TcGemm a{};
   a.A = state_b; a.W = lw.w1_b; a.M = (int)M; a.N = kHid; a.K = kE; a.epi = TC_EPI_GELU_BF16; a.out_bf16 = ws.hid_b;
   MMPFN_TRY(launch_tc_gemm(a, st));
@@ -390,7 +398,7 @@ static int out_proj_ln(const LayerW& lw, float* state, uint16_t* state_b, long l
   TcGemm o{};
   o.A = ws.att_b; o.W = lw.iout_b; o.M = (int)M; o.N = kE; o.K = kE; o.epi = TC_EPI_RESID_LN;
   o.resid_f32 = state; o.ln_bf16 = state_b;
-  return proj_gemm(o, st);
+  return proj_gemm(o, st, fmt_of(precision));
 }
 
 // The fp32 (parity mode) passes over one [B][S][T] state.  train != 0: self-attention over the S rows, head-0 K/V
@@ -485,10 +493,13 @@ static size_t kv_block_elems(int c, int T, int n_pad) { return (size_t)2 * c * T
 // train == 0: the S rows are test rows attending to the n_train rows' context segs[i].kv
 // n_rows / n_ctx (device, one entry per estimator of every segment in list order, or NULL): per-entry row counts of
 // this pass and context rows of the test pass (mmpfn_layers_*_ragged)
+// precision: MMPFN_BF16, or MMPFN_F16 (state_b, the K/V context and every 16-bit buffer are then fp16, the weights
+// are read from layers_f16)
 static int layers_run(const mmpfn_geometry* g, const mmpfn_weights* w, float* state, uint16_t* state_b,
                       const mmpfn_kv_segment* ks, int n_seg, int S, int n_train, int train, int layer_begin,
                       int layer_end, int phase, void* workspace, size_t workspace_bytes, cudaStream_t st,
-                      const int* n_rows, const int* n_ctx) {
+                      const int* n_rows, const int* n_ctx, int precision = MMPFN_BF16) {
+  const int fmt = fmt_of(precision);
   MMPFN_TRY(check_geometry(g));
   MMPFN_TRY(require_device());
   if (!ks || n_seg < 1 || n_seg > MMPFN_MAX_SEGMENTS) { set_error("layers_run: bad segment list"); return MMPFN_EINVAL; }
@@ -496,7 +507,10 @@ static int layers_run(const mmpfn_geometry* g, const mmpfn_weights* w, float* st
   for (int i = 0; i < n_seg; ++i) { segs[i].B = ks[i].B; segs[i].T = ks[i].T; }
   long long M = 0;
   MMPFN_TRY(check_segments(segs, n_seg, S, &M));
-  if (!w || !w->layers_f32 || !w->layers_bf16 || !state || !state_b) { set_error("layers_run: null argument (bf16 mode only)"); return MMPFN_EINVAL; }
+  if (!w || !w->layers_f32 || !(fmt == FMT_F16 ? w->layers_f16 : w->layers_bf16) || !state || !state_b) {
+    set_error("layers_run: null argument (16-bit modes only)");
+    return MMPFN_EINVAL;
+  }
   if (layer_begin < 0 || layer_end > g->nlayers || layer_begin >= layer_end) { set_error("layers_run: bad layer range [%d, %d)", layer_begin, layer_end); return MMPFN_EINVAL; }
   if (phase < 0 || phase > 2 || (phase != 0 && layer_end != layer_begin + 1)) { set_error("layers_run: phase %d needs a single layer", phase); return MMPFN_EINVAL; }
   for (int i = 0; i < n_seg; ++i) {
@@ -528,7 +542,7 @@ static int layers_run(const mmpfn_geometry* g, const mmpfn_weights* w, float* st
   constexpr bool feat_fused = true;
 #endif
   for (int l = layer_begin; l < layer_end; ++l) {
-    const LayerW lw = layer_w(w, l);
+    const LayerW lw = layer_w(w, l, fmt);
     // features: QKV over all tokens, attention per segment (rows of T_i tokens), out-projection + LN over all
     if (phase != 2) {
       // rows of up to 64 tokens: projection and attention in one kernel (the qkv block stays on chip); wider rows:
@@ -537,20 +551,22 @@ static int layers_run(const mmpfn_geometry* g, const mmpfn_weights* w, float* st
       for (int i = 0; i < n_seg; ++i) {
         const long long m = (long long)segs[i].B * S * segs[i].T;
         if (feat_fused && feat_qkv_attn_supported(segs[i].T)) {
-          MMPFN_TRY(launch_feat_qkv_attn(state_b + off * kE, lw.fqkv_b, m, segs[i].T, ws.att_b + off * kE, st));
+          MMPFN_TRY(launch_feat_qkv_attn(state_b + off * kE, lw.fqkv_b, m, segs[i].T, ws.att_b + off * kE, st, fmt));
         } else {
           TcGemm a{};
           a.A = state_b + off * kE; a.W = lw.fqkv_b; a.M = (int)m; a.N = 3 * kE; a.K = kE; a.epi = TC_EPI_BF16;
           a.out_bf16 = ws.hid_b + off * 3 * kE;
-          MMPFN_TRY(proj_gemm(a, st));
-          MMPFN_TRY(launch_feat_attn_bf16(ws.hid_b + off * 3 * kE, ws.att_b + off * kE, (long long)segs[i].B * S, segs[i].T, st));
+          MMPFN_TRY(proj_gemm(a, st, fmt));
+          const long long n_seq = (long long)segs[i].B * S;
+          MMPFN_TRY(fmt == FMT_F16 ? launch_feat_attn_f16(ws.hid_b + off * 3 * kE, ws.att_b + off * kE, n_seq, segs[i].T, st)
+                                   : launch_feat_attn_bf16(ws.hid_b + off * 3 * kE, ws.att_b + off * kE, n_seq, segs[i].T, st));
         }
         off += m;
       }
       TcGemm o{};
       o.A = ws.att_b; o.W = lw.fout_b; o.M = (int)M; o.N = kE; o.K = kE; o.epi = TC_EPI_RESID_LN;
       o.resid_f32 = state; o.ln_bf16 = state_b;
-      MMPFN_TRY(proj_gemm(o, st));
+      MMPFN_TRY(proj_gemm(o, st, fmt));
     }
     // items: QKV scatter + attention per segment (tiles follow T_i), out-projection + LN over all
     {
@@ -604,14 +620,14 @@ static int layers_run(const mmpfn_geometry* g, const mmpfn_weights* w, float* st
             a.kv_seg_rows = ks[i].seg_rows; a.kv_seg_stride = ks[i].rank_stride / 2;
           }
         }
-        if (phase != 2) MMPFN_TRY(proj_gemm(q, st));
-        if (phase != 1) MMPFN_TRY(launch_tc_item_attn(a, st));
+        if (phase != 2) MMPFN_TRY(proj_gemm(q, st, fmt));
+        if (phase != 1) MMPFN_TRY(launch_tc_item_attn(a, st, fmt));
         off += (long long)B * S * T;
         entry += B;
       }
-      if (phase != 1) MMPFN_TRY(out_proj_ln(lw, state, state_b, M, MMPFN_BF16, flat, st));
+      if (phase != 1) MMPFN_TRY(out_proj_ln(lw, state, state_b, M, precision, flat, st));
     }
-    if (phase != 1) MMPFN_TRY(mlp(lw, state, state_b, M, MMPFN_BF16, flat, st));
+    if (phase != 1) MMPFN_TRY(mlp(lw, state, state_b, M, precision, flat, st));
   }
   return MMPFN_OK;
 }
@@ -627,7 +643,7 @@ int mmpfn_layers_run(const mmpfn_geometry* g, const mmpfn_weights* w, float* sta
 size_t mmpfn_layers_ragged_ws_bytes(const mmpfn_geometry* g, const mmpfn_segment* segs, int n_seg, int S, int precision) {
   long long M = 0;
   if (check_geometry(g) != MMPFN_OK || check_segments(segs, n_seg, S, &M) != MMPFN_OK) return 0;
-  if (precision == MMPFN_BF16) return carve_multi(nullptr, segs, n_seg, S, M).bytes;
+  if (precision == MMPFN_BF16 || precision == MMPFN_F16) return carve_multi(nullptr, segs, n_seg, S, M).bytes;
   if (precision != MMPFN_F32) return 0;
   long long m_max = 0;         // fp32: one segment after another
   for (int i = 0; i < n_seg; ++i) {
@@ -647,14 +663,19 @@ static int layers_ragged(const mmpfn_geometry* g, const mmpfn_weights* w, float*
   if (!kv) { set_error("layers_ragged: null context list"); return MMPFN_EINVAL; }
   MMPFN_TRY(check_segments(segs, n_seg, S, &M));
   if (!train && n_train < 1) { set_error("layers_ragged: the test pass needs n_train >= 1"); return MMPFN_EINVAL; }
-  if (precision == MMPFN_BF16) {
+  if (precision == MMPFN_BF16 || precision == MMPFN_F16) {
+    if (precision == MMPFN_F16) {
+      // the fp16 shadow of the state, which the stem writes only in bf16 (the stem takes no fp16 shadow)
+      if (!state || !state_b) { set_error("layers_ragged: null state"); return MMPFN_EINVAL; }
+      MMPFN_TRY(launch_f16_shadow(state, state_b, M * kE, st));
+    }
     mmpfn_kv_segment ks[MMPFN_MAX_SEGMENTS];
     for (int i = 0; i < n_seg; ++i) {
       ks[i] = mmpfn_kv_segment{};
       ks[i].B = segs[i].B; ks[i].T = segs[i].T; ks[i].kv = kv[i];
     }
     return layers_run(g, w, state, state_b, ks, n_seg, S, n_train, train, 0, g->nlayers, 0, workspace, workspace_bytes,
-                      st, n_rows, n_ctx);
+                      st, n_rows, n_ctx, precision);
   }
   if (precision != MMPFN_F32 || !w || !w->layers_f32 || !state) { set_error("layers_ragged: bad arguments"); return MMPFN_EINVAL; }
   if (workspace_bytes < mmpfn_layers_ragged_ws_bytes(g, segs, n_seg, S, precision) || !workspace) {
@@ -869,6 +890,66 @@ int mmpfn_feature_qkv_attention_bf16(const uint16_t* x, const uint16_t* w_qkv, l
   MMPFN_TRY(require_device());
   if (!x || !w_qkv || !att || n_rows < 1 || T < 2) { set_error("feature_qkv_attention: bad arguments"); return MMPFN_EINVAL; }
   return launch_feat_qkv_attn(x, w_qkv, n_rows * T, T, att, (cudaStream_t)stream);
+}
+
+// ---- fp16 twins of the tensor-core building blocks (MMPFN_F16): same layouts and contracts, fp16 in and out ----
+int mmpfn_linear_ln_f16(const uint16_t* A, const uint16_t* W, int M, float* state_f32, uint16_t* state_f16,
+                        void* stream) {
+  MMPFN_TRY(require_device());
+  if (!A || !W || !state_f32 || !state_f16 || M < 1) { set_error("linear_ln_f16: bad arguments"); return MMPFN_EINVAL; }
+  TcGemm o{};
+  o.A = A; o.W = W; o.M = M; o.N = kE; o.K = kE; o.epi = TC_EPI_RESID_LN; o.resid_f32 = state_f32; o.ln_bf16 = state_f16;
+  return proj_gemm(o, (cudaStream_t)stream, FMT_F16);
+}
+
+int mmpfn_item_qkv_f16(const uint16_t* state_f16, const uint16_t* w_qkv, int B, int S, int T, int S_pad, int n_proj,
+                       uint16_t* q, uint16_t* k, uint16_t* vt, uint16_t* k0, uint16_t* vt0, void* stream) {
+  MMPFN_TRY(require_device());
+  if (!state_f16 || !w_qkv || !q || B < 1 || S < 1 || T < 1 || S_pad < S || S_pad % 64 || (n_proj != 1 && n_proj != 3) ||
+      (n_proj == 3 && (!k || !vt))) {
+    set_error("item_qkv_f16: bad arguments");
+    return MMPFN_EINVAL;
+  }
+  TcGemm g{};
+  g.A = state_f16; g.W = w_qkv; g.N = n_proj * kE; g.K = kE; g.items = 1; g.B = B; g.S = S; g.T = T;
+  g.epi = TC_EPI_QKV_ITEMS; g.q_out = q; g.k_out = k; g.vt_out = vt; g.k0_out = k0; g.vt0_out = vt0; g.S_pad = S_pad;
+  return proj_gemm(g, (cudaStream_t)stream, FMT_F16);
+}
+
+int mmpfn_mlp_f16(float* state_f32, uint16_t* state_f16, const uint16_t* w1, const uint16_t* w2, int M, void* stream) {
+  MMPFN_TRY(require_device());
+  if (!state_f32 || !state_f16 || !w1 || !w2 || M < 1) { set_error("mlp_f16: bad arguments"); return MMPFN_EINVAL; }
+  TcMlp f{};
+  f.state_b = state_f16; f.state_b_out = state_f16; f.resid_f32 = state_f32; f.w1 = w1; f.w2 = w2; f.M = M;
+  return launch_tc_mlp(f, (cudaStream_t)stream, FMT_F16);
+}
+
+int mmpfn_item_attention_f16(const uint16_t* q, const uint16_t* k, const uint16_t* vt, int B, int T, int n_q,
+                             int Sq_pad, int n_kv, int Skv_pad, int shared_kv, const int32_t* q_len,
+                             const int32_t* kv_len, uint16_t* out, void* stream) {
+  MMPFN_TRY(require_device());
+  if (!q || !k || !vt || !out || B < 1 || T < 1 || n_q < 1 || n_kv < 1 || Sq_pad < n_q || Skv_pad < n_kv ||
+      Sq_pad % 8 || Skv_pad % 8) {
+    set_error("item_attention_f16: bad arguments");
+    return MMPFN_EINVAL;
+  }
+  TcItemAttn a{};
+  a.q = q; a.k = k; a.vt = vt; a.out = out; a.B = B; a.T = T; a.n_q = n_q; a.Sq_pad = Sq_pad; a.n_kv = n_kv;
+  a.Skv_pad = Skv_pad; a.shared_kv = shared_kv; a.q_len = q_len; a.kv_len = kv_len;
+  return launch_tc_item_attn(a, (cudaStream_t)stream, FMT_F16);
+}
+
+int mmpfn_feature_attention_f16(const uint16_t* qkv, uint16_t* att, long long n_rows, int T, void* stream) {
+  MMPFN_TRY(require_device());
+  if (!qkv || !att || n_rows < 1 || T < 1) { set_error("feature_attention_f16: bad arguments"); return MMPFN_EINVAL; }
+  return launch_feat_attn_f16(qkv, att, n_rows, T, (cudaStream_t)stream);
+}
+
+int mmpfn_feature_qkv_attention_f16(const uint16_t* x, const uint16_t* w_qkv, long long n_rows, int T, uint16_t* att,
+                                    void* stream) {
+  MMPFN_TRY(require_device());
+  if (!x || !w_qkv || !att || n_rows < 1 || T < 2) { set_error("feature_qkv_attention_f16: bad arguments"); return MMPFN_EINVAL; }
+  return launch_feat_qkv_attn(x, w_qkv, n_rows * T, T, att, (cudaStream_t)stream, FMT_F16);
 }
 
 }  // extern "C"

@@ -90,6 +90,20 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
   __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
   return *reinterpret_cast<uint32_t*>(&v);
 }
+// fp16 pair (lo = first), round to nearest; out-of-range values saturate to +-65504 instead of becoming inf
+__device__ __forceinline__ uint32_t pack_f16x2_sat(float lo, float hi) {
+  uint32_t r;
+  asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+  return r;
+}
+// 16-bit operand format of the tensor-core layer kernels, a compile-time parameter of each: bf16 (MMPFN_BF16) or
+// fp16 (MMPFN_F16).  Only the MMA operand type and the fp32 -> 16-bit roundings differ between the two.
+enum { FMT_BF16 = 0, FMT_F16 = 1 };
+template <int FMT>
+__device__ __forceinline__ uint32_t pack16x2(float lo, float hi) {
+  if constexpr (FMT == FMT_F16) return pack_f16x2_sat(lo, hi);
+  else return pack_bf16x2(lo, hi);
+}
 __device__ __forceinline__ float fast_exp2f(float x) {   // MUFU.EX2
   float y;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
@@ -118,6 +132,8 @@ int launch_sgemm(const SgemmParams& p, int epi, cudaStream_t st);
 // x_stride: elements between consecutive input rows (0 = width).
 int launch_layernorm(const float* x, const float* res, const float* gamma, const float* beta, long long rows,
                      int width, float* y_f32, uint16_t* y_bf16, cudaStream_t st, long long x_stride = 0);
+// y[i] = fp16(x[i]) (round to nearest, saturating) for n values, n % 4 == 0: the fp16 shadow of the fp32 state
+int launch_f16_shadow(const float* x, uint16_t* y, long long n, cudaStream_t st);
 // copy head-0 k|v of the item-attention qkv buffer [B][S][T][3E] into the fp32 context [B][T][S][2][kD]; with
 // n_rows (device [B]) the rows s >= n_rows[b] are written as zeros instead
 int launch_kv_extract_f32(const float* qkv, float* kv, int B, int S, int T, cudaStream_t st, const int* n_rows = nullptr);
@@ -125,9 +141,11 @@ int launch_kv_extract_f32(const float* qkv, float* kv, int B, int S, int T, cuda
 // attention between features: qkv [rows = n_seq*T][3*kE] (q|k|v, head-major) -> att [rows][kE]
 int launch_feat_attn_f32(const float* qkv, float* att, long long n_seq, int T, cudaStream_t st);
 int launch_feat_attn_bf16(const uint16_t* qkv, uint16_t* att, long long n_seq, int T, cudaStream_t st);
+int launch_feat_attn_f16(const uint16_t* qkv, uint16_t* att, long long n_seq, int T, cudaStream_t st);
 // QKV projection + feature attention in one kernel (kernels_featfused.cu); T <= 64
 bool feat_qkv_attn_supported(int T);
-int launch_feat_qkv_attn(const uint16_t* x, const uint16_t* w_qkv, long long M, int T, uint16_t* att, cudaStream_t st);
+int launch_feat_qkv_attn(const uint16_t* x, const uint16_t* w_qkv, long long M, int T, uint16_t* att, cudaStream_t st,
+                         int fmt = FMT_BF16);
 
 // attention between items, fp32 flash kernel.  For plane p in [0, planes) and head h:
 //   q row i  at  q  + plane_off(q)  + i*q_row  + h*kD          (n_q rows)
@@ -170,7 +188,7 @@ struct TcGemm {
 };
 int launch_tc_gemm(const TcGemm& p, cudaStream_t st);
 // persistent variant for K = 192, N % 192 == 0 (kernels_rowgemm.cu): BF16 / RESID_LN / QKV_ITEMS epilogues
-int launch_tc_rowgemm(const TcGemm& p, cudaStream_t st);
+int launch_tc_rowgemm(const TcGemm& p, cudaStream_t st, int fmt = FMT_BF16);
 
 // Fused MLP sublayer (kernels_mlp.cu): state <- LN(state + W2 gelu(W1 state)), in place.
 struct TcMlp {
@@ -181,7 +199,7 @@ struct TcMlp {
   const uint16_t* w2;        // [kE][kHid] bf16
   int M;
 };
-int launch_tc_mlp(const TcMlp& p, cudaStream_t st);
+int launch_tc_mlp(const TcMlp& p, cudaStream_t st, int fmt = FMT_BF16);
 
 struct TcItemAttn {
   const uint16_t* q;    // [planes_q = B*T*kH][Sq_pad][kD]
@@ -207,7 +225,7 @@ struct TcItemAttn {
   const int* q_len;
   const int* kv_len;
 };
-int launch_tc_item_attn(const TcItemAttn& p, cudaStream_t st);
+int launch_tc_item_attn(const TcItemAttn& p, cudaStream_t st, int fmt = FMT_BF16);
 
 // ---- stem / tail (kernels_stem.cu) -----------------------------------------------------------
 // Statistics block per estimator, indexed by COMPACTED slot c = g*fpg + j (encoders.py:102-130):

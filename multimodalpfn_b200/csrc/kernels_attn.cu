@@ -3,7 +3,8 @@
 //
 //   S = Q K^T and O += P V on tcgen05 (accumulators in TMEM, operands staged by TMA), online softmax
 //   in fp32 by four warps (thread = query row).  P goes back into tensor memory over the S columns it
-//   came from (bf16 pairs) and the second MMA reads its A operand there: no st.shared, no proxy fence.
+//   came from (bf16 pairs; fp16 pairs in the fp16 instantiation) and the second MMA reads its A operand there: no
+//   st.shared, no proxy fence.
 //
 // At d = 32 every exponential buys only 128 tensor FLOP, so the kernel lives on the MUFU pipe
 // (16 ex2/clk/SM = 595 TFLOP/s at 1965 MHz if every exponential went there) and on the issue slots of
@@ -255,7 +256,7 @@ __device__ __forceinline__ void tmem_st_cols(uint32_t taddr, const uint32_t* v) 
 // RAGGED: entry b has its own key count kv_len[b] (tiles past it are not visited; its last tile is masked like the
 // tail tile) and query count q_len[b] (output rows from there up to n_q are written as zeros; a tile holding only
 // such rows stores its zeros and issues nothing else).  The other instantiation is the one the layer passes use.
-template <int BK, int PP, bool RAGGED>
+template <int BK, int PP, bool RAGGED, int FMT>
 __global__ void __launch_bounds__(A_THREADS, AttnCfg<BK>::kMinCtas)
     tc_item_attn_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
                         const __grid_constant__ CUtensorMap map_vt, const AttnArgs p) {
@@ -361,8 +362,8 @@ __global__ void __launch_bounds__(A_THREADS, AttnCfg<BK>::kMinCtas)
     }
   } else if (warp == 5) {
     if (elect_one()) {
-      constexpr uint32_t idesc_s = make_idesc(A_BQ, BK);
-      constexpr uint32_t idesc_o = make_idesc(A_BQ, kD);
+      constexpr uint32_t idesc_s = make_idesc_fmt<FMT>(A_BQ, BK);
+      constexpr uint32_t idesc_o = make_idesc_fmt<FMT>(A_BQ, kD);
       const uint64_t qdesc = make_desc(sbase, 512, kSw64);
       const uint64_t kdesc0 = make_desc(sbase + C::kOffK, 512, kSw64);
       const uint64_t vdesc0 = make_desc(sbase + C::kOffVt, 1024, kSw128);
@@ -464,7 +465,7 @@ __global__ void __launch_bounds__(A_THREADS, AttnCfg<BK>::kMinCtas)
         auto retire = [&](int k) {
           const float a = __uint_as_float(sv[2 * k]), b = __uint_as_float(sv[2 * k + 1]);
           lsum2 = add_f32x2(lsum2, pack_f32x2(a, b));
-          sv[k] = pack_bf16x2(a, b);       // slot k belonged to pair k / 2, retired no later than this one
+          sv[k] = pack16x2<FMT>(a, b);       // slot k belonged to pair k / 2, retired no later than this one
         };
 #pragma unroll
         for (int k = 0; k < kAhead; ++k) scale(k);
@@ -573,10 +574,10 @@ __global__ void __launch_bounds__(A_THREADS, AttnCfg<BK>::kMinCtas)
       uint4* d4 = reinterpret_cast<uint4*>(dst);
 #pragma unroll
       for (int i = 0; i < 4; ++i)
-        d4[i] = make_uint4(pack_bf16x2(__uint_as_float(v[8 * i]) * inv, __uint_as_float(v[8 * i + 1]) * inv),
-                           pack_bf16x2(__uint_as_float(v[8 * i + 2]) * inv, __uint_as_float(v[8 * i + 3]) * inv),
-                           pack_bf16x2(__uint_as_float(v[8 * i + 4]) * inv, __uint_as_float(v[8 * i + 5]) * inv),
-                           pack_bf16x2(__uint_as_float(v[8 * i + 6]) * inv, __uint_as_float(v[8 * i + 7]) * inv));
+        d4[i] = make_uint4(pack16x2<FMT>(__uint_as_float(v[8 * i]) * inv, __uint_as_float(v[8 * i + 1]) * inv),
+                           pack16x2<FMT>(__uint_as_float(v[8 * i + 2]) * inv, __uint_as_float(v[8 * i + 3]) * inv),
+                           pack16x2<FMT>(__uint_as_float(v[8 * i + 4]) * inv, __uint_as_float(v[8 * i + 5]) * inv),
+                           pack16x2<FMT>(__uint_as_float(v[8 * i + 6]) * inv, __uint_as_float(v[8 * i + 7]) * inv));
     }
     tc_fence_before();
   }
@@ -587,18 +588,18 @@ __global__ void __launch_bounds__(A_THREADS, AttnCfg<BK>::kMinCtas)
   }
 }
 
-template <int BK, int PP, bool RAGGED = false>
+template <int BK, int PP, bool RAGGED = false, int FMT = FMT_BF16>
 int launch_attn_t(const CUtensorMap& mq, const CUtensorMap& mk, const CUtensorMap& mvt, const AttnArgs& a, dim3 grid,
                   cudaStream_t st) {
   using C = AttnCfg<BK>;
-  MMPFN_OPT_IN_SMEM((tc_item_attn_kernel<BK, PP, RAGGED>), C::kSmem);
-  tc_item_attn_kernel<BK, PP, RAGGED><<<grid, A_THREADS, C::kSmem, st>>>(mq, mk, mvt, a);
+  MMPFN_OPT_IN_SMEM((tc_item_attn_kernel<BK, PP, RAGGED, FMT>), C::kSmem);
+  tc_item_attn_kernel<BK, PP, RAGGED, FMT><<<grid, A_THREADS, C::kSmem, st>>>(mq, mk, mvt, a);
   return count_launch();
 }
 
 }  // namespace
 
-int launch_tc_item_attn(const TcItemAttn& p, cudaStream_t st) {
+int launch_tc_item_attn(const TcItemAttn& p, cudaStream_t st, int fmt) {
   constexpr int BK = 48;
   if (p.n_q <= 0 || p.B <= 0) return MMPFN_OK;
   if (p.n_kv <= 0) { set_error("item attention: empty key set"); return MMPFN_EINVAL; }
@@ -658,6 +659,11 @@ int launch_tc_item_attn(const TcItemAttn& p, cudaStream_t st) {
   }
   AttnArgs a{p.out, p.T, p.n_q, p.n_kv, p.shared_kv, q_tiles, stack ? p.Sq_pad : 0, slots, tiles_per_seg, p.q_len, p.kv_len};
   const dim3 grid((unsigned)(grid_planes * q_tiles));
+  if (fmt == FMT_F16) {
+    // fp16: P is stored only after the row-sum decision, so every stored p is <= kSumLimit (2^8), far inside fp16's range
+    if (p.q_len || p.kv_len) return launch_attn_t<BK, kPolyPairsDefault, true, FMT_F16>(mq, mk, mvt, a, grid, st);
+    return launch_attn_t<BK, kPolyPairsDefault, false, FMT_F16>(mq, mk, mvt, a, grid, st);
+  }
   if (p.q_len || p.kv_len) return launch_attn_t<BK, kPolyPairsDefault, true>(mq, mk, mvt, a, grid, st);
 #ifdef MMPFN_DEBUG
   // tuning builds only (-DMMPFN_DEBUG): MMPFN_ATTN_PP = polynomial pairs of every 24.  The product

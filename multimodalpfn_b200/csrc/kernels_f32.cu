@@ -6,6 +6,8 @@
 //   layernorm_kernel    y = LN(x + res) [* gamma + beta]   layer.py:40-64 (no affine), nn.LayerNorm in the stem
 //   feat_attn_kernel    per-row attention across tokens    layer.py:332-339
 //   item_attn_f32       flash attention across items       layer.py:341-379
+#include <cuda_fp16.h>
+
 #include "common.cuh"
 #include "feat_attn_core.cuh"
 
@@ -198,11 +200,20 @@ template <>
 __device__ __forceinline__ float ld_as_float<float>(const float* p) { return *p; }
 template <>
 __device__ __forceinline__ float ld_as_float<uint16_t>(const uint16_t* p) { return bf16_bits_to_float(*p); }
+// fp16 element of the fp16 layer pass (a type of its own so that uint16_t keeps meaning bf16 here)
+struct f16_bits {
+  uint16_t b;
+};
+template <>
+__device__ __forceinline__ float ld_as_float<f16_bits>(const f16_bits* p) {
+  return __half2float(__ushort_as_half(p->b));
+}
 __device__ __forceinline__ void st_from_float(float* p, float v) { *p = v; }
 __device__ __forceinline__ void st_from_float(uint16_t* p, float v) {
   __nv_bfloat16 b = __float2bfloat16_rn(v);
   *p = *reinterpret_cast<uint16_t*>(&b);
 }
+__device__ __forceinline__ void st_from_float(f16_bits* p, float v) { p->b = (uint16_t)pack_f16x2_sat(v, 0.f); }
 
 template <typename TIn, typename TOut>
 __global__ void __launch_bounds__(128) feat_attn_kernel(const TIn* __restrict__ qkv, TOut* __restrict__ att,
@@ -287,7 +298,7 @@ constexpr int FA_ROW_BYTES = 3 * kE * 2 + 16;   // 1168
 // A CTA walks table rows blockIdx.x, blockIdx.x + gridDim.x, ... with two staging buffers: the qkv block
 // of the next row streams in (cp.async) while the current row is computed, so the DRAM latency of a row is
 // paid under the previous row's arithmetic instead of once per CTA.
-template <int KT>
+template <int KT, int FMT>
 __global__ void __launch_bounds__(384) feat_attn_mma_kernel(const uint16_t* __restrict__ qkv,
                                                             uint16_t* __restrict__ att, int T, long long n_rows,
                                                             int n_buf) {
@@ -336,7 +347,7 @@ __global__ void __launch_bounds__(384) feat_attn_mma_kernel(const uint16_t* __re
     const int h = item / n_kt, mt = item % n_kt;
     // (the output block of the item overwrites the item's own Q block in shared memory: the row then leaves as whole
     // 16-byte pieces, coalesced, instead of 4-byte stores scattered over 8 token rows)
-    feat_attn_item<KT>(sbase, FA_ROW_BYTES, h * kD * 2, (kE + h * kD) * 2, (2 * kE + h * kD) * 2, T, n_kt, mt, lane);
+    feat_attn_item<KT, FMT>(sbase, FA_ROW_BYTES, h * kD * 2, (kE + h * kD) * 2, (2 * kE + h * kD) * 2, T, n_kt, mt, lane);
   }
   __syncthreads();
   {
@@ -355,12 +366,12 @@ __global__ void __launch_bounds__(384) feat_attn_mma_kernel(const uint16_t* __re
   }
 }
 
-template <int KT>
+template <int KT, int FMT>
 int launch_feat_attn_mma_t(const uint16_t* qkv, uint16_t* att, long long n_seq, int T, cudaStream_t st) {
   const int Tp = (T + 15) / 16 * 16;
   const int n_buf = (size_t)2 * Tp * FA_ROW_BYTES <= 200 * 1024 ? 2 : 1;
   const size_t smem = (size_t)n_buf * Tp * FA_ROW_BYTES;
-  auto kern = feat_attn_mma_kernel<KT>;
+  auto kern = feat_attn_mma_kernel<KT, FMT>;
   MMPFN_OPT_IN_SMEM(kern, 227 * 1024);
   const int n_sm = device_sm_count();
   const int n_items = kH * (Tp / 16);
@@ -381,12 +392,46 @@ int launch_feat_attn_f32(const float* qkv, float* att, long long n_seq, int T, c
 }
 int launch_feat_attn_bf16(const uint16_t* qkv, uint16_t* att, long long n_seq, int T, cudaStream_t st) {
   if (n_seq <= 0) return MMPFN_OK;
-  if (T <= 32) return launch_feat_attn_mma_t<2>(qkv, att, n_seq, T, st);
-  if (T <= 64) return launch_feat_attn_mma_t<4>(qkv, att, n_seq, T, st);
-  if (T <= 96) return launch_feat_attn_mma_t<6>(qkv, att, n_seq, T, st);
-  if (T <= 144) return launch_feat_attn_mma_t<9>(qkv, att, n_seq, T, st);
-  if (T <= 192) return launch_feat_attn_mma_t<12>(qkv, att, n_seq, T, st);
+  if (T <= 32) return launch_feat_attn_mma_t<2, FMT_BF16>(qkv, att, n_seq, T, st);
+  if (T <= 64) return launch_feat_attn_mma_t<4, FMT_BF16>(qkv, att, n_seq, T, st);
+  if (T <= 96) return launch_feat_attn_mma_t<6, FMT_BF16>(qkv, att, n_seq, T, st);
+  if (T <= 144) return launch_feat_attn_mma_t<9, FMT_BF16>(qkv, att, n_seq, T, st);
+  if (T <= 192) return launch_feat_attn_mma_t<12, FMT_BF16>(qkv, att, n_seq, T, st);
   return launch_feat_attn<uint16_t, uint16_t>(qkv, att, n_seq, T, st);   // CUDA-core fallback for very wide rows
+}
+// the same over an fp16 qkv block (fp16 out)
+int launch_feat_attn_f16(const uint16_t* qkv, uint16_t* att, long long n_seq, int T, cudaStream_t st) {
+  if (n_seq <= 0) return MMPFN_OK;
+  if (T <= 32) return launch_feat_attn_mma_t<2, FMT_F16>(qkv, att, n_seq, T, st);
+  if (T <= 64) return launch_feat_attn_mma_t<4, FMT_F16>(qkv, att, n_seq, T, st);
+  if (T <= 96) return launch_feat_attn_mma_t<6, FMT_F16>(qkv, att, n_seq, T, st);
+  if (T <= 144) return launch_feat_attn_mma_t<9, FMT_F16>(qkv, att, n_seq, T, st);
+  if (T <= 192) return launch_feat_attn_mma_t<12, FMT_F16>(qkv, att, n_seq, T, st);
+  return launch_feat_attn<f16_bits, f16_bits>(reinterpret_cast<const f16_bits*>(qkv), reinterpret_cast<f16_bits*>(att),
+                                              n_seq, T, st);
+}
+
+// ---------------------------------------------------------------------------------------------
+// The fp16 shadow of the fp32 state (the MMA operand of the fp16 layer pass): one pass, 4 values per thread.
+// ---------------------------------------------------------------------------------------------
+namespace {
+__global__ void __launch_bounds__(256) f16_shadow_kernel(const float4* __restrict__ x, uint2* __restrict__ y, long long n4) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long long)gridDim.x * blockDim.x) {
+    const float4 v = x[i];
+    y[i] = make_uint2(pack_f16x2_sat(v.x, v.y), pack_f16x2_sat(v.z, v.w));
+  }
+}
+}  // namespace
+
+int launch_f16_shadow(const float* x, uint16_t* y, long long n, cudaStream_t st) {
+  if (n <= 0) return MMPFN_OK;
+  if (n % 4) { set_error("f16_shadow: %lld values (a multiple of 4 expected)", n); return MMPFN_EINVAL; }
+  const long long n4 = n / 4;
+  long long grid = (n4 + 255) / 256;
+  const long long cap = (long long)device_sm_count() * 8;
+  if (grid > cap) grid = cap;
+  f16_shadow_kernel<<<(unsigned)grid, 256, 0, st>>>(reinterpret_cast<const float4*>(x), reinterpret_cast<uint2*>(y), n4);
+  return count_launch();
 }
 
 // ---------------------------------------------------------------------------------------------

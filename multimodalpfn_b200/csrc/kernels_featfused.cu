@@ -57,7 +57,7 @@ struct FusedArgs {
   int m_tiles, ctas_per_pair;
 };
 
-template <int KT>
+template <int KT, int FMT>
 __global__ void __launch_bounds__(U_THREADS, 1) feat_qkv_attn_kernel(const __grid_constant__ CUtensorMap map_a,
                                                                     const __grid_constant__ CUtensorMap map_w,
                                                                     const FusedArgs p) {
@@ -127,7 +127,7 @@ __global__ void __launch_bounds__(U_THREADS, 1) feat_qkv_attn_kernel(const __gri
     }
   } else if (warp == 1) {
     if (elect_one()) {
-      constexpr uint32_t idesc = make_idesc(U_BM, U_BN);
+      constexpr uint32_t idesc = make_idesc_fmt<FMT>(U_BM, U_BN);
       const uint32_t sbase = smem_u32(smem);
       mbar_wait(w_full, 0);
       for (int i = 0; i < my_tiles; ++i) {
@@ -169,10 +169,10 @@ __global__ void __launch_bounds__(U_THREADS, 1) feat_qkv_attn_kernel(const __gri
           tmem_ld_wait();
 #pragma unroll
           for (int k = 0; k < 4; ++k)
-            st_shared_v4(row + c * 64 + k * 16, pack_bf16x2(__uint_as_float(v[8 * k]), __uint_as_float(v[8 * k + 1])),
-                         pack_bf16x2(__uint_as_float(v[8 * k + 2]), __uint_as_float(v[8 * k + 3])),
-                         pack_bf16x2(__uint_as_float(v[8 * k + 4]), __uint_as_float(v[8 * k + 5])),
-                         pack_bf16x2(__uint_as_float(v[8 * k + 6]), __uint_as_float(v[8 * k + 7])));
+            st_shared_v4(row + c * 64 + k * 16, pack16x2<FMT>(__uint_as_float(v[8 * k]), __uint_as_float(v[8 * k + 1])),
+                         pack16x2<FMT>(__uint_as_float(v[8 * k + 2]), __uint_as_float(v[8 * k + 3])),
+                         pack16x2<FMT>(__uint_as_float(v[8 * k + 4]), __uint_as_float(v[8 * k + 5])),
+                         pack16x2<FMT>(__uint_as_float(v[8 * k + 6]), __uint_as_float(v[8 * k + 7])));
         }
         mbar_arrive_warp(&qkv_full[ab * 2 + h2]);
       }
@@ -195,7 +195,7 @@ __global__ void __launch_bounds__(U_THREADS, 1) feat_qkv_attn_kernel(const __gri
       for (int item = aw; item < n_items; item += 8) {
         const int g = item / n_kt, mt = item % n_kt;
         const uint32_t rbase = qbase + g * p.T * U_ROW;
-        feat_attn_item<KT>(rbase, U_ROW, h2 * 64, 128 + h2 * 64, 256 + h2 * 64, p.T, n_kt, mt, lane);
+        feat_attn_item<KT, FMT>(rbase, U_ROW, h2 * 64, 128 + h2 * 64, 256 + h2 * 64, p.T, n_kt, mt, lane);
         // the item's 16 query rows x 64 B sit over its q block: they leave from this warp right away (two 16-byte
         // pieces per lane), no barrier across the group
         __syncwarp();
@@ -221,10 +221,10 @@ __global__ void __launch_bounds__(U_THREADS, 1) feat_qkv_attn_kernel(const __gri
   }
 }
 
-template <int KT>
+template <int KT, int FMT>
 int launch_fused_t(const CUtensorMap& ma, const CUtensorMap& mw, const FusedArgs& a, int grid, cudaStream_t st) {
-  MMPFN_OPT_IN_SMEM(feat_qkv_attn_kernel<KT>, U_SMEM);
-  feat_qkv_attn_kernel<KT><<<grid, U_THREADS, U_SMEM, st>>>(ma, mw, a);
+  MMPFN_OPT_IN_SMEM((feat_qkv_attn_kernel<KT, FMT>), U_SMEM);
+  feat_qkv_attn_kernel<KT, FMT><<<grid, U_THREADS, U_SMEM, st>>>(ma, mw, a);
   return count_launch();
 }
 
@@ -232,8 +232,9 @@ int launch_fused_t(const CUtensorMap& ma, const CUtensorMap& mw, const FusedArgs
 
 bool feat_qkv_attn_supported(int T) { return T >= 2 && T <= 64; }
 
-// x [M][192] bf16 (M = n_rows * T), w_qkv [576][192] bf16 -> att [M][192] bf16
-int launch_feat_qkv_attn(const uint16_t* x, const uint16_t* w_qkv, long long M, int T, uint16_t* att, cudaStream_t st) {
+// x [M][192] bf16 (M = n_rows * T), w_qkv [576][192] bf16 -> att [M][192] bf16; all three fp16 with fmt = FMT_F16
+int launch_feat_qkv_attn(const uint16_t* x, const uint16_t* w_qkv, long long M, int T, uint16_t* att, cudaStream_t st,
+                         int fmt) {
   if (M <= 0) return MMPFN_OK;
   if (!feat_qkv_attn_supported(T) || M % T != 0 || M > 2147483647LL) {
     set_error("feat_qkv_attn: unsupported shape (M %lld, T %d)", M, T);
@@ -262,7 +263,9 @@ int launch_feat_qkv_attn(const uint16_t* x, const uint16_t* w_qkv, long long M, 
   if (per > a.m_tiles) per = a.m_tiles;
   if (per < 1) per = 1;
   a.ctas_per_pair = per;
-  return T <= 32 ? launch_fused_t<2>(ma, mw, a, per * 3, st) : launch_fused_t<4>(ma, mw, a, per * 3, st);
+  if (fmt == FMT_F16)
+    return T <= 32 ? launch_fused_t<2, FMT_F16>(ma, mw, a, per * 3, st) : launch_fused_t<4, FMT_F16>(ma, mw, a, per * 3, st);
+  return T <= 32 ? launch_fused_t<2, FMT_BF16>(ma, mw, a, per * 3, st) : launch_fused_t<4, FMT_BF16>(ma, mw, a, per * 3, st);
 }
 
 }  // namespace mmpfn

@@ -29,8 +29,9 @@
 //
 // GELU: 0.5 x (1 + erf(x / sqrt 2)) with erf(z) = tanh(g(z)), g an odd polynomial fitted to
 // atanh(erf) (max |error| of the GELU 3e-5 before the hardware tanh, whose 2^-11 relative error is
-// a quarter of the bf16 rounding the hidden activation gets anyway); one MUFU.TANH and ~5 issue
-// slots per element with packed f32x2 arithmetic, against ~30 for erff().
+// a quarter of the bf16 rounding the hidden activation gets anyway, and about the size of the fp16
+// one); one MUFU.TANH and ~5 issue slots per element with packed f32x2 arithmetic, against ~30 for erff().
+// The kernel is instantiated for bf16 and for fp16 operands (FMT): the tiles and bytes are the same.
 #include "tc_common.cuh"
 
 namespace mmpfn {
@@ -75,8 +76,9 @@ __device__ __forceinline__ uint64_t mul_f32x2(uint64_t a, uint64_t b) {
   asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
   return r;
 }
-// gelu of two values; returns them packed as bf16x2 (lo = first)
-__device__ __forceinline__ uint32_t gelu2_bf16(float x0, float x1) {
+// gelu of two values; returns them packed as a 16-bit pair of format FMT (lo = first)
+template <int FMT>
+__device__ __forceinline__ uint32_t gelu2_16(float x0, float x1) {
   const uint64_t x = pack_f32x2(x0, x1);
   float q0, q1;
   unpack_f32x2(mul_f32x2(x, x), q0, q1);
@@ -94,7 +96,7 @@ __device__ __forceinline__ uint32_t gelu2_bf16(float x0, float x1) {
   const uint64_t h = mul_f32x2(x, half);
   float y0, y1;
   unpack_f32x2(fma_f32x2(h, t, h), y0, y1);
-  return pack_bf16x2(y0, y1);
+  return pack16x2<FMT>(y0, y1);
 }
 
 // DBG = 1: clock64 trace of the MMA thread of CTA 0 (8 stamps per chunk: before / after each wait)
@@ -109,7 +111,7 @@ __device__ long long g_mlp_trace[4096];
     MLP_TRACE_BODY(slot)                                                                   \
   } while (0)
 
-template <int DBG>
+template <int DBG, int FMT>
 __global__ void __launch_bounds__(F_THREADS, 1) tc_mlp_kernel(const __grid_constant__ CUtensorMap map_a,
                                                             const __grid_constant__ CUtensorMap map_w1,
                                                             const __grid_constant__ CUtensorMap map_w2,
@@ -229,7 +231,7 @@ __global__ void __launch_bounds__(F_THREADS, 1) tc_mlp_kernel(const __grid_const
     // (~1900 cycles per chunk against 768 of tensor work).  The two streams only meet through
     // mbarriers (h_full/h_free via the GELU warps), so no ordering between the threads is needed.
     if (elect_one()) {
-      constexpr uint32_t idesc1 = make_idesc(F_BM, F_CH);
+      constexpr uint32_t idesc1 = make_idesc_fmt<FMT>(F_BM, F_CH);
       const uint32_t sbase = smem_u32(smem);
       for (int g = 0; g < G; ++g) {
         const int i = g / F_NCH, c = g % F_NCH;
@@ -260,7 +262,7 @@ __global__ void __launch_bounds__(F_THREADS, 1) tc_mlp_kernel(const __grid_const
   } else if (warp == 3) {
     // ---- GEMM2 issue: OUT[tile & 1] (+)= gelu(chunk g) W2c^T ----
     if (elect_one()) {
-      constexpr uint32_t idesc2 = make_idesc(F_BM, kE);
+      constexpr uint32_t idesc2 = make_idesc_fmt<FMT>(F_BM, kE);
       const uint32_t sbase = smem_u32(smem);
       for (int g = 0; g < G; ++g) {
         const int i = g / F_NCH, c = g % F_NCH;
@@ -318,9 +320,9 @@ __global__ void __launch_bounds__(F_THREADS, 1) tc_mlp_kernel(const __grid_const
       mbar_arrive_warp(&h_free[hb]);
       uint32_t pk[32];
 #pragma unroll
-      for (int i = 0; i < 16; ++i) pk[i] = gelu2_bf16(__uint_as_float(v0[2 * i]), __uint_as_float(v0[2 * i + 1]));
+      for (int i = 0; i < 16; ++i) pk[i] = gelu2_16<FMT>(__uint_as_float(v0[2 * i]), __uint_as_float(v0[2 * i + 1]));
 #pragma unroll
-      for (int i = 0; i < 16; ++i) pk[16 + i] = gelu2_bf16(__uint_as_float(v1[2 * i]), __uint_as_float(v1[2 * i + 1]));
+      for (int i = 0; i < 16; ++i) pk[16 + i] = gelu2_16<FMT>(__uint_as_float(v1[2 * i]), __uint_as_float(v1[2 * i + 1]));
       mbar_wait(&hs_empty[hb], ph ^ 1);          // GEMM2 of chunk g-2 has released this buffer
       // 64 hidden columns = the row's 128 B = eight 16-byte pieces, XOR-swizzled
 #pragma unroll
@@ -395,9 +397,9 @@ __global__ void __launch_bounds__(F_THREADS, 1) tc_mlp_kernel(const __grid_const
                        __float_as_uint(y[4 * k + 2]), __float_as_uint(y[4 * k + 3]));
 #pragma unroll
         for (int k = 0; k < 4; ++k)
-          st_shared_v4(y16 + ((k ^ ((r >> 1) & 3)) << 4), pack_bf16x2(y[8 * k], y[8 * k + 1]),
-                       pack_bf16x2(y[8 * k + 2], y[8 * k + 3]), pack_bf16x2(y[8 * k + 4], y[8 * k + 5]),
-                       pack_bf16x2(y[8 * k + 6], y[8 * k + 7]));
+          st_shared_v4(y16 + ((k ^ ((r >> 1) & 3)) << 4), pack16x2<FMT>(y[8 * k], y[8 * k + 1]),
+                       pack16x2<FMT>(y[8 * k + 2], y[8 * k + 3]), pack16x2<FMT>(y[8 * k + 4], y[8 * k + 5]),
+                       pack16x2<FMT>(y[8 * k + 6], y[8 * k + 7]));
         fence_proxy_async();
         if (store_leader) bulk_wait_read0();
         epi_bar();
@@ -427,7 +429,7 @@ __global__ void __launch_bounds__(F_THREADS, 1) tc_mlp_kernel(const __grid_const
 
 }  // namespace
 
-int launch_tc_mlp(const TcMlp& p, cudaStream_t st) {
+int launch_tc_mlp(const TcMlp& p, cudaStream_t st, int fmt) {
   if (p.M <= 0) return MMPFN_OK;
   if (!p.state_b || !p.w1 || !p.w2 || !p.resid_f32 || !p.state_b_out) { set_error("tc_mlp: null argument"); return MMPFN_EINVAL; }
   CUtensorMap ma, mw1, mw2, mr, my;
@@ -462,27 +464,30 @@ int launch_tc_mlp(const TcMlp& p, cudaStream_t st) {
     MMPFN_TRY(encode_map(&mw2, p.w2, 2, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B));
   }
   const int n_sm = device_sm_count();
-  MMPFN_OPT_IN_SMEM(tc_mlp_kernel<0>, F_SMEM);
-#ifdef MMPFN_DEBUG
-  MMPFN_OPT_IN_SMEM(tc_mlp_kernel<1>, F_SMEM);
-  static int dbg = -1;
-  if (dbg < 0) {
-    const char* e = getenv("MMPFN_MLP_DBG");          // tuning build only: clock64 trace variant
-    dbg = e ? atoi(e) : 0;
-  }
-#endif
   MlpArgs a{};
   a.M = p.M;
   a.n_tiles = (p.M + F_BM - 1) / F_BM;
   a.state_b = p.state_b;
   const int grid = a.n_tiles < n_sm ? a.n_tiles : n_sm;
+  if (fmt == FMT_F16) {
+    MMPFN_OPT_IN_SMEM((tc_mlp_kernel<0, FMT_F16>), F_SMEM);
+    tc_mlp_kernel<0, FMT_F16><<<grid, F_THREADS, F_SMEM, st>>>(ma, mw1, mw2, mr, my, a);
+    return count_launch();
+  }
+  MMPFN_OPT_IN_SMEM((tc_mlp_kernel<0, FMT_BF16>), F_SMEM);
 #ifdef MMPFN_DEBUG
+  MMPFN_OPT_IN_SMEM((tc_mlp_kernel<1, FMT_BF16>), F_SMEM);
+  static int dbg = -1;
+  if (dbg < 0) {
+    const char* e = getenv("MMPFN_MLP_DBG");          // tuning build only: clock64 trace variant
+    dbg = e ? atoi(e) : 0;
+  }
   if (dbg) {
-    tc_mlp_kernel<1><<<grid, F_THREADS, F_SMEM, st>>>(ma, mw1, mw2, mr, my, a);
+    tc_mlp_kernel<1, FMT_BF16><<<grid, F_THREADS, F_SMEM, st>>>(ma, mw1, mw2, mr, my, a);
     return count_launch();
   }
 #endif
-  tc_mlp_kernel<0><<<grid, F_THREADS, F_SMEM, st>>>(ma, mw1, mw2, mr, my, a);
+  tc_mlp_kernel<0, FMT_BF16><<<grid, F_THREADS, F_SMEM, st>>>(ma, mw1, mw2, mr, my, a);
   return count_launch();
 }
 

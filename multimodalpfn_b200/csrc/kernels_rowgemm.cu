@@ -67,7 +67,7 @@ struct alignas(64) ItemMaps {
   CUtensorMap q, k, vt, k0, vt0;
 };
 
-template <int EPI>
+template <int EPI, int FMT>
 __global__ void __launch_bounds__(R_THREADS, 1) tc_rowgemm_kernel(const __grid_constant__ CUtensorMap map_a,
                                                                   const __grid_constant__ CUtensorMap map_w,
                                                                   const __grid_constant__ CUtensorMap map_r,
@@ -171,7 +171,7 @@ __global__ void __launch_bounds__(R_THREADS, 1) tc_rowgemm_kernel(const __grid_c
     }
   } else if (warp == 1) {
     if (elect_one()) {
-      constexpr uint32_t idesc = make_idesc(R_BM, R_BN);
+      constexpr uint32_t idesc = make_idesc_fmt<FMT>(R_BM, R_BN);
       const uint32_t sbase = smem_u32(smem);
       mbar_wait(w_full, 0);
       for (int i = 0; i < my_tiles; ++i) {
@@ -186,7 +186,7 @@ __global__ void __launch_bounds__(R_THREADS, 1) tc_rowgemm_kernel(const __grid_c
           // rows (s) on the N side — so that the accumulator already IS V^T (lane = d, column = s) and the epilogue
           // writes whole 16-byte pieces of a d row instead of 2-byte elements.  192 d rows = two M = 128 MMAs (the
           // second one's upper 64 lanes multiply whatever follows the W tile in shared memory and are never read).
-          constexpr uint32_t idesc_t = make_idesc(128, R_BM);
+          constexpr uint32_t idesc_t = make_idesc_fmt<FMT>(128, R_BM);
 #pragma unroll
           for (int half = 0; half < 2; ++half)
 #pragma unroll
@@ -237,10 +237,10 @@ __global__ void __launch_bounds__(R_THREADS, 1) tc_rowgemm_kernel(const __grid_c
 #pragma unroll
             for (int k = 0; k < 4; ++k)
               st_shared_v4(yrow + (((hh * 4 + k) ^ rsw) << 4),
-                           pack_bf16x2(__uint_as_float(v[8 * k]), __uint_as_float(v[8 * k + 1])),
-                           pack_bf16x2(__uint_as_float(v[8 * k + 2]), __uint_as_float(v[8 * k + 3])),
-                           pack_bf16x2(__uint_as_float(v[8 * k + 4]), __uint_as_float(v[8 * k + 5])),
-                           pack_bf16x2(__uint_as_float(v[8 * k + 6]), __uint_as_float(v[8 * k + 7])));
+                           pack16x2<FMT>(__uint_as_float(v[8 * k]), __uint_as_float(v[8 * k + 1])),
+                           pack16x2<FMT>(__uint_as_float(v[8 * k + 2]), __uint_as_float(v[8 * k + 3])),
+                           pack16x2<FMT>(__uint_as_float(v[8 * k + 4]), __uint_as_float(v[8 * k + 5])),
+                           pack16x2<FMT>(__uint_as_float(v[8 * k + 6]), __uint_as_float(v[8 * k + 7])));
           }
           fence_proxy_async();
           if (store_leader) bulk_wait_read0();        // the previous chunk's store has read the other slot
@@ -300,9 +300,9 @@ __global__ void __launch_bounds__(R_THREADS, 1) tc_rowgemm_kernel(const __grid_c
                          __float_as_uint(y[4 * k + 2]), __float_as_uint(y[4 * k + 3]));
 #pragma unroll
           for (int k = 0; k < 4; ++k)
-            st_shared_v4(y16 + ((k ^ ((r >> 1) & 3)) << 4), pack_bf16x2(y[8 * k], y[8 * k + 1]),
-                         pack_bf16x2(y[8 * k + 2], y[8 * k + 3]), pack_bf16x2(y[8 * k + 4], y[8 * k + 5]),
-                         pack_bf16x2(y[8 * k + 6], y[8 * k + 7]));
+            st_shared_v4(y16 + ((k ^ ((r >> 1) & 3)) << 4), pack16x2<FMT>(y[8 * k], y[8 * k + 1]),
+                         pack16x2<FMT>(y[8 * k + 2], y[8 * k + 3]), pack16x2<FMT>(y[8 * k + 4], y[8 * k + 5]),
+                         pack16x2<FMT>(y[8 * k + 6], y[8 * k + 7]));
           fence_proxy_async();
           if (store_leader) bulk_wait_read0();
           epi_bar();
@@ -335,10 +335,10 @@ __global__ void __launch_bounds__(R_THREADS, 1) tc_rowgemm_kernel(const __grid_c
 #pragma unroll
             for (int k = 0; k < 4; ++k)
               st_shared_v4(yrow + ((k ^ ((r >> 1) & 3)) << 4),
-                           pack_bf16x2(__uint_as_float(v[8 * k]), __uint_as_float(v[8 * k + 1])),
-                           pack_bf16x2(__uint_as_float(v[8 * k + 2]), __uint_as_float(v[8 * k + 3])),
-                           pack_bf16x2(__uint_as_float(v[8 * k + 4]), __uint_as_float(v[8 * k + 5])),
-                           pack_bf16x2(__uint_as_float(v[8 * k + 6]), __uint_as_float(v[8 * k + 7])));
+                           pack16x2<FMT>(__uint_as_float(v[8 * k]), __uint_as_float(v[8 * k + 1])),
+                           pack16x2<FMT>(__uint_as_float(v[8 * k + 2]), __uint_as_float(v[8 * k + 3])),
+                           pack16x2<FMT>(__uint_as_float(v[8 * k + 4]), __uint_as_float(v[8 * k + 5])),
+                           pack16x2<FMT>(__uint_as_float(v[8 * k + 6]), __uint_as_float(v[8 * k + 7])));
           }
         } else {
           // the accumulators hold V^T: lanes of half 0 = d rows of heads 0-3 (warp = head), half 1 = heads 4, 5 (warps
@@ -357,10 +357,10 @@ __global__ void __launch_bounds__(R_THREADS, 1) tc_rowgemm_kernel(const __grid_c
 #pragma unroll
               for (int k = 0; k < 4; ++k)
                 st_shared_v4(drow + (c >> 1) * (kD * 128) + ((((c & 1) * 4 + k) ^ (lane & 7)) << 4),
-                             pack_bf16x2(__uint_as_float(v[8 * k]), __uint_as_float(v[8 * k + 1])),
-                             pack_bf16x2(__uint_as_float(v[8 * k + 2]), __uint_as_float(v[8 * k + 3])),
-                             pack_bf16x2(__uint_as_float(v[8 * k + 4]), __uint_as_float(v[8 * k + 5])),
-                             pack_bf16x2(__uint_as_float(v[8 * k + 6]), __uint_as_float(v[8 * k + 7])));
+                             pack16x2<FMT>(__uint_as_float(v[8 * k]), __uint_as_float(v[8 * k + 1])),
+                             pack16x2<FMT>(__uint_as_float(v[8 * k + 2]), __uint_as_float(v[8 * k + 3])),
+                             pack16x2<FMT>(__uint_as_float(v[8 * k + 4]), __uint_as_float(v[8 * k + 5])),
+                             pack16x2<FMT>(__uint_as_float(v[8 * k + 6]), __uint_as_float(v[8 * k + 7])));
             }
           }
         }
@@ -402,18 +402,19 @@ __global__ void __launch_bounds__(R_THREADS, 1) tc_rowgemm_kernel(const __grid_c
   }
 }
 
-template <int EPI>
+template <int EPI, int FMT>
 int launch_rowgemm_t(const CUtensorMap& ma, const CUtensorMap& mw, const CUtensorMap& mr, const CUtensorMap& my,
                      const ItemMaps& im, const RowGemmArgs& a, int grid, cudaStream_t st) {
-  MMPFN_OPT_IN_SMEM(tc_rowgemm_kernel<EPI>, R_SMEM);
-  tc_rowgemm_kernel<EPI><<<grid, R_THREADS, R_SMEM, st>>>(ma, mw, mr, my, im, a);
+  MMPFN_OPT_IN_SMEM((tc_rowgemm_kernel<EPI, FMT>), R_SMEM);
+  tc_rowgemm_kernel<EPI, FMT><<<grid, R_THREADS, R_SMEM, st>>>(ma, mw, mr, my, im, a);
   return count_launch();
 }
 
 }  // namespace
 
-// Same contract as launch_tc_gemm for K = 192, N % 192 == 0 and the BF16 / RESID_LN / QKV_ITEMS epilogues.
-int launch_tc_rowgemm(const TcGemm& p, cudaStream_t st) {
+// Same contract as launch_tc_gemm for K = 192, N % 192 == 0 and the BF16 / RESID_LN / QKV_ITEMS epilogues; with
+// fmt = FMT_F16 every 16-bit operand and output is fp16 instead of bf16 (the epilogue names keep saying "BF16").
+int launch_tc_rowgemm(const TcGemm& p, cudaStream_t st, int fmt) {
   if (p.K != R_K || p.N % R_BN != 0 || p.N <= 0) {
     set_error("tc_rowgemm: needs K=%d and N a multiple of %d (got N=%d K=%d)", R_K, R_BN, p.N, p.K);
     return MMPFN_EUNSUPPORTED;
@@ -500,10 +501,17 @@ int launch_tc_rowgemm(const TcGemm& p, cudaStream_t st) {
   if (per_n < 1) per_n = 1;
   a.ctas_per_n = per_n;
   const int grid = per_n * a.n_tiles;
+  const bool f16 = fmt == FMT_F16;
   switch (p.epi) {
-    case TC_EPI_BF16: return launch_rowgemm_t<TC_EPI_BF16>(ma, mw, mr, my, im, a, grid, st);
-    case TC_EPI_RESID_LN: return launch_rowgemm_t<TC_EPI_RESID_LN>(ma, mw, mr, my, im, a, grid, st);
-    case TC_EPI_QKV_ITEMS: return launch_rowgemm_t<TC_EPI_QKV_ITEMS>(ma, mw, mr, my, im, a, grid, st);
+    case TC_EPI_BF16:
+      return f16 ? launch_rowgemm_t<TC_EPI_BF16, FMT_F16>(ma, mw, mr, my, im, a, grid, st)
+                 : launch_rowgemm_t<TC_EPI_BF16, FMT_BF16>(ma, mw, mr, my, im, a, grid, st);
+    case TC_EPI_RESID_LN:
+      return f16 ? launch_rowgemm_t<TC_EPI_RESID_LN, FMT_F16>(ma, mw, mr, my, im, a, grid, st)
+                 : launch_rowgemm_t<TC_EPI_RESID_LN, FMT_BF16>(ma, mw, mr, my, im, a, grid, st);
+    case TC_EPI_QKV_ITEMS:
+      return f16 ? launch_rowgemm_t<TC_EPI_QKV_ITEMS, FMT_F16>(ma, mw, mr, my, im, a, grid, st)
+                 : launch_rowgemm_t<TC_EPI_QKV_ITEMS, FMT_BF16>(ma, mw, mr, my, im, a, grid, st);
   }
   set_error("tc_rowgemm: unsupported epilogue %d", p.epi);
   return MMPFN_EINVAL;

@@ -312,6 +312,11 @@ __device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t sbo_bytes
 __host__ __device__ constexpr uint32_t make_idesc(int M, int N) {
   return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
+// the same for A/B of format FMT: format bits [7,10) / [10,13) are 1 for bf16 (FMT_BF16), 0 for fp16 (FMT_F16)
+template <int FMT>
+__host__ __device__ constexpr uint32_t make_idesc_fmt(int M, int N) {
+  return FMT == FMT_F16 ? make_idesc(M, N) & ~((7u << 7) | (7u << 10)) : make_idesc(M, N);
+}
 
 // ---------------------------------------------------------------------------------------------
 // LayerNorm statistics of the residual + LayerNorm epilogues (kernels_mlp.cu, kernels_rowgemm.cu,

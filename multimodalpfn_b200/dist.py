@@ -143,6 +143,9 @@ class ShardedEngine:
         self.groups = engine.groups
         self.members = engine.members
         m = self.model
+        if getattr(m, "precision", None) == 2:        # _lib.F16
+            raise ValueError("ShardedEngine does not run fp16 models (the multi-GPU layer entry point is bf16 only); "
+                             "build the model with precision='bf16' or 'fp32'")
         n_tr = engine.groups[0]["y_train"].shape[1]
         H_img = 0
         if engine.img_train_dev is not None:

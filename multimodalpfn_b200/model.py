@@ -72,14 +72,19 @@ class B200PerFeatureTransformer:
             raise RuntimeError(f"{torch.cuda.get_device_name(self.device)} is not an sm_100 device")
         self.geom = geom
         self.precision_name = precision
-        self.precision = {"fp32": _lib.F32, "bf16": _lib.BF16}[precision]
+        self.precision = {"fp32": _lib.F32, "bf16": _lib.BF16, "fp16": _lib.F16}[precision]
+        # the 16-bit shadow of the fp32 state the tensor-core layers read (None: the fp32 layers need none)
+        self.shadow_dtype = {_lib.F32: None, _lib.BF16: torch.bfloat16, _lib.F16: torch.float16}[self.precision]
         self.seed = seed
         # reference: classifier.py:396-406 switches the outlier step on with sigma 12; a model used
         # without that call keeps InferenceConfig.remove_outliers = False (model/config.py:43).
         self.outlier_std = outlier_std
         self.pos_emb_device = pos_emb_device
         with torch.cuda.device(self.device):
-            self.w = PackedWeights(state_dict, geom, self.device, with_bf16=True, stem_bf16=(precision == "bf16"))
+            # fp16: an fp16 copy of the layer blocks instead of the bf16 one; the stem stays on the fp32 FFMA path
+            f16 = precision == "fp16"
+            self.w = PackedWeights(state_dict, geom, self.device, with_bf16=not f16, stem_bf16=(precision == "bf16"),
+                                   with_f16=f16)
         self._g = C.byref(self.w.c_geom)
         self._w = C.byref(self.w.c_weights)
         self._w_test = C.byref(self.w.c_weights_test)      # second query set of two_sets_of_queries checkpoints
@@ -129,6 +134,11 @@ class B200PerFeatureTransformer:
                 self.scratch_epoch += 1
             self._buf[name] = t
         return t
+
+    def _stem_shadow(self, state_b):
+        """What the stem writes the 16-bit shadow into: the bf16 shadow; nothing in fp16 mode (the layer passes write
+        the fp16 shadow themselves) or in fp32 mode."""
+        return state_b if self.precision == _lib.BF16 else None
 
     def n_image_tokens(self, n_tok: int) -> int:
         return int(self.lib.mmpfn_image_tokens(self._g, n_tok)) if n_tok > 0 else 0
@@ -198,7 +208,7 @@ class B200PerFeatureTransformer:
         return y_train.to(torch.float32).mean(dim=1).contiguous(), mask
 
     def embed(self, X, stats, img_tok, y, y_mean, y_mask, pos_emb, *, B, S, F, x_bstride, y_bstride, nan_flag, out=None):
-        """Token assembly -> (state_f32 [B,S,T,E], state_bf16 or None)."""
+        """Token assembly -> (state_f32 [B,S,T,E], 16-bit shadow (bf16 / fp16) or None)."""
         G = self._n_groups(F) if X is not None else 0
         # img_tok [S, H, E]: shared by the B entries; [B, S, H, E]: one set per entry (packed tasks)
         H_img = 0 if img_tok is None else img_tok.shape[-2]
@@ -215,12 +225,13 @@ class B200PerFeatureTransformer:
             assert tuple(state.shape) == (B, S, T, E) and state.is_contiguous()
         else:
             state = torch.empty((B, S, T, E), dtype=torch.float32, device=self.device)
-            state_b = torch.empty((B, S, T, E), dtype=torch.bfloat16, device=self.device) \
-                if self.precision == _lib.BF16 else None
+            state_b = torch.empty((B, S, T, E), dtype=self.shadow_dtype, device=self.device) \
+                if self.shadow_dtype is not None else None
         _lib.check(self.lib.mmpfn_stem_tokens(
             self._g, self._w, _ptr(X), _ptr(stats), _ptr(img_tok), y.data_ptr(), y_mean.data_ptr(),
             y_mask.data_ptr(), pos_emb.data_ptr(), B, S, F if X is not None else 0, H_img, x_bstride, y_bstride,
-            img_bstride, state.data_ptr(), _ptr(state_b), nan_flag.data_ptr(), self._stream()), "mmpfn_stem_tokens")
+            img_bstride, state.data_ptr(), _ptr(self._stem_shadow(state_b)), nan_flag.data_ptr(), self._stream()),
+            "mmpfn_stem_tokens")
         return state, state_b
 
     # ------------------------------------------------------------------ layers / decoder
@@ -262,6 +273,8 @@ class B200PerFeatureTransformer:
         ``layer_stride`` / ``rank_stride`` (bytes) and ``slots``.  ``n_train=None``: train pass (writes the K/V),
         else test pass against ``n_train`` context rows.  ``phase`` 1 leaves the queries in the workspace for
         ``phase`` 2: callers that interleave several states between the two name a workspace each (``ws_key``)."""
+        if self.precision != _lib.BF16:
+            raise ValueError("layers_run (the multi-GPU layer entry point) runs in bf16 only")
         n = len(segs)
         def seg(s):
             k = _lib.KvSegment()
@@ -298,7 +311,7 @@ class B200PerFeatureTransformer:
         L = self.geom.nlayers
         out = torch.empty(self.lib.mmpfn_kv_bytes(self._g, B, n_train, T, self.precision), dtype=torch.uint8,
                           device=self.device)
-        if self.precision == _lib.BF16:       # per layer: K0 [B][T][Sp][32] then V0^T [B][T][32][Sp]
+        if self.precision != _lib.F32:        # per layer: K0 [B][T][Sp][32] then V0^T [B][T][32][Sp] (bf16 / fp16)
             per_b = out.numel() // (L * 2 * B)
             dst = out.view(L, 2, B, per_b)
             for kv, pos in parts:
@@ -375,12 +388,12 @@ class B200PerFeatureTransformer:
 
     # ---- several estimator groups in one layer pass ----------------------------------------------------------
     def _group_buffers(self, shapes):
-        """One fp32 buffer (and, in bf16, one bf16 shadow) for states of the given [(B, S, T)] shapes, and the
-        per-group views."""
+        """One fp32 buffer (and, in bf16 / fp16, one 16-bit shadow) for states of the given [(B, S, T)] shapes, and
+        the per-group views."""
         E = self.geom.emsize
         total = sum(b * s * t for b, s, t in shapes)
         st = torch.empty((total, E), dtype=torch.float32, device=self.device)
-        stb = torch.empty((total, E), dtype=torch.bfloat16, device=self.device) if self.precision == _lib.BF16 else None
+        stb = torch.empty((total, E), dtype=self.shadow_dtype, device=self.device) if self.shadow_dtype is not None else None
         views, off = [], 0
         for b, s, t in shapes:
             n = b * s * t
@@ -636,7 +649,7 @@ class B200PerFeatureTransformer:
         _lib.check(self.lib.mmpfn_stem_tokens_ragged(
             self._g, self._w, _ptr(x), _ptr(stats), _ptr(tok), y_tr.data_ptr() if train else y_nan.data_ptr(),
             y_mean.data_ptr(), y_mask.data_ptr(), pos.data_ptr(), B, S, F, H, x_bstride, S_tr if train else 0,
-            _ptr(off), _ptr(cnt), out.data_ptr(), _ptr(out_b), flag.data_ptr(), self._stream()),
+            _ptr(off), _ptr(cnt), out.data_ptr(), _ptr(self._stem_shadow(out_b)), flag.data_ptr(), self._stream()),
             "mmpfn_stem_tokens_ragged")
 
     def forward_batch(self, X_full, img_full, y_train, *, check=True, return_embeddings=False):

@@ -3,7 +3,8 @@ encoding, ``EnsembleConfig`` generation, numpy/sklearn preprocessing) and swap o
 engine calls at ``inference.py:343-348`` for ``B200PerFeatureTransformer``.
 
     import multimodalpfn_b200.plugin as plugin
-    plugin.install(precision="bf16")          # after `mmpfn` is importable
+    plugin.install(precision="bf16")          # after `mmpfn` is importable; "fp16" (the reference's own CUDA
+                                              # autocast type, closer to fp32) and "fp32" work the same way
     clf = mmpfn.models.mmpfn.MMPFNClassifier(..., device="cuda").fit(X, img, y)
     clf.predict_proba(X_te, img_te)           # forward runs on libmmpfn_b200.so
 
@@ -195,7 +196,13 @@ def install(precision: str = "bf16", model_cls=None, pos_emb_device: str = "cuda
     swapped (one B = 1 CUDA forward per estimator).  ``mode="engine"`` (default): the engine object itself is
     replaced by ``B200PluginEngine`` (all estimators in one batched pass) — what SURVEY.md section 7 step 1(i)
     describes.  Both leave every line of the reference's ``fit`` / ``predict_proba`` in charge; ``replay=False`` also
-    keeps the reference's own per-member ``transform`` calls at predict time (``B200PluginEngine`` docstring)."""
+    keeps the reference's own per-member ``transform`` calls at predict time (``B200PluginEngine`` docstring).
+
+    ``precision``: the layer precision of the swapped-in model — "bf16" (default), "fp16" (fp16 tensor-core operands:
+    the type the reference itself autocasts to on CUDA, about 1/8 of bf16's distance from fp32) or "fp32" (the
+    1e-5 parity mode); torch dtypes and the estimators' ``inference_precision`` spellings are accepted too."""
+    from .classifier import precision_name
+    precision = precision_name(precision)
     import mmpfn.models.mmpfn.classifier as C
     import mmpfn.models.mmpfn.regressor as R
 

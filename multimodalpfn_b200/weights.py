@@ -38,7 +38,7 @@ class PackedWeights:
     """Device-resident weights + the ctypes structs the C ABI takes."""
 
     def __init__(self, state_dict, geom: Geometry, device: torch.device, *, with_bf16: bool = True,
-                 stem_bf16: bool = True):
+                 stem_bf16: bool = True, with_f16: bool = False):
         sd = {k: _np(v).astype(np.float64) for k, v in state_dict.items()}
         self.geom = geom
         self.device = torch.device(device)
@@ -73,12 +73,14 @@ class PackedWeights:
         layers = layer_blocks(0)
         self._t = {}
         self._t["layers_f32"] = torch.from_numpy(layers).to(self.device)
-        if with_bf16:
-            self._t["layers_bf16"] = self._t["layers_f32"].to(torch.bfloat16)
+        # 16-bit copies of the layer blocks for the tensor-core layers: bf16 (MMPFN_BF16) and / or fp16 (MMPFN_F16)
+        half = [(sfx, dt) for sfx, dt, on in (("bf16", torch.bfloat16, with_bf16), ("f16", torch.float16, with_f16)) if on]
+        for sfx, dt in half:
+            self._t["layers_" + sfx] = self._t["layers_f32"].to(dt)
         if self.two_sets_of_queries:
             self._t["layers_test_f32"] = torch.from_numpy(layer_blocks(1)).to(self.device)
-            if with_bf16:
-                self._t["layers_test_bf16"] = self._t["layers_test_f32"].to(torch.bfloat16)
+            for sfx, dt in half:
+                self._t["layers_test_" + sfx] = self._t["layers_test_f32"].to(dt)
 
         def put(name, arr):
             self._t[name] = torch.from_numpy(np.ascontiguousarray(arr, dtype=np.float32)).to(self.device)
@@ -168,7 +170,8 @@ class PackedWeights:
         if self.two_sets_of_queries:
             self.c_weights_test = _lib.Weights()
             for name in _lib.WEIGHT_FIELDS:
-                t = self._t.get({"layers_f32": "layers_test_f32", "layers_bf16": "layers_test_bf16"}.get(name, name))
+                t = self._t.get({"layers_f32": "layers_test_f32", "layers_bf16": "layers_test_bf16",
+                                 "layers_f16": "layers_test_f16"}.get(name, name))
                 setattr(self.c_weights_test, name, None if t is None else t.data_ptr())
         expected = _lib.load().mmpfn_layer_weight_elems(C.byref(self.c_geom)) * L
         if expected != layers.size:
@@ -178,7 +181,7 @@ class PackedWeights:
         return self._t[name]
 
     def n_params(self) -> int:
-        return sum(t.numel() for k, t in self._t.items() if not k.endswith("_bf16"))
+        return sum(t.numel() for k, t in self._t.items() if not k.endswith(("_bf16", "_f16")))
 
 
 def geometry_from_checkpoint(config: dict, state_dict, *, mixer_type, mgm_heads, cap_heads,
