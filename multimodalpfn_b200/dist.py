@@ -13,8 +13,12 @@ own offset of the gather buffer) on a communication stream, as soon as the owner
 the transfer of layer ``l`` overlaps layers ``l+1 .. 11`` of the context build and only the last one is
 exposed.  The buffer is laid out so that the test pass reads it where it lands — ``[layer][rank][group:
 K[slots][T][Np][32], V^T[slots][T][32][Np]]`` addressed by a 5-D TMA tensor map (estimator ``b`` of a
-group = (rank, slot)) — so nothing is re-gathered or merged.  The per-rank probabilities are
-all-gathered at the end.  Nothing else crosses GPUs.
+group = (rank, slot)) — so nothing is re-gathered or merged.  The per-rank probabilities (classifier) or the
+requested bar-distribution outputs (regressor) are all-gathered at the end.  Nothing else crosses GPUs.
+
+Test rows: rank r runs rows [r * c, (r + 1) * c) of the table, c = ceil(Nte / W) (``ShardedEngine.test_rows``); a short
+or empty last chunk repeats the table's last row, so that every rank's outputs have the same shape for the all-gather,
+and the gathered rows past Nte are dropped.
 
 Ownership (``KvPlan``): with W ranks and groups of B_g estimators (one group per preprocessed feature
 count),
@@ -35,6 +39,7 @@ from __future__ import annotations
 import dataclasses
 from typing import Dict, List, Optional, Tuple
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -133,13 +138,17 @@ class ShardedEngine:
         """``shard="estimators"`` (default): every estimator's context is built by one owner rank (module docstring).
         ``shard="rows"``: the TRAIN ROWS of every estimator are split over the ranks (``_logits_rows``) — the mode for
         fewer estimators than GPUs, where a single estimator's 50 000-row self-attention would otherwise run on one
-        GPU (SURVEY.md section 8(f) rank 2).  ``group="emulate"`` with ``shard="rows"``: the shares of all ``world``
-        ranks run one after the other on this device without any collective (tests of the segment addressing on a
-        single GPU)."""
+        GPU (SURVEY.md section 8(f) rank 2).  ``group="emulate"``: this process plays all ``world`` ranks on one device,
+        without any collective (tests of the addressing on a single GPU).  With ``shard="rows"`` the shares of all ranks
+        run one after the other; with estimator ownership every rank's owned build runs in turn into its offset of the
+        gather buffer (which then holds every rank's block, as after the all-gathers), or, in the broadcast mode, every
+        owner's contexts are built in turn and merged.  Then the staged test rows run, which for ``test_rows`` are the
+        chunks of all ranks, and the gathers of ``proba_gathered`` / ``regression_gathered`` have nothing to move."""
         self.engine = engine
         self.shard = shard
         self.model = engine.model
         self.rank, self.world, self.group = rank, world, group
+        self.emulate = group == "emulate"
         self.groups = engine.groups
         self.members = engine.members
         m = self.model
@@ -185,6 +194,21 @@ class ShardedEngine:
     def stage(self, X_test_per_member, image_test):
         return self.engine.stage(X_test_per_member, image_test)
 
+    def test_rows(self, n_test: int) -> np.ndarray:
+        """Row indices (into a table of ``n_test`` test rows) that this rank runs: rows [r * c, (r + 1) * c) with
+        c = ceil(n_test / W), a short or empty chunk padded by repeating row ``n_test - 1``.  Test rows are independent
+        and a repeated row cannot change the stem's "column varies over all rows" test, so the padding changes no real
+        row's result.  ``group="emulate"``: the chunks of all ranks, rank-major."""
+        if n_test < 1:
+            raise ValueError("no test rows")
+        c = -(-n_test // self.world)
+        ranks = range(self.world) if self.emulate else [self.rank]
+        return np.concatenate([np.minimum(np.arange(r * c, (r + 1) * c), n_test - 1) for r in ranks])
+
+    def _gather_rows(self, x: torch.Tensor) -> torch.Tensor:
+        """``all_gather_rows``; emulated, this process already holds the rows of every rank."""
+        return x if self.emulate else all_gather_rows(x, self.group)
+
     def _buffers(self):
         m = self.model
         if self._gather is None:
@@ -225,7 +249,8 @@ class ShardedEngine:
                         B=len(g["idx"]), S=n_te, F=g["F"], x_bstride=n_te * g["F"], y_bstride=0, nan_flag=flag, out=v)
             return bufs
         test_ready = None
-        if cuda and m.geom.mgm_heads < 32:      # (from 32 MGM heads the stem has a TMA / tcgen05 kernel: keep it in line)
+        # (from 32 MGM heads the stem has a TMA / tcgen05 kernel: keep it in line; emulated ranks run in line too)
+        if cuda and m.geom.mgm_heads < 32 and not self.emulate:
             main = torch.cuda.current_stream(dev)
             if self._side is None:
                 self._side = torch.cuda.Stream(device=dev)
@@ -239,20 +264,26 @@ class ShardedEngine:
         else:
             st2, stb2, views2 = embed_test_rows()
         # ---- 1. context build of the estimators this rank owns, all-gather of layer l under layers l+1.. -------
-        owned = plan.owned(self.rank)
-        shapes = [(len(pos), n_tr, self.Ts[gi]) for gi, pos in owned]
-        st, stb, views = m._group_buffers(shapes)
-        segs = []
-        for (gi, pos), v in zip(owned, views):
-            g, gp = eng.groups[gi], plan.groups[gi]
-            ls = g["label_stats"]
-            sel = slice(pos[0], pos[-1] + 1)
-            m.embed(g["X_train"][sel].contiguous(), stats[gi][sel].contiguous(), tok_tr, g["y_train"][sel].contiguous(),
-                    ls[0][sel].contiguous(), ls[1][sel].contiguous(), m.positional_embeddings(self.Ts[gi] - 1),
-                    B=len(pos), S=n_tr, F=g["F"], x_bstride=n_tr * g["F"], y_bstride=n_tr, nan_flag=flag, out=v)
-            segs.append(dict(B=len(pos), T=self.Ts[gi], kv=G[0, self.rank, gp.offset:gp.offset + gp.block],
-                             layer_stride=self.world * plan.chunk, slots=0, rank_stride=0,
-                             kv_buffer=G, kv_offset=self.rank * plan.chunk + gp.offset))
+        # (``group="emulate"``: the owned builds of all ranks, each into its own offset of the gather buffer)
+        builds = []
+        for rk in (range(self.world) if self.emulate else [self.rank]):
+            owned = plan.owned(rk)
+            shapes = [(len(pos), n_tr, self.Ts[gi]) for gi, pos in owned]
+            st, stb, views = m._group_buffers(shapes)
+            segs = []
+            for (gi, pos), v in zip(owned, views):
+                g, gp = eng.groups[gi], plan.groups[gi]
+                # the label statistics of the whole group, never of this rank's estimators (float targets: DESIGN.md
+                # section 6, label-mean rule)
+                ls = g["label_stats"]
+                sel = slice(pos[0], pos[-1] + 1)
+                m.embed(g["X_train"][sel].contiguous(), stats[gi][sel].contiguous(), tok_tr, g["y_train"][sel].contiguous(),
+                        ls[0][sel].contiguous(), ls[1][sel].contiguous(), m.positional_embeddings(self.Ts[gi] - 1),
+                        B=len(pos), S=n_tr, F=g["F"], x_bstride=n_tr * g["F"], y_bstride=n_tr, nan_flag=flag, out=v)
+                segs.append(dict(B=len(pos), T=self.Ts[gi], kv=G[0, rk, gp.offset:gp.offset + gp.block],
+                                 layer_stride=self.world * plan.chunk, slots=0, rank_stride=0,
+                                 kv_buffer=G, kv_offset=rk * plan.chunk + gp.offset))
+            builds.append((st, stb, segs))
         # this rank's test rows against every estimator read the gathered buffer in place (5-D tensor maps)
         tsegs = []
         for gi, g in enumerate(eng.groups):
@@ -267,8 +298,11 @@ class ShardedEngine:
         interleave = cuda and test_ready is not None
         landed = []
         for l in range(L):
-            if segs:
-                m.layers_run(st, stb, segs, n_tr, None, l, l + 1)
+            for st, stb, segs in builds:
+                if segs:
+                    m.layers_run(st, stb, segs, n_tr, None, l, l + 1)
+            if self.emulate:
+                continue
             if cuda:
                 ev = torch.cuda.Event()
                 ev.record(torch.cuda.current_stream(dev))
@@ -284,13 +318,14 @@ class ShardedEngine:
                         m.layers_run(st2, stb2, tsegs, n_te, n_tr, l, l + 1, ws_key="_test")
             else:
                 dist.all_gather_into_tensor(G[l].view(-1), G[l, self.rank].clone(), group=self.group)
-        self.exchange = {"collective": "all_gather_into_tensor", "calls_per_step": L,
-                         "bytes_received_per_rank": int(L * (self.world - 1) * plan.chunk), "mode": plan.mode}
+        self.exchange = {"collective": None, "mode": plan.mode} if self.emulate else \
+            {"collective": "all_gather_into_tensor", "calls_per_step": L,
+             "bytes_received_per_rank": int(L * (self.world - 1) * plan.chunk), "mode": plan.mode}
         if interleave:
             torch.cuda.current_stream(dev).wait_stream(self._side)
         else:
             for l in range(L):
-                if cuda:
+                if cuda and not self.emulate:
                     torch.cuda.current_stream(dev).wait_event(landed[l])
                 m.layers_run(st2, stb2, tsegs, n_te, n_tr, l, l + 1)
         out = [None] * len(self.members)
@@ -423,7 +458,33 @@ class ShardedEngine:
         [Nte_local, n_classes] per rank -> [W * Nte_local, n_classes] on every rank (device tensor)."""
         from .engine import proba_device
         p = proba_device(logits, class_perms, n_classes=n_classes, softmax_temperature=softmax_temperature)
-        return all_gather_rows(p, self.group)
+        return self._gather_rows(p)
+
+    def regression_gathered(self, logits: torch.Tensor, src_bucket, src_share, cancel, borders, *,
+                            softmax_temperature: float, average_before_softmax: bool, quantiles=None,
+                            outputs=("mean",), n_rows: Optional[int] = None) -> dict:
+        """The regressor's bar-distribution tail (``regressor.bar_tail_device``) on this rank's logits
+        [n_est, rows_r, K] and the all-gather of the requested outputs; the logits never leave the rank.  "mean",
+        "median", "mode" and "quantiles" travel as one [rows_r, 3 + n_q] block (one collective), "log_prob"
+        ([rows_r, K]) as a second one, only when it is requested.  -> dict of device tensors over the rows of all ranks
+        in test-row order, on every rank: [rows], [n_q, rows], [rows, K]; ``n_rows`` drops the padding rows of the last
+        chunk (``test_rows``)."""
+        from .regressor import bar_tail_device
+        out = bar_tail_device(logits, src_bucket, src_share, cancel, borders, softmax_temperature=softmax_temperature,
+                              average_before_softmax=average_before_softmax, quantiles=quantiles, outputs=outputs)
+        keep = slice(None) if n_rows is None else slice(0, n_rows)
+        scalars = [k for k in ("mean", "median", "mode") if k in out]
+        cols = [out[k][:, None] for k in scalars] + ([out["quantiles"].t()] if "quantiles" in out else [])
+        res = {}
+        if cols:
+            block = self._gather_rows(torch.cat(cols, dim=1))[keep]
+            for j, k in enumerate(scalars):
+                res[k] = block[:, j].contiguous()
+            if "quantiles" in out:
+                res["quantiles"] = block[:, len(scalars):].t().contiguous()
+        if "log_prob" in out:
+            res["log_prob"] = self._gather_rows(out["log_prob"])[keep]
+        return res
 
     def logits(self, X_test_per_member, image_test, *, graph: bool = False) -> torch.Tensor:
         return self.logits_staged(self.stage(X_test_per_member, image_test))
@@ -442,19 +503,22 @@ class ShardedEngine:
         tok_tr = tok_te = None
         if staged["img_test"] is not None:
             tok_tr, tok_te = eng.train_image_tokens(), m.stem_image(staged["img_test"])
-        owned = [si for si, sub in enumerate(self.subs) if sub.owner == self.rank]
-        specs = []
-        for si in owned:
-            sub = self.subs[si]
-            g = eng.groups[sub.group]
-            Xtr = None if g["X_train"] is None else g["X_train"][sub.pos].contiguous()
-            Xte = staged["X_test"][sub.group]
-            Xte = None if Xte is None else Xte[sub.pos].contiguous()
-            ls = g["label_stats"]
-            specs.append(dict(X_train=Xtr, y_train=g["y_train"][sub.pos].contiguous(),
-                              X_all=None if Xte is None else torch.cat([Xtr, Xte], dim=1), img_tok_train=tok_tr,
-                              label_stats=(ls[0][sub.pos].contiguous(), ls[1][sub.pos].contiguous())))
-        mine: Dict[int, TrainContext] = dict(zip(owned, m.fit_contexts(specs, nan_flag=eng.nan_flag))) if specs else {}
+        mine: Dict[int, TrainContext] = {}
+        for rk in (range(self.world) if self.emulate else [self.rank]):      # emulated: every owner in turn
+            owned = [si for si, sub in enumerate(self.subs) if sub.owner == rk]
+            specs = []
+            for si in owned:
+                sub = self.subs[si]
+                g = eng.groups[sub.group]
+                Xtr = None if g["X_train"] is None else g["X_train"][sub.pos].contiguous()
+                Xte = staged["X_test"][sub.group]
+                Xte = None if Xte is None else Xte[sub.pos].contiguous()
+                ls = g["label_stats"]
+                specs.append(dict(X_train=Xtr, y_train=g["y_train"][sub.pos].contiguous(),
+                                  X_all=None if Xte is None else torch.cat([Xtr, Xte], dim=1), img_tok_train=tok_tr,
+                                  label_stats=(ls[0][sub.pos].contiguous(), ls[1][sub.pos].contiguous())))
+            if specs:
+                mine.update(zip(owned, m.fit_contexts(specs, nan_flag=eng.nan_flag)))
         ctxs: Dict[int, TrainContext] = {}
         for si, sub in enumerate(self.subs):
             g = eng.groups[sub.group]
@@ -468,10 +532,10 @@ class ShardedEngine:
             if G_:
                 shapes.append(((B, n_stats), torch.float32))
             src = None
-            if sub.owner == self.rank:
+            if si in mine:
                 c = mine[si]
                 src = [c.kv, c.y_mean, c.y_mask] + ([c.tab_stats] if G_ else [])
-            got = broadcast_bundle(src, shapes, sub.owner, dev, self.group)
+            got = src if self.emulate else broadcast_bundle(src, shapes, sub.owner, dev, self.group)
             ctxs[si] = TrainContext(B=B, n_train=n_tr, F=F, T=T, kv=got[0], tab_stats=got[3] if G_ else None,
                                     y_mean=got[1], y_mask=got[2], pos_emb=m.positional_embeddings(T - 1),
                                     precision=m.precision)
@@ -502,7 +566,7 @@ class ShardedEngine:
         for g, lg in zip(eng.groups, lgs):
             for k, i in enumerate(g["idx"]):
                 out[i] = lg[k]
-        self.exchange = {"collective": "broadcast", "mode": "broadcast"}
+        self.exchange = {"collective": None if self.emulate else "broadcast", "mode": "broadcast"}
         return torch.stack(out)
 
 

@@ -323,23 +323,40 @@ class MMPFNRegressor(RegressorMixin, BaseEstimator):
                                              cache_context=(self.fit_mode == "fit_with_cache"))
         return self
 
-    def predict(self, X, image_test, *, output_type: str = "mean", quantiles=None):
+    def predict(self, X, image_test, *, output_type: str = "mean", quantiles=None, sharded=None):
         """float32 numpy per test row: "mean" / "median" / "mode" -> [Nte]; "quantiles" -> a list with one [Nte]
         array per quantile (default 0.1, 0.2, ..., 0.9); "main" -> dict of those four; "full" -> "main" plus
-        "logits" (log P, [Nte, K]) and "borders" (G, [K + 1])."""
+        "logits" (log P, [Nte, K]) and "borders" (G, [K + 1]).
+
+        ``sharded``: a ``dist.ShardedEngine`` built on ``self.executor_``.  Every rank passes the whole test table,
+        transforms and runs only its own chunk of rows (``ShardedEngine.test_rows``) and gets the whole result: the
+        bar tail runs on each rank's rows and only the requested outputs are all-gathered
+        (``ShardedEngine.regression_gathered``)."""
         check_is_fitted(self, "executor_")
         want, qs = output_request(output_type, quantiles)
         Xn = None if X is None else self._to_numeric(X, fit=False)
-        X_tests = transform_all(self.members_, Xn)
         if image_test is not None:
             image_test = np.asarray(image_test, dtype=np.float32)
             if image_test.ndim == 2:
                 image_test = image_test[:, None]
-        logits = self.executor_.logits(X_tests, image_test)
+        if sharded is not None:
+            if sharded.engine is not self.executor_:
+                raise ValueError("sharded must be a ShardedEngine built on this regressor's executor_")
+            n_test = len(Xn) if Xn is not None else len(image_test)
+            rows = sharded.test_rows(n_test)
+            Xn = None if Xn is None else Xn[rows]
+            image_test = None if image_test is None else image_test[rows]
+        X_tests = transform_all(self.members_, Xn)
         q_dev = torch.from_numpy(qs.astype(np.float32)).to(self.model_.device) if "quantiles" in want else None
-        out = bar_tail_device(logits, self._src_bucket, self._src_share, self._cancel, self._borders_dev,
-                              softmax_temperature=self.softmax_temperature,
-                              average_before_softmax=self.average_before_softmax, quantiles=q_dev, outputs=want)
+        tail = dict(softmax_temperature=self.softmax_temperature, average_before_softmax=self.average_before_softmax,
+                    quantiles=q_dev, outputs=want)
+        if sharded is None:
+            logits = self.executor_.logits(X_tests, image_test)
+            out = bar_tail_device(logits, self._src_bucket, self._src_share, self._cancel, self._borders_dev, **tail)
+        else:
+            logits = sharded.logits(X_tests, image_test)
+            out = sharded.regression_gathered(logits, self._src_bucket, self._src_share, self._cancel,
+                                              self._borders_dev, n_rows=n_test, **tail)
         host = {k: v.cpu().numpy() for k, v in out.items()}
         self.executor_.check_nan()
         return format_result(host, output_type, self.target_borders_)
